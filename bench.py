@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2|cfg5|cfg4]       # this repo's sm_100a path
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...   # N > 1
     python bench.py --impl reference ...                                  # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR      # also write the last timed step's outputs (.npy) to compare two builds
 
 One step (cfg2 / cfg5) = pack (features, ragged -> cu_seqlens) -> aligner forward (bf16 autocast regime) -> masked MSE against T5
 targets -> aligner backward -> gradient exchange between ranks when N > 1 -> AdamW, on one batch of synthetic Qwen2-VL-7B
@@ -54,6 +55,29 @@ def measured_peaks():
         return {"hbm_gbs": p["hbm_gbs"], "bf16_tflops": p["bf16_tflops"], "bf16_tflops_sustained": p.get("bf16_tflops_sustained", p["bf16_tflops"]),
                 "sm_max_mhz": p.get("sm_max_mhz"), "source": "measured"}
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0, "sm_max_mhz": 1965.0, "source": "fallback"}
+
+
+DUMP_SAMPLE = 1 << 22  # entries kept of a larger output array: at most 16 MB per file
+DUMP_LIMIT = 64 << 20  # bytes of one whole dump
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write ``arrays`` ({name: tensor}) as ``out_dir/<name>.npy`` in float32, so that two builds of the project can be compared
+    output for output from the same command line. An array of more than DUMP_SAMPLE entries is flattened and written as a fixed
+    sample of them: sorted flat indices drawn by a generator seeded with the array's size, the same on every run. A set of arrays
+    that would take more than DUMP_LIMIT bytes is refused before anything is written."""
+    import numpy as np
+
+    total = sum(4 * min(t.numel(), DUMP_SAMPLE) for t in arrays.values())
+    if total > DUMP_LIMIT:
+        raise ValueError(f"--dump-outputs: {total} bytes of outputs exceed the limit of {DUMP_LIMIT}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.size > DUMP_SAMPLE:
+            idx = np.sort(np.random.RandomState(a.size % (1 << 32)).choice(a.size, DUMP_SAMPLE, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def load_synth():
@@ -204,17 +228,18 @@ def cpu_reference_run(steps: int, warmup: int, din: int, seqs: int, max_len: int
         loss.backward()
         opt.step()
         opt.zero_grad(set_to_none=True)
-        return float(loss.detach())
+        return loss.detach()
 
     for _ in range(warmup):
         step()
     t0 = time.perf_counter()
     for _ in range(steps):
-        step()
+        loss = step()
     dt = time.perf_counter() - t0
     return {"value": tokens * steps / dt, "unit": UNIT, "cores": cores, "kind": "port",
             "sample": f"first {keep} sequences of the batch = {tokens} valid tokens, fp32, fwd+MSE+bwd+AdamW, {steps} steps after {warmup} warm-up",
-            "ms_per_step": dt / steps * 1e3, "tokens_per_step": tokens}
+            "ms_per_step": dt / steps * 1e3, "tokens_per_step": tokens,
+            "outputs": {"loss": loss, **{"param." + k: p for k, p in m.named_parameters()}}}
 
 
 def run_reference_arm(args, emit):
@@ -222,10 +247,11 @@ def run_reference_arm(args, emit):
     if rank != 0:
         return
     din, seqs, max_len, _ = WORKLOADS["cfg2" if args.workload == "cfg4" else args.workload]
-    steps = min(args.steps, 8)
-    r = cpu_reference_run(steps, min(args.warmup, 2), din, seqs, max_len)
-    line = {"metric": METRIC, "value": r["value"], "unit": UNIT, "impl": "reference", "n_gpus": args.gpus, "steps": steps,
-            "warmup": min(args.warmup, 2), "ms_per_step": r["ms_per_step"], "higher_is_better": True, "scaling": "weak",
+    r = cpu_reference_run(args.steps, args.warmup, din, seqs, max_len)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, r["outputs"])
+    line = {"metric": METRIC, "value": r["value"], "unit": UNIT, "impl": "reference", "n_gpus": args.gpus, "steps": args.steps,
+            "warmup": args.warmup, "ms_per_step": r["ms_per_step"], "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": workload_config(args.workload, args.gpus),
             "cpu_baseline": {k: r[k] for k in ("value", "unit", "cores", "kind", "sample")},
@@ -523,7 +549,13 @@ def main():
                     help="fused: this repo's one-pass AdamW (+ bf16 copies, per-bucket overlap); torch: torch.optim.AdamW(fused=True)")
     ap.add_argument("--loss-path", default="fused", choices=["fused", "module"],
                     help="fused: fused norm + MSE + norm backward (y/dy stay on chip); module: forward() -> masked MSE -> backward()")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32): the loss and every "
+                         "parameter after its update (cfg4: the padded prompt embeddings and their mask; --impl reference: the CPU "
+                         f"arm's loss and parameters); arrays of more than {DUMP_SAMPLE} entries as a fixed sample of them")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     # stdout carries exactly ONE line (the JSON); anything a library prints there meanwhile (e.g. NCCL's version
     # banner) is diverted to stderr
     real_stdout = os.dup(1)
@@ -659,6 +691,8 @@ def main():
     tokens = sum_over_ranks(float(sum(tokens_per_step[i % num_batches] for i in range(steps))))
     value = tokens / (ms * 1e-3)
     final_loss = float(loss)
+    if args.dump_outputs and rank == 0:  # before the passes below train the aligner further
+        dump_outputs(args.dump_outputs, {"loss": loss, **{"param." + k: p for k, p in aligner.named_parameters()}})
 
     # ---- end to end: pinned host buffers -> H2D -> step -> D2H loss, every step ---------------------
     e2e = None
@@ -860,9 +894,11 @@ def run_cfg4(args, emit, td, L, dev, world, rank, local, sync_all, max_over_rank
     with clocks:
         e0.record()
         for i in range(steps):
-            step(*batches[i % nb])
+            out = step(*batches[i % nb])
         e1.record()
         sync_all()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"prompt_embeds": out[0], "prompt_mask": out[1]})
     ms = max_over_ranks(e0.elapsed_time(e1))
     tokens = sum_over_ranks(float(sum(batches[i % nb][3] for i in range(steps))))
     L.profile_enable(True)
