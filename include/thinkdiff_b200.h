@@ -43,7 +43,8 @@ int32_t td_device_check(void);
 
 /* Per-launch device timing for benchmarks: while enabled, every kernel launch of the library is bracketed by CUDA
  * events on its stream. td_profile_report fills `buf` [host] with "tag,launches,total_ms,total_work\n" lines, where
- * work = algorithmic FLOPs for gemm_* tags and algorithmic bytes for the row kernels. Enabling clears old records. */
+ * work = algorithmic FLOPs for gemm_* tags and for the attention kernels attn_fwd / attn_bwd_dkdv / attn_bwd_dq (visible
+ * (query, key) pairs only, see td_t5_attention_fwd), and algorithmic bytes for the row kernels. Enabling clears old records. */
 int32_t td_profile_enable(int32_t on);
 int32_t td_profile_report(char* buf /*[host]*/, int32_t buflen);
 /* One "tag,stream,start_ms,end_ms\n" line per recorded launch, relative to the first record: a per-stream device timeline. */
@@ -283,6 +284,39 @@ int32_t td_lm_head_ce_fwd_bwd(const void* seq, int64_t R, int32_t K, const void*
                               void* dlogits /* [R, V] bf16, may be == logits, may be NULL */,
                               void* dseq /* [R, K] bf16, may be NULL */, void* workspace, int64_t workspace_bytes,
                               td_stream_t stream);
+
+/* ---- SURVEY section 8 f-1: the frozen T5 decoder's attention core on PACKED rows -----------------------------------------
+ * Replaces the score / softmax / value product of transformers' T5Attention.forward (models/t5/modeling_t5.py, transformers==4.46.1
+ * as pinned by requirements.txt:14) for both of a decoder block's uses, called from T5ForDecoder.forward
+ * (thinkdiff/models/mllama_vllm_t5_embed_decoder_2.py:211-224) under the bf16 autocast of tasks/base_task.py:237:
+ *   cross (self_attention = 0): decoder rows cu_q[b]..cu_q[b+1] attend to aligner rows cu_k[b]..cu_k[b+1]   s = q.k
+ *   self  (self_attention = 1): decoder rows attend to the same rows (cu_k must be NULL or cu_q), causal    s = q.k + bias
+ * with T5's rules: no 1/sqrt(d_kv) scaling, fp32 softmax, d_kv = 64. The relative position bias arrives as a per-distance table
+ * bias_by_distance [H, n_dist] (fp32; row h = head h), entry min(i - j, n_dist - 1) for query position i >= key position j, both
+ * counted from the sample's first row (n_dist = max_distance = 128 is exact for T5's 32 buckets: every distance >= 113 is in the
+ * last bucket). Cross-attention takes no table.
+ *   Q [Mq, >= inner], K / V [Mk, >= inner], O [Mq, >= inner] bf16 with row pitches ld* (elements, multiples of 8; Q/K/V may be column
+ *   slices of one fused projection output), inner = 64 H columns per row, head h = columns [64 h, 64 h + 64).
+ *   lse [H, Mq] fp32 (natural-log softmax normaliser per row and head; NULL = inference). A sample with no keys gets O = 0 and
+ *   lse = -inf. max_len_q / max_len_k bound every sample's length (host-known, like flash-attn's max_seqlen): the grid is
+ *   (ceil(max_len / 128), H, B); cu_* stay on the device and nothing synchronises. Rows outside every sample are not written.
+ * The backward writes dQ [Mq], dK, dV [Mk] (bf16, pitches lddq / lddk / lddv: dK and dV may be the two halves of one [Mk, 2 inner]
+ * buffer, the input gradient of a fused [Wk; Wv] projection) in three launches: Delta = rowsum(dO * O) into the workspace, dK / dV
+ * (one CTA per key tile), dQ (one CTA per query tile). Deterministic: every output element is written once, no atomics. Keys of a
+ * sample that no query sees get zero dK / dV. The bias table is frozen: it has no gradient.
+ * Profiling tags: attn_fwd, attn_bwd_delta (bytes), attn_bwd_dkdv, attn_bwd_dq (FLOPs of the products each kernel runs, over the
+ * VISIBLE (query, key) pairs only: 4, 8 and 6 x 64 H per pair). While profiling is enabled a call copies cu_* to the host to count
+ * the pairs (a synchronisation of `stream`). */
+int64_t td_t5_attention_workspace_bytes(int64_t Mq, int32_t H);
+int32_t td_t5_attention_fwd(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv,
+                            const int32_t* cu_q, const int32_t* cu_k, int32_t B, int32_t H, int32_t inner, int32_t max_len_q,
+                            int32_t max_len_k, int64_t Mq, int32_t self_attention, const float* bias_by_distance /* [H, n_dist] or NULL */,
+                            int32_t n_dist, void* o, int64_t ldo, float* lse /* [H, Mq] or NULL */, td_stream_t stream);
+int32_t td_t5_attention_bwd(const void* dout, int64_t lddo, const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v,
+                            int64_t ldv, const int32_t* cu_q, const int32_t* cu_k, int32_t B, int32_t H, int32_t inner,
+                            int32_t max_len_q, int32_t max_len_k, int64_t Mq, int32_t self_attention, const float* bias_by_distance,
+                            int32_t n_dist, const void* o, int64_t ldo, const float* lse, void* dq, int64_t lddq, void* dk,
+                            int64_t lddk, void* dv, int64_t lddv, void* workspace, int64_t workspace_bytes, td_stream_t stream);
 
 #ifdef __cplusplus
 }

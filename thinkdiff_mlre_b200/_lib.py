@@ -48,6 +48,10 @@ SIGNATURES = {
     "td_linear_bf16_dx": (_i32, [_vp, _i64, _i32, _vp, _i32, _vp, _vp, _i64, _vp]),
     "td_lm_head_ce_workspace_bytes": (_i64, [_i64]),
     "td_lm_head_ce_fwd_bwd": (_i32, [_vp, _i64, _i32, _vp, _i32, _vp, _f32, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
+    "td_t5_attention_workspace_bytes": (_i64, [_i64, _i32]),
+    "td_t5_attention_fwd": (_i32, [_vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i64, _i32, _vp, _i32, _vp, _i64, _vp, _vp]),
+    "td_t5_attention_bwd": (_i32, [_vp, _i64, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i64, _i32, _vp, _i32, _vp, _i64,
+                                   _vp, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _i64, _vp]),
     "td_gemm_bf16_f32out": (_i32, [_vp, _i64, _i32, _vp, _i64, _i32, _i64, _i32, _i64, _f32, _vp, _i32, _i32, _vp, _i64, _vp]),
     "td_adamw_step": (_i32, [_i32, _vp, _vp, _vp, _vp, _vp, C.POINTER(_i64), C.POINTER(_f32), _f32, _f32, _f32, _f32, _i64, _f32, _vp, _vp]),
     "td_step_ctl_bytes": (_i64, []),

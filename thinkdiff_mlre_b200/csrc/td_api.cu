@@ -6,6 +6,7 @@
 #include "gemm_host.cuh"
 #include "rowops_sm100.cuh"
 #include "peer_sm100.cuh"
+#include "attn_sm100.cuh"
 
 #include <cmath>
 
@@ -1171,6 +1172,151 @@ int32_t td_lm_head_ce_fwd_bwd(const void* seq, int64_t R, int32_t K, const void*
   if (rc) return rc;
   if (dseq) rc = td_linear_bf16_dx(dlogits, R, V, W_lm, K, dseq, sk, sk_bytes, stream);
   return rc;
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------ T5 attention (8 f-1)
+namespace {
+struct AttnCall {
+  int B, H, max_len_q, max_len_k;
+  bool causal;
+  AttnParams p;
+};
+
+inline bool misaligned16(const void* ptr) { return (reinterpret_cast<uintptr_t>(ptr) & 15) != 0; }
+
+// Host checks shared by the forward and the backward; fills the kernel parameters that both use.
+int attn_check(const char* fn, const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv, const int32_t* cu_q,
+               const int32_t* cu_k, int32_t B, int32_t H, int32_t inner, int32_t max_len_q, int32_t max_len_k, int64_t Mq,
+               int32_t self_attention, const float* bias, int32_t n_dist, AttnCall& c) {
+  if (B < 0 || B > 65535 || H <= 0 || H > 65535 || max_len_q < 0 || max_len_k < 0 || Mq < 0)
+    TD_FAIL(TD_ERR_ARG, "%s: bad sizes (B=%d H=%d max_len_q=%d max_len_k=%d Mq=%lld)", fn, B, H, max_len_q, max_len_k, (long long)Mq);
+  if (inner != kAttnDk * H) TD_FAIL(TD_ERR_UNSUPPORTED, "%s: inner=%d must be 64 * H = %d (d_kv = 64 only)", fn, inner, kAttnDk * H);
+  if (!q || !k || !v || !cu_q || (!self_attention && !cu_k)) TD_FAIL(TD_ERR_ARG, "%s: null pointer", fn);
+  if (misaligned16(q) || misaligned16(k) || misaligned16(v)) TD_FAIL(TD_ERR_ARG, "%s: q / k / v must be 16-byte aligned", fn);
+  if (ldq % 8 || ldk % 8 || ldv % 8 || ldq < inner || ldk < inner || ldv < inner)
+    TD_FAIL(TD_ERR_ARG, "%s: row pitches must be multiples of 8 and >= inner (ldq=%lld ldk=%lld ldv=%lld)", fn, (long long)ldq,
+            (long long)ldk, (long long)ldv);
+  if (self_attention) {
+    if (!bias) TD_FAIL(TD_ERR_ARG, "%s: self-attention needs the relative position bias table", fn);
+    if (cu_k && cu_k != cu_q) TD_FAIL(TD_ERR_ARG, "%s: self-attention attends to its own rows: cu_k must be NULL or cu_q", fn);
+    if (n_dist < 1 || n_dist > kAttnMaxDist) TD_FAIL(TD_ERR_ARG, "%s: n_dist=%d must be in [1, %d]", fn, n_dist, kAttnMaxDist);
+  } else if (bias) {
+    TD_FAIL(TD_ERR_ARG, "%s: cross-attention takes no position bias", fn);
+  }
+  c.B = B; c.H = H; c.max_len_q = max_len_q; c.max_len_k = max_len_k; c.causal = self_attention != 0;
+  memset(&c.p, 0, sizeof(c.p));
+  c.p.q = static_cast<const __nv_bfloat16*>(q); c.p.k = static_cast<const __nv_bfloat16*>(k); c.p.v = static_cast<const __nv_bfloat16*>(v);
+  c.p.ldq = ldq; c.p.ldk = ldk; c.p.ldv = ldv;
+  c.p.cu_q = cu_q; c.p.cu_k = self_attention ? cu_q : cu_k;
+  c.p.bias = self_attention ? bias : nullptr; c.p.n_dist = self_attention ? n_dist : 0;
+  c.p.H = H; c.p.Mq = Mq;
+  return TD_OK;
+}
+
+// Visible (query, key) pairs summed over the samples, for the profiler's FLOP count; 0 unless profiling is on (then it reads
+// cu_* back, which synchronises the stream).
+double attn_visible_pairs(const AttnCall& c, cudaStream_t st) {
+  if (!Profiler::get().on.load(std::memory_order_relaxed) || c.B == 0) return 0.0;
+  std::vector<int> hq(c.B + 1), hk(c.B + 1);
+  if (cudaMemcpyAsync(hq.data(), c.p.cu_q, sizeof(int) * (c.B + 1), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+      cudaMemcpyAsync(hk.data(), c.p.cu_k, sizeof(int) * (c.B + 1), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+      cudaStreamSynchronize(st) != cudaSuccess) {
+    cudaGetLastError();
+    return 0.0;
+  }
+  double pairs = 0.0;
+  for (int b = 0; b < c.B; ++b) {
+    const double T = hq[b + 1] - hq[b], L = hk[b + 1] - hk[b];
+    pairs += c.causal ? T * (T + 1) / 2 : T * L;
+  }
+  return pairs;
+}
+
+template <class K>
+int attn_launch(K kernel, dim3 grid, int threads, int smem, cudaStream_t st, const AttnParams& p, const char* tag, double work) {
+  if (grid.x == 0 || grid.y == 0 || grid.z == 0) return TD_OK;
+  TD_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  {
+    ProfScope prof(tag, work, st);
+    kernel<<<grid, threads, smem, st>>>(p);
+  }
+  TD_CUDA(cudaGetLastError());
+  return TD_OK;
+}
+
+inline unsigned attn_tiles(int max_len) { return unsigned((max_len + kAttnTile - 1) / kAttnTile); }
+}  // namespace
+
+extern "C" {
+
+int64_t td_t5_attention_workspace_bytes(int64_t Mq, int32_t H) {
+  const size_t rows = (size_t)(Mq > 0 ? Mq : 1), heads = (size_t)(H > 0 ? H : 1);
+  return (int64_t)align_up(sizeof(float) * rows * heads, 256);  // Delta [H, Mq]
+}
+
+int32_t td_t5_attention_fwd(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv, const int32_t* cu_q,
+                            const int32_t* cu_k, int32_t B, int32_t H, int32_t inner, int32_t max_len_q, int32_t max_len_k, int64_t Mq,
+                            int32_t self_attention, const float* bias, int32_t n_dist, void* o, int64_t ldo, float* lse,
+                            td_stream_t stream) {
+  TD_DEVICE_OR_RETURN();
+  AttnCall c;
+  int rc = attn_check("td_t5_attention_fwd", q, ldq, k, ldk, v, ldv, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, Mq, self_attention,
+                      bias, n_dist, c);
+  if (rc) return rc;
+  if (!o) TD_FAIL(TD_ERR_ARG, "td_t5_attention_fwd: null pointer (o)");
+  if (misaligned16(o) || ldo % 8 || ldo < inner) TD_FAIL(TD_ERR_ARG, "td_t5_attention_fwd: o must be 16-byte aligned with a pitch that is a multiple of 8 and >= inner");
+  c.p.out = static_cast<__nv_bfloat16*>(o); c.p.ld_out = ldo; c.p.lse = lse;
+  cudaStream_t st = (cudaStream_t)stream;
+  const double flops = 4.0 * kAttnDk * H * attn_visible_pairs(c, st);
+  const dim3 grid(attn_tiles(max_len_q), H, B);
+  const int smem = attn_smem_bytes(AttnFwdSmem::kBias, c.p.n_dist);
+  return c.causal ? attn_launch(t5_attn_fwd_kernel<true>, grid, kAttnThreads, smem, st, c.p, "attn_fwd", flops)
+                  : attn_launch(t5_attn_fwd_kernel<false>, grid, kAttnThreads, smem, st, c.p, "attn_fwd", flops);
+}
+
+int32_t td_t5_attention_bwd(const void* dout, int64_t lddo, const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v,
+                            int64_t ldv, const int32_t* cu_q, const int32_t* cu_k, int32_t B, int32_t H, int32_t inner, int32_t max_len_q,
+                            int32_t max_len_k, int64_t Mq, int32_t self_attention, const float* bias, int32_t n_dist, const void* o,
+                            int64_t ldo, const float* lse, void* dq, int64_t lddq, void* dk, int64_t lddk, void* dv, int64_t lddv,
+                            void* ws, int64_t ws_bytes, td_stream_t stream) {
+  TD_DEVICE_OR_RETURN();
+  AttnCall c;
+  int rc = attn_check("td_t5_attention_bwd", q, ldq, k, ldk, v, ldv, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, Mq, self_attention,
+                      bias, n_dist, c);
+  if (rc) return rc;
+  if (!dout || !o || !lse || !dq || !dk || !dv) TD_FAIL(TD_ERR_ARG, "td_t5_attention_bwd: null pointer");
+  if (misaligned16(dout) || misaligned16(o) || misaligned16(dq) || misaligned16(dk) || misaligned16(dv))
+    TD_FAIL(TD_ERR_ARG, "td_t5_attention_bwd: dout / o / dq / dk / dv must be 16-byte aligned");
+  if (lddo % 8 || ldo % 8 || lddq % 8 || lddk % 8 || lddv % 8 || lddo < inner || ldo < inner || lddq < inner || lddk < inner || lddv < inner)
+    TD_FAIL(TD_ERR_ARG, "td_t5_attention_bwd: row pitches must be multiples of 8 and >= inner");
+  if (!ws || ws_bytes < td_t5_attention_workspace_bytes(Mq, H)) TD_FAIL(TD_ERR_ARG, "td_t5_attention_bwd: workspace too small");
+  c.p.dout = static_cast<const __nv_bfloat16*>(dout); c.p.lddo = lddo;
+  c.p.o = static_cast<const __nv_bfloat16*>(o); c.p.ldo = ldo;
+  c.p.lse = const_cast<float*>(lse);
+  c.p.delta = static_cast<float*>(ws);
+  c.p.dq = static_cast<__nv_bfloat16*>(dq); c.p.lddq = lddq;
+  c.p.dk = static_cast<__nv_bfloat16*>(dk); c.p.lddk = lddk;
+  c.p.dv = static_cast<__nv_bfloat16*>(dv); c.p.lddv = lddv;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (B == 0) return TD_OK;
+  const double pairs = attn_visible_pairs(c, st);
+  const long long delta_threads = Mq * H * 8;
+  rc = attn_launch(t5_attn_delta_kernel, dim3(unsigned((delta_threads + 255) / 256)), 256, 0, st, c.p, "attn_bwd_delta",
+                   double(Mq) * H * (4.0 * kAttnDk + 4.0));
+  if (rc) return rc;
+  const dim3 grid_k(attn_tiles(max_len_k), H, B), grid_q(attn_tiles(max_len_q), H, B);
+  const int smem_kv = attn_smem_bytes(AttnDkdvSmem::kBias, c.p.n_dist), smem_q = attn_smem_bytes(AttnDqSmem::kBias, c.p.n_dist);
+  const double f = 2.0 * kAttnDk * H * pairs;
+  if (c.causal) {
+    rc = attn_launch(t5_attn_dkdv_kernel<true>, grid_q, kAttnThreads, smem_kv, st, c.p, "attn_bwd_dkdv", 4 * f);
+    if (rc) return rc;
+    return attn_launch(t5_attn_dq_kernel<true>, grid_q, kAttnThreads, smem_q, st, c.p, "attn_bwd_dq", 3 * f);
+  }
+  rc = attn_launch(t5_attn_dkdv_kernel<false>, grid_k, kAttnThreads, smem_kv, st, c.p, "attn_bwd_dkdv", 4 * f);
+  if (rc) return rc;
+  return attn_launch(t5_attn_dq_kernel<false>, grid_q, kAttnThreads, smem_q, st, c.p, "attn_bwd_dq", 3 * f);
 }
 
 }  // extern "C"

@@ -446,3 +446,88 @@ def lm_head_ce(seq, W_lm, labels, grad_scale: float = 1.0, want_grad: bool = Tru
                                           L.stream_ptr()), "td_lm_head_ce_fwd_bwd")
     return loss, dseq, (logits if keep_logits or not want_grad else None)
 
+
+
+# ------------------------------------------------------------------------------------------------ T5 attention (8 f-1)
+def _rows_operand(t, name, inner):
+    """A [rows, >= inner] bf16 operand with unit inner stride and a row pitch that is a multiple of 8 (column slices allowed)."""
+    if t.dtype != torch.bfloat16 or t.dim() != 2 or t.shape[1] != inner:
+        raise TypeError(f"{name} must be a bfloat16 [rows, {inner}] tensor, got {t.dtype} {tuple(t.shape)}")
+    if t.stride(1) != 1 or t.stride(0) % 8 or t.stride(0) < inner:
+        raise ValueError(f"{name} must have unit column stride and a row pitch that is a multiple of 8 (stride {t.stride()})")
+    return t
+
+
+def _attn_common(q, k, v, cu_q, cu_k, n_heads, bias_by_distance):
+    _need_cuda(q, k, v, cu_q, cu_k, bias_by_distance)
+    inner = q.shape[1]
+    for t, n in ((q, "q"), (k, "k"), (v, "v")):
+        _rows_operand(t, n, inner)
+    if k.shape[0] != v.shape[0]:
+        raise ValueError("k and v must have the same rows")
+    if cu_q.dtype != torch.int32 or (cu_k is not None and (cu_k.dtype != torch.int32 or cu_k.numel() != cu_q.numel())):
+        raise TypeError("cu_q / cu_k must be int32 [B + 1]")
+    self_attention = bias_by_distance is not None
+    n_dist = 0
+    if self_attention:
+        if bias_by_distance.dtype != torch.float32 or bias_by_distance.dim() != 2 or bias_by_distance.shape[0] != n_heads:
+            raise TypeError(f"bias_by_distance must be float32 [{n_heads}, n_dist]")
+        _contig(bias_by_distance, "bias_by_distance")
+        if cu_k is not None and cu_k.data_ptr() != cu_q.data_ptr():
+            raise ValueError("self-attention attends to its own rows: pass cu_k=None or cu_q")
+        cu_k = None
+        n_dist = bias_by_distance.shape[1]
+    elif cu_k is None:
+        raise ValueError("cross-attention needs cu_k")
+    return inner, self_attention, cu_k, n_dist
+
+
+def t5_attention_fwd(q, k, v, cu_q, cu_k, max_len_q: int, max_len_k: int, n_heads: int, bias_by_distance=None, o=None,
+                     need_lse: bool = True):
+    """T5 attention core on packed rows (no 1/sqrt(d_kv) scaling, fp32 softmax, d_kv = 64): sample b's queries are rows
+    ``cu_q[b]:cu_q[b+1]`` of ``q [Mq, 64 H]``, its keys / values rows ``cu_k[b]:cu_k[b+1]`` of ``k`` / ``v [Mk, 64 H]``.
+    ``bias_by_distance`` ([H, n_dist] fp32, see ``t5.t5_position_bias_by_distance``) selects causal self-attention (keys = the
+    query rows, ``cu_k`` None or ``cu_q``). Inputs may be column slices of a fused projection output. ``max_len_*`` bound the
+    samples' lengths (host-known; no device sync). Returns ``(o [Mq, 64 H] bf16, lse [H, Mq] fp32 or None)``; ``o`` may be given."""
+    inner, self_attention, cu_k, n_dist = _attn_common(q, k, v, cu_q, cu_k, n_heads, bias_by_distance)
+    Mq = q.shape[0]
+    if o is None:
+        o = torch.empty((Mq, inner), dtype=torch.bfloat16, device=q.device)
+    _rows_operand(o, "o", inner)
+    lse = torch.empty((n_heads, Mq), dtype=torch.float32, device=q.device) if need_lse else None
+    L.launch_count += 1
+    L.check(L.lib().td_t5_attention_fwd(L.ptr(q), q.stride(0), L.ptr(k), k.stride(0), L.ptr(v), v.stride(0), L.ptr(cu_q), L.ptr(cu_k),
+                                        cu_q.numel() - 1, n_heads, inner, int(max_len_q), int(max_len_k), Mq, int(self_attention),
+                                        L.ptr(bias_by_distance), n_dist, L.ptr(o), o.stride(0), L.ptr(lse), L.stream_ptr()),
+            "td_t5_attention_fwd")
+    return o, lse
+
+
+def t5_attention_bwd(dout, q, k, v, o, lse, cu_q, cu_k, max_len_q: int, max_len_k: int, n_heads: int, bias_by_distance=None,
+                     dq=None, dk=None, dv=None):
+    """Backward of ``t5_attention_fwd``: returns ``(dq, dk, dv)`` bf16. Any of them may be given, e.g. ``dk`` / ``dv`` as the two
+    column halves of one ``[Mk, 2 inner]`` buffer -- the input gradient of a fused ``[Wk; Wv]`` projection. Three launches
+    (row sums of dO * O, dK / dV, dQ); deterministic."""
+    inner, self_attention, cu_k, n_dist = _attn_common(q, k, v, cu_q, cu_k, n_heads, bias_by_distance)
+    Mq, Mk = q.shape[0], k.shape[0]
+    _need_cuda(dout, o, lse)
+    _rows_operand(dout, "dout", inner)
+    _rows_operand(o, "o", inner)
+    if lse is None or lse.dtype != torch.float32 or tuple(lse.shape) != (n_heads, Mq):
+        raise TypeError(f"lse must be float32 [{n_heads}, {Mq}] (run the forward with need_lse=True)")
+    _contig(lse, "lse")
+    dev = q.device
+    dq = torch.empty((Mq, inner), dtype=torch.bfloat16, device=dev) if dq is None else dq
+    dk = torch.empty((Mk, inner), dtype=torch.bfloat16, device=dev) if dk is None else dk
+    dv = torch.empty((Mk, inner), dtype=torch.bfloat16, device=dev) if dv is None else dv
+    for t, n in ((dq, "dq"), (dk, "dk"), (dv, "dv")):
+        _rows_operand(t, n, inner)
+    ws_bytes = L.lib().td_t5_attention_workspace_bytes(Mq, n_heads)
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+    L.launch_count += 3
+    L.check(L.lib().td_t5_attention_bwd(L.ptr(dout), dout.stride(0), L.ptr(q), q.stride(0), L.ptr(k), k.stride(0), L.ptr(v), v.stride(0),
+                                        L.ptr(cu_q), L.ptr(cu_k), cu_q.numel() - 1, n_heads, inner, int(max_len_q), int(max_len_k), Mq,
+                                        int(self_attention), L.ptr(bias_by_distance), n_dist, L.ptr(o), o.stride(0), L.ptr(lse),
+                                        L.ptr(dq), dq.stride(0), L.ptr(dk), dk.stride(0), L.ptr(dv), dv.stride(0), L.ptr(ws), ws_bytes,
+                                        L.stream_ptr()), "td_t5_attention_bwd")
+    return dq, dk, dv
