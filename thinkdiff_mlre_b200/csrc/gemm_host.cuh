@@ -33,6 +33,8 @@ enum : int { TD_OK = 0, TD_ERR_ARG = -1, TD_ERR_UNSUPPORTED = -2, TD_ERR_DRIVER 
 // by a pair of CUDA events on the launch stream; td_profile_report() sums them per tag, td_profile_timeline() lists them
 // with their offsets from the first record (events of different streams share the device clock, so this is a per-stream
 // timeline). Off by default (zero cost). Launches may come from several host threads (autograd runs backward on its own).
+// An event recorded between two kernels ends programmatic dependent launch there: with profiling on, every kernel starts after
+// its predecessor has completed, so the per-kernel times include the prologue that PDL otherwise hides under the previous kernel.
 struct ProfRecord { const char* tag; cudaEvent_t e0, e1; double work; cudaStream_t stream; };
 struct Profiler {
   std::atomic<bool> on{false};
@@ -205,8 +207,22 @@ struct GemmOperand {
 // Workspace for the stream-K tail of one GEMM launch: one accumulator slot per CTA.
 inline size_t gemm_sk_workspace_bytes() { return sizeof(float) * (size_t)device_sm_count() * kSkSlotFloats; }
 
+// Largest number of tail ranges that share one tail tile when the R * KB tail k-blocks are cut into p.tail_workers ranges.
+inline int max_tail_participants(const GemmParams& p, int R) {
+  const int KB = p.num_k_blocks;
+  int most = 1;
+  for (int t = 0; t < R; ++t) {
+    const int n = sk_worker_of(p, (t + 1) * KB - 1) - sk_worker_of(p, t * KB) + 1;
+    if (n > most) most = n;
+  }
+  return most;
+}
+
 // Fill the schedule fields of `p` for `workers` workers. With a stream-K workspace the tiles left over after the full waves are
 // cut along K into equal ranges (never shorter than kMinTailKBlocks); without one they form a last, partially filled wave.
+// The number of ranges minimises the tail's estimated time in k-blocks: the longest range plus kTailFoldKBlocks for every
+// partial the busiest owner folds in. More ranges shorten the MMA part but give each tail tile more contributors, and an
+// owner folds those in one after another.
 inline void plan_schedule(GemmParams& p, int max_workers, bool stream_k) {
   const int tiles = p.num_m_blocks * p.num_n_blocks;
   const int KB = p.num_k_blocks;
@@ -223,12 +239,21 @@ inline void plan_schedule(GemmParams& p, int max_workers, bool stream_k) {
   p.tail_workers = 0; p.tail_q = 0; p.tail_r = 0;
   if (stream_k && R > 0) {
     const long long units = (long long)R * KB;
-    long long wt = units / kMinTailKBlocks;
-    if (wt < R) wt = R;  // at least one worker per tile: a range never spans more than two tiles
-    if (wt > W) wt = W;
-    p.tail_workers = int(wt);
-    p.tail_q = int(units / wt);
-    p.tail_r = int(units % wt);
+    long long hi = units / kMinTailKBlocks;
+    if (hi < R) hi = R;  // at least one worker per tile: a range never spans more than two tiles
+    if (hi > W) hi = W;
+    long long best_cost = -1;
+    int best = int(hi);
+    for (int wt = int(hi); wt >= R; --wt) {  // ties keep the larger count (the shorter ranges)
+      p.tail_q = int(units / wt);
+      p.tail_r = int(units % wt);
+      const long long cost = (units + wt - 1) / wt + (long long)kTailFoldKBlocks * (max_tail_participants(p, R) - 1);
+      if (best_cost < 0 || cost < best_cost) { best_cost = cost; best = wt; }
+    }
+    p.tail_workers = best;
+    p.tail_q = int(units / best);
+    p.tail_r = int(units % best);
+    if (p.full_waves == 0) p.workers = best;  // every worker holds one tail range: launch no idle ones
   }
 }
 
@@ -293,13 +318,16 @@ int launch_gemm(GemmOperand a, GemmOperand b, GemmParams p, void* ws, cudaStream
   cfg.blockDim = dim3(kGemmThreads);
   cfg.dynamicSmemBytes = S::kTotal;
   cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
+  cudaLaunchAttribute attr[2];
   attr[0].id = cudaLaunchAttributeClusterDimension;
   attr[0].val.clusterDim.x = CTAS;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
+  // programmatic dependent launch: the prologue (barriers, TMEM, cluster sync) overlaps the previous kernel's tail
+  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = 1;
+  cfg.numAttrs = 2;
   ProfScope prof(tag, 2.0 * double(p.M) * double(p.N) * double(p.K), stream);
   TD_CUDA(cudaLaunchKernelEx(&cfg, kern, ma, mb, mo0, mo1, maux, smaps, p));
   return TD_OK;

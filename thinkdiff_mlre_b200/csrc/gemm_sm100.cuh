@@ -105,6 +105,14 @@ constexpr int kProducerWarp = TD_ROLES_HI ? 8 : 0;   // TMA producer
 constexpr int kMmaWarp = TD_ROLES_HI ? 9 : 1;        // TMEM owner + MMA issuer
 constexpr int kAccStages = 2;
 constexpr int kMinTailKBlocks = 8;  // a stream-K range shorter than this costs more in fix-up than it saves
+// What an owner pays to fold one contributor's partial into its accumulator, in k-blocks of MMA time (plan_schedule's tail cost
+// model). The fold reads 4 chunks of 4 KB per epilogue warp, one L2 round trip each, about 2 us, against about 0.3 us per k-block
+// of a 256 x 256 pair tile. On a B200 (1000 W) the config-2 step measured the same with 8, 16 and 32 (dW1 0.204-0.217 ms, inside
+// run-to-run noise; 0.229-0.243 ms with the old finest cut), so the estimate stands. TD_SK_FOLD_KBLOCKS overrides it for such A/Bs.
+#ifndef TD_SK_FOLD_KBLOCKS
+#define TD_SK_FOLD_KBLOCKS 8
+#endif
+constexpr int kTailFoldKBlocks = TD_SK_FOLD_KBLOCKS;
 
 // Eight epilogue warps: warp e (0..7) owns TMEM lane quarter (warp % 4) and column half e / 4 of the 256-column
 // accumulator, i.e. 32 rows x 128 columns, walked in 4 chunks of 32 columns. Thread = one output row.
@@ -539,6 +547,10 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
   tc_fence_before();
   if constexpr (CTAS == 2) cluster_sync_all(); else __syncthreads();
   tc_fence_after();
+  // Everything above touches only this CTA's (or pair's) shared memory, TMEM and kernel parameters, so it may run under the
+  // previous kernel's tail (programmatic dependent launch). The scheduler counter, every TMA load, the bias / alpha_ptr /
+  // stream-K flag reads and every store come after the wait.
+  grid_dependency_wait();
   const uint32_t tmem_base = *tmem_slot;
   const int num_workers = gridDim.x / CTAS;
   const int n_units = num_units(p);
@@ -616,6 +628,8 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
           }
         });
       }
+      // this worker has no unit left: the next kernel of the stream may start its prologue on the SMs that free up
+      grid_launch_dependents();
       if (leader) {
         // the last worker to run out of units re-arms the counter pair for the next launch that uses this slot
         __threadfence();

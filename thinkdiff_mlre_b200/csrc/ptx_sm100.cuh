@@ -136,6 +136,16 @@ __device__ __forceinline__ void spin_until_set(const int* p) {
   asm volatile("fence.acq_rel.gpu;" ::: "memory");
 }
 
+// ---------------------------------------------------------------- programmatic dependent launch
+// A kernel launched with cudaLaunchAttributeProgrammaticStreamSerialization may start while the previous kernel of its stream
+// is still running. grid_dependency_wait() blocks until that kernel has completed and its memory is visible; without the
+// attribute it returns at once. It only orders a kernel after its immediate predecessor, so every kernel launched with the
+// attribute must call it on every path -- otherwise it could finish before its predecessor, and its own successor's wait would
+// no longer cover that predecessor.
+__device__ __forceinline__ void grid_dependency_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+// Let the next kernel of the stream start launching (its CTAs run up to their grid_dependency_wait()).
+__device__ __forceinline__ void grid_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
 // ---------------------------------------------------------------- cluster
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;

@@ -66,6 +66,8 @@ __device__ __forceinline__ float warp_max(float v) {
 // ------------------------------------------------------------------------------------------ cu_seqlens
 // Exclusive scan of B lengths into int32 cu_seqlens[B+1] (one block; B is a batch size, at most a few thousand).
 __global__ void cu_seqlens_kernel(const int* __restrict__ lens, int B, int* __restrict__ cu) {
+  grid_dependency_wait();  // launched with programmatic dependent launch: nothing global before this
+  grid_launch_dependents();
   __shared__ int warp_tot[32];
   __shared__ int carry;
   if (threadIdx.x == 0) { carry = 0; cu[0] = 0; }
@@ -116,6 +118,8 @@ pack_rows_kernel(const uint4* __restrict__ src, const long long* __restrict__ sr
                  const int* __restrict__ cu, int B, long long dst_rows, int Lmax, int vec_per_row,
                  uint4* __restrict__ dst, long long* __restrict__ mask, long long* __restrict__ src_row_out,
                  const uint4* __restrict__ src2 = nullptr) {
+  grid_dependency_wait();  // launched with programmatic dependent launch: nothing global before this
+  grid_launch_dependents();
   __shared__ int s_cu[kPackMaxStagedSeqs + 1];
   __shared__ long long s_start[kPackMaxStagedSeqs];
   const bool staged = B <= kPackMaxStagedSeqs;
@@ -565,6 +569,8 @@ norm_mse_bwd_kernel(const __nv_bfloat16* __restrict__ h2, const float* __restric
                     const long long* __restrict__ t_row_index, int M, int D, int rows_per_cta, float dy_coef,
                     __nv_bfloat16* __restrict__ dh2, float* __restrict__ dg_part, float* __restrict__ db2_part,
                     float* __restrict__ loss_part) {
+  grid_dependency_wait();  // launched with programmatic dependent launch: nothing global before this
+  grid_launch_dependents();
   constexpr int R = kNormBwdRows;
   constexpr int PF = T_BF16 ? 2 : 1;  // iterations of loads in flight beyond the one being computed
   constexpr int NB = PF + 1;
@@ -740,6 +746,8 @@ struct FinishParams {
 
 __global__ void __launch_bounds__(256)
 finish_kernel(const FinishParams f) {
+  grid_dependency_wait();  // launched with programmatic dependent launch: nothing global before this
+  grid_launch_dependents();
   __shared__ float red[8][33];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   if (int(blockIdx.y) == f.njobs) {  // the loss job
@@ -921,6 +929,8 @@ masked_mse_kernel(const void* __restrict__ y_in, const void* __restrict__ t_in, 
 // loss = sum(part[0..P)) * (use_nd ? 1 / (n_valid * D) : 1 / n_valid); NaN when n_valid == 0 (as torch)
 __global__ void loss_finish_kernel(const float* __restrict__ part, int P, const float* __restrict__ meta, float d_or_1,
                                    float* __restrict__ loss, float n_valid_if_no_meta = 0.f) {
+  grid_dependency_wait();  // launched with programmatic dependent launch: nothing global before this
+  grid_launch_dependents();
   __shared__ float wsum[32];
   float acc = 0.f;
   for (int i = threadIdx.x; i < P; i += blockDim.x) acc += part[i];

@@ -58,6 +58,25 @@ inline int grid_for_rows(long long rows, int rows_per_block, int blocks_per_sm) 
   return int(want < cap ? (want > 0 ? want : 1) : cap);
 }
 
+// Launch configuration with programmatic dependent launch, for the row kernels that sit between the GEMMs on the train step's
+// compute stream (cu_seqlens, pack, norm_mse_bwd, loss_finish, finish). Each of them calls grid_dependency_wait() before it
+// touches global memory, as the GEMM kernel does.
+struct PdlConfig {
+  cudaLaunchAttribute attr;
+  cudaLaunchConfig_t cfg;
+  PdlConfig(dim3 grid, dim3 block, cudaStream_t st) {
+    memset(&cfg, 0, sizeof(cfg));
+    cfg.gridDim = grid;
+    cfg.blockDim = block;
+    cfg.stream = st;
+    attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr.val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = &attr;
+    cfg.numAttrs = 1;
+  }
+  PdlConfig(const PdlConfig&) = delete;  // cfg points at attr
+};
+
 inline int norm_bwd_grid(long long M, int* rows_per_cta) {
   // one slab of rows per CTA, a multiple of the R rows it walks at a time
   int ctas = device_sm_count() * 2;
@@ -148,8 +167,8 @@ int32_t td_profile_timeline(char* buf, int32_t buflen) {
 int32_t td_cu_seqlens(const int32_t* lens, int32_t B, int32_t* cu, td_stream_t stream) {
   TD_DEVICE_OR_RETURN();
   if (B < 0 || !cu || (B > 0 && !lens)) TD_FAIL(TD_ERR_ARG, "td_cu_seqlens: bad arguments");
-  cu_seqlens_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(lens, B, cu);
-  TD_CUDA(cudaGetLastError());
+  PdlConfig l(1, 1024, (cudaStream_t)stream);
+  TD_CUDA(cudaLaunchKernelEx(&l.cfg, cu_seqlens_kernel, lens, B, cu));
   return TD_OK;
 }
 
@@ -173,11 +192,11 @@ int32_t td_pack_varlen_indexed(const void* src, const int64_t* src_row_start, co
   const int grid = grid_for_rows(total_rows, 8, 8);
   {
     ProfScope prof("pack_varlen", 2.0 * double(total_rows) * double(row_bytes), (cudaStream_t)stream);
-    pack_rows_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>(
-        static_cast<const uint4*>(src), reinterpret_cast<const long long*>(src_row_start), cu, B, total_rows, 0,
-        int(row_bytes / 16), static_cast<uint4*>(dst), nullptr, reinterpret_cast<long long*>(src_row_out));
+    PdlConfig l(grid, 256, (cudaStream_t)stream);
+    TD_CUDA(cudaLaunchKernelEx(&l.cfg, pack_rows_kernel<false>, static_cast<const uint4*>(src),
+                               reinterpret_cast<const long long*>(src_row_start), cu, B, total_rows, 0, int(row_bytes / 16),
+                               static_cast<uint4*>(dst), nullptr, reinterpret_cast<long long*>(src_row_out), nullptr));
   }
-  TD_CUDA(cudaGetLastError());
   return TD_OK;
 }
 
@@ -193,11 +212,11 @@ int32_t td_pack_varlen2(const void* src, const void* src2, const int64_t* src_ro
   const int grid = grid_for_rows(total_rows, 8, 8);
   {
     ProfScope prof("pack_varlen", 2.0 * double(total_rows) * double(row_bytes), (cudaStream_t)stream);
-    pack_rows_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>(
-        static_cast<const uint4*>(src), reinterpret_cast<const long long*>(src_row_start), cu, B, total_rows, 0,
-        int(row_bytes / 16), static_cast<uint4*>(dst), nullptr, nullptr, static_cast<const uint4*>(src2));
+    PdlConfig l(grid, 256, (cudaStream_t)stream);
+    TD_CUDA(cudaLaunchKernelEx(&l.cfg, pack_rows_kernel<false>, static_cast<const uint4*>(src),
+                               reinterpret_cast<const long long*>(src_row_start), cu, B, total_rows, 0, int(row_bytes / 16),
+                               static_cast<uint4*>(dst), nullptr, nullptr, static_cast<const uint4*>(src2)));
   }
-  TD_CUDA(cudaGetLastError());
   return TD_OK;
 }
 
@@ -214,11 +233,11 @@ int32_t td_pack_padded(const void* src, const int64_t* src_row_start, const int3
   const int grid = grid_for_rows(rows, 8, 8);
   {
     ProfScope prof("pack_padded", 2.0 * double(rows) * double(row_bytes), (cudaStream_t)stream);
-    pack_rows_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>(
-        static_cast<const uint4*>(src), reinterpret_cast<const long long*>(src_row_start), cu, B, rows, L_max,
-        int(row_bytes / 16), static_cast<uint4*>(dst), reinterpret_cast<long long*>(mask), nullptr);
+    PdlConfig l(grid, 256, (cudaStream_t)stream);
+    TD_CUDA(cudaLaunchKernelEx(&l.cfg, pack_rows_kernel<true>, static_cast<const uint4*>(src),
+                               reinterpret_cast<const long long*>(src_row_start), cu, B, rows, L_max, int(row_bytes / 16),
+                               static_cast<uint4*>(dst), reinterpret_cast<long long*>(mask), nullptr, nullptr));
   }
-  TD_CUDA(cudaGetLastError());
   return TD_OK;
 }
 
@@ -556,8 +575,8 @@ int bwd_from_dh2(const __nv_bfloat16* dh2, const void* x, const void* h0, const 
       f.n_post = sc->n_post; f.post_base = sc->post_base; f.post_numel = sc->post_numel;
     }
     if (f.njobs > 0 || f.loss_out != nullptr) {
-      finish_kernel<<<dim3((D + 31) / 32, f.njobs + (f.loss_out ? 1 : 0)), 256, 0, st>>>(f);
-      TD_CUDA(cudaGetLastError());
+      PdlConfig l(dim3((D + 31) / 32, f.njobs + (f.loss_out ? 1 : 0)), 256, st);
+      TD_CUDA(cudaLaunchKernelEx(&l.cfg, finish_kernel, f));
     }
   }
   if (phases & (TD_BWD_PHASE_GELU_W1 | TD_BWD_PHASE_W1_ONLY)) {
@@ -670,17 +689,15 @@ int32_t td_aligner_mse_fwd(const void* x, int64_t M, int32_t Din, int32_t D, con
   const long long* tri = reinterpret_cast<const long long*>(target_row_index);
   {
     ProfScope prof("norm_mse_bwd_fused", double(M) * D * (4.0 + (target_dtype == TD_DTYPE_BF16 ? 2.0 : 4.0)), st);
-    if (target_dtype == TD_DTYPE_BF16)
-      norm_mse_bwd_kernel<true><<<np.grid, kNormBwdThreads, 0, st>>>(h2, w.ssq_part, nparts, eps, g, target, tri, int(M), D, np.rows_per_cta,
-                                                                     dy_coef, static_cast<__nv_bfloat16*>(dh2), np.dg_part, np.db_part, np.loss_part);
-    else
-      norm_mse_bwd_kernel<false><<<np.grid, kNormBwdThreads, 0, st>>>(h2, w.ssq_part, nparts, eps, g, target, tri, int(M), D, np.rows_per_cta,
-                                                                      dy_coef, static_cast<__nv_bfloat16*>(dh2), np.dg_part, np.db_part, np.loss_part);
+    PdlConfig l(np.grid, kNormBwdThreads, st);
+    TD_CUDA(cudaLaunchKernelEx(&l.cfg, target_dtype == TD_DTYPE_BF16 ? norm_mse_bwd_kernel<true> : norm_mse_bwd_kernel<false>, h2,
+                               w.ssq_part, nparts, eps, g, target, tri, int(M), D, np.rows_per_cta, dy_coef,
+                               static_cast<__nv_bfloat16*>(dh2), np.dg_part, np.db_part, np.loss_part));
   }
-  TD_CUDA(cudaGetLastError());
   if (!(stages & TD_FWD_STAGE_DEFER_LOSS)) {
-    loss_finish_kernel<<<1, 256, 0, st>>>(np.loss_part, np.grid, nullptr, float(D), loss, float(M));
-    TD_CUDA(cudaGetLastError());
+    PdlConfig l(1, 256, st);
+    TD_CUDA(cudaLaunchKernelEx(&l.cfg, loss_finish_kernel, static_cast<const float*>(np.loss_part), np.grid,
+                               static_cast<const float*>(nullptr), float(D), loss, float(M)));
   }
   return TD_OK;
 }
