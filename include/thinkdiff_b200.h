@@ -318,6 +318,30 @@ int32_t td_t5_attention_bwd(const void* dout, int64_t lddo, const void* q, int64
                             int32_t n_dist, const void* o, int64_t ldo, const float* lse, void* dq, int64_t lddq, void* dk,
                             int64_t lddk, void* dv, int64_t lddv, void* workspace, int64_t workspace_bytes, td_stream_t stream);
 
+/* ---- SURVEY section 8 f-1: the frozen T5 decoder's feed-forward sublayer on PACKED rows ------------------------------------
+ * transformers' T5LayerFF with T5DenseGatedActDense (feed_forward_proj = "gated-gelu", Flan-T5), the model cast to bf16 and run
+ * under bf16 autocast with dropout off, rounded where HF materialises a bf16 tensor and accumulated in fp32:
+ *   rstd = rsqrt(mean(x^2) + eps)            xn = bf16(bf16(ln_w) * bf16(x * rstd))      (td_rmsnorm_fwd's bf16 rule)
+ *   a = bf16(xn . wi_0^T)   b = bf16(xn . wi_1^T)   g = bf16(bf16(gelu_new(a)) * b)   out = bf16(x + bf16(g . wo^T))
+ * gelu_new (tanh form) is evaluated once in fp32 from a. The backward gives the gradient to x only (the weights are frozen):
+ *   t = bf16(dy . wo)   d_b = bf16(t * bf16(gelu_new(a)))   d_a = bf16(bf16(t * b) * gelu_new'(a))   dxn = bf16([d_a|d_b] . [wi_0; wi_1])
+ *   dx = bf16(dy + rstd * ln_w * dxn - x * rstd^3 * mean(x * ln_w * dxn))
+ * x, out, dy, dx [M, d] bf16; ln_w [d] fp32; rstd [M] fp32 (written by the forward); wo [d, d_ff] bf16 (nn.Linear layout);
+ * wi [2 d_ff, d] bf16 holds wi_0 and wi_1 INTERLEAVED in blocks of 32 rows: rows [64k, 64k + 32) = wi_0 rows [32k, 32k + 32),
+ * rows [64k + 32, 64k + 64) = wi_1 rows [32k, 32k + 32). ab / d_ab [M, 2 d_ff] bf16 carry a / b (their gradients) in the same
+ * column order; gated [M, d_ff] bf16 is g. ab = NULL (inference) skips writing it; gated = NULL and d_ab = NULL keep them in the
+ * workspace. Every buffer is contiguous and 16-byte aligned. Needs d % 64 == 0, d <= 4096, d_ff % 32 == 0; M == 0 does nothing.
+ * Forward: 3 launches (norm, [wi_0; wi_1] GEMM with the gate in its epilogue, wo GEMM with the residual add in its epilogue);
+ * backward: 3 launches (dy . wo GEMM with the gate's backward in its epilogue, d_ab . wi GEMM, norm backward with the residual).
+ * Profiling tags: ffn_norm, gemm_ffn_gate, gemm_ffn_out, gemm_ffn_dgate, gemm_ffn_dx (2 M N K FLOPs each), ffn_norm_bwd (bytes). */
+int64_t td_t5_ffn_workspace_bytes(int64_t M, int32_t d, int32_t d_ff);
+int32_t td_t5_ffn_fwd(const void* x, int64_t M, int32_t d, int32_t d_ff, const float* ln_w, float eps, const void* wi, const void* wo,
+                      void* out, float* rstd, void* ab /* [M, 2 d_ff] or NULL */, void* gated /* [M, d_ff] or NULL */, void* workspace,
+                      int64_t workspace_bytes, td_stream_t stream);
+int32_t td_t5_ffn_bwd(const void* dy, const void* x, const float* rstd, const float* ln_w, const void* ab, const void* wi, const void* wo,
+                      int64_t M, int32_t d, int32_t d_ff, void* dx, void* d_ab /* [M, 2 d_ff] or NULL */, void* workspace,
+                      int64_t workspace_bytes, td_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -16,11 +16,12 @@ from .train_step import AlignerTrainStep, synthetic_lvlm_batch  # noqa: E402
 from .optim import DeviceGradScaler, FusedAdamW  # noqa: E402
 from .shards import EmbedShardReader, EmbedShardSet, EmbedShardWriter, convert_webdataset_shards, iter_webdataset_samples  # noqa: E402
 from .lr_schedule import LinearWarmupCosineLRScheduler, LinearWarmupStepLRScheduler, get_lr_scheduler_class  # noqa: E402
-from .t5 import t5_attention, t5_position_bias_by_distance  # noqa: E402
+from .t5 import T5FeedForwardWeights, t5_attention, t5_layer_ff, t5_position_bias_by_distance  # noqa: E402
 
 __all__ = [
     "ops", "ThinkDiffAligner", "build_vision_projector", "FUSED_TYPE", "masked_mse", "masked_cross_entropy", "lm_head_cross_entropy", "frozen_linear",
     "FlatBatch", "FlatCollater", "PackedBatch", "kept_lengths", "pack_batch", "pack_device", "compose_image_text", "AlignerTrainStep",
     "synthetic_lvlm_batch", "FusedAdamW", "DeviceGradScaler", "EmbedShardReader", "EmbedShardSet", "EmbedShardWriter", "convert_webdataset_shards", "iter_webdataset_samples", "LinearWarmupCosineLRScheduler",
-    "LinearWarmupStepLRScheduler", "get_lr_scheduler_class", "t5_attention", "t5_position_bias_by_distance",
+    "LinearWarmupStepLRScheduler", "get_lr_scheduler_class", "t5_attention", "t5_position_bias_by_distance", "t5_layer_ff",
+    "T5FeedForwardWeights",
 ]

@@ -271,12 +271,20 @@ int launch_gemm(GemmOperand a, GemmOperand b, GemmParams p, void* ws, cudaStream
   if (rc) return rc;
   rc = make_operand_map(&mb, b.ptr, p.N, p.K, b.ld, B_MN, kBlockN / CTAS);
   if (rc) return rc;
+  if (EPI == EPI_GATED && p.N % 64)
+    TD_FAIL(TD_ERR_UNSUPPORTED, "gated GEMM: N=%d must be a multiple of 64 (whole (a, b) pairs)", p.N);
+  // EPI_DGATED's output and aux are the interleaved [M, 2N] pair buffers; EPI_GATED's out1 is the contiguous [M, N / 2] product
+  const long long out_cols = EPI == EPI_DGATED ? 2ll * p.N : p.N;
   if (EPI != EPI_F32_SCATTER && p.out0 != nullptr) {
-    rc = make_epilogue_map(&mo0, p.out0, p.M, p.N, p.ld_out, EPI == EPI_F32);
+    rc = make_epilogue_map(&mo0, p.out0, p.M, out_cols, p.ld_out, EPI == EPI_F32);
     if (rc) return rc;
   }
   if (EPI == EPI_BIAS_GELU) {
     rc = make_epilogue_map(&mo1, p.out1, p.M, p.N, p.ld_out, false);
+    if (rc) return rc;
+  }
+  if (EPI == EPI_GATED) {
+    rc = make_epilogue_map(&mo1, p.out1, p.M, p.N / 2, p.N / 2, false);
     if (rc) return rc;
   }
   if (EPI == EPI_F32_SCATTER) {
@@ -287,8 +295,8 @@ int launch_gemm(GemmOperand a, GemmOperand b, GemmParams p, void* ws, cudaStream
       if (rc) return rc;
     }
   }
-  if (EPI == EPI_DGELU) {
-    rc = make_epilogue_map(&maux, p.aux0, p.M, p.N, p.ld_out, false);
+  if (EPI == EPI_DGELU || EPI == EPI_RESIDUAL || EPI == EPI_DGATED) {
+    rc = make_epilogue_map(&maux, p.aux0, p.M, out_cols, p.ld_out, false);
     if (rc) return rc;
   }
   p.num_m_blocks = (p.M + kBlockM * CTAS - 1) / (kBlockM * CTAS);

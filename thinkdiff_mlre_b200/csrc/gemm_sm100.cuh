@@ -48,6 +48,12 @@ enum EpiKind : int {
   // buffer in rank o's HBM mapped into this process (the TMA bulk stores then travel over NVLink), or local memory for
   // o == this rank. One fp32 tensor map per owner; the staging and the store are those of EPI_F32.
   EPI_F32_SCATTER = 5,
+  // T5 gated-GELU feed-forward (DESIGN.md section 7). The wi_0 / wi_1 rows are interleaved in blocks of 32 (t5.py), so an epilogue
+  // warp's chunks 2j / 2j + 1 are a matched (a, b) pair of 32 columns: pair k = accumulator columns [64k, 64k + 64).
+  EPI_GATED = 6,      // out0 = ab = bf16(acc) (optional); out1 [M, N / 2] = g = bf16(bf16(gelu_tanh(a)) * b), column 32k + i of pair k
+  EPI_DGATED = 7,     // acc = dy . wo, t = bf16(acc) [M, N]; aux0 = ab [M, 2N]; out0 = d_ab [M, 2N] with, for t column 32k + i,
+                      // d_a = bf16(bf16(t * b) * gelu_tanh'(a)) at column 64k + i and d_b = bf16(t * bf16(gelu_tanh(a))) at 64k + 32 + i
+  EPI_RESIDUAL = 8,   // out0 = bf16(aux0 + bf16(acc)): the residual add of a sublayer's output projection
 };
 constexpr int kMaxPeers = 8;
 
@@ -129,6 +135,9 @@ constexpr int kSkSlotFloats = kEpiWarps * kEpiChunks * 32 * 32;  // one CTA's 12
 // 64-byte rows with the 64-byte swizzle for bf16, 128-byte rows with the 128-byte swizzle for fp32.
 template <int EPI> struct EpiStage { static constexpr int kBytesPerWarp = 4096; };          // two 2 KB bf16 boxes
 template <> struct EpiStage<EPI_DGELU> { static constexpr int kBytesPerWarp = 6144; };      // + two aux boxes, one out box
+template <> struct EpiStage<EPI_RESIDUAL> { static constexpr int kBytesPerWarp = 6144; };   // the same layout (aux = x)
+// one (d_a, d_b) output pair + two (a, b) aux pairs: 96 KB for the 8 warps leaves 4 pipeline stages
+template <> struct EpiStage<EPI_DGATED> { static constexpr int kBytesPerWarp = 12288; };
 // fp32 output: two 4 KB boxes, so a warp converts chunk c + 1 while the bulk store of chunk c is still reading its box -- over
 // NVLink (scatter) that read is paced by the link, and a single box made the epilogue longer than the next tile's mainloop
 template <> struct EpiStage<EPI_F32> { static constexpr int kBytesPerWarp = 8192; };
@@ -312,19 +321,29 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, const CUtenso
     if (p.alpha_ptr != nullptr) alpha *= __ldg(p.alpha_ptr);
   }
 
-  // EPI_DGELU: the saved pre-activation h0 arrives by TMA, one 32 x 32 box per chunk, one box ahead of the math
-  uint8_t* aux_box = stage + 2048;  // boxes at +2048 and +4096; the output box is at +0
+  // EPI_DGELU: the saved pre-activation h0 arrives by TMA, one 32 x 32 box per chunk, one box ahead of the math (EPI_RESIDUAL: x).
+  // EPI_DGATED: the (a, b) box pair of chunk c, columns 2 col0 and 2 col0 + 32 of ab, at +4096 / +8192; the output pair is at +0.
+  constexpr bool kAux = EPI == EPI_DGELU || EPI == EPI_RESIDUAL || EPI == EPI_DGATED;
+  uint8_t* aux_box = stage + (EPI == EPI_DGATED ? 4096 : 2048);  // otherwise boxes at +2048 and +4096; the output box is at +0
   auto aux_request = [&](int c) {
     if (lane == 0) {
       const uint32_t b = st.aux_req & 1;
-      mbar_arrive_expect_tx(&aux_bar[b], 2048);
-      tma_load_2d(aux_box + b * 2048, map_aux, &aux_bar[b], ncol0 + c * 32, slab_row0);
+      if constexpr (EPI == EPI_DGATED) {
+        const int ab_col = 2 * (ncol0 + c * 32);
+        mbar_arrive_expect_tx(&aux_bar[b], 4096);
+        tma_load_2d(aux_box + b * 4096, map_aux, &aux_bar[b], ab_col, slab_row0);
+        tma_load_2d(aux_box + b * 4096 + 2048, map_aux, &aux_bar[b], ab_col + 32, slab_row0);
+      } else {
+        mbar_arrive_expect_tx(&aux_bar[b], 2048);
+        tma_load_2d(aux_box + b * 2048, map_aux, &aux_bar[b], ncol0 + c * 32, slab_row0);
+      }
     }
     st.aux_req++;
   };
-  if constexpr (EPI == EPI_DGELU) {
+  if constexpr (kAux) {
     if (ncol0 < p.N) aux_request(0);
   }
+  float gate[EPI == EPI_GATED ? 32 : 1];  // EPI_GATED: bf16(gelu_tanh(a)) of the last a chunk, for the b chunk that follows it
 
 #pragma unroll 1
   for (int c = 0; c < kEpiChunks; ++c) {
@@ -332,7 +351,7 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, const CUtenso
     if (col0 >= p.N) break;  // N % 32 == 0 is enforced on the host
     uint32_t v[32];
     tmem_ld_32x32(taddr + c * 32, v);
-    if constexpr (EPI == EPI_DGELU) {
+    if constexpr (kAux) {
       if (c + 1 < kEpiChunks && col0 + 32 < p.N) aux_request(c + 1);
     }
     tmem_ld_wait();
@@ -410,6 +429,116 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, const CUtenso
         }
       }
       p.red0[(long long)(m_slab * 4 + quarter) * p.N + col0 + lane] = colsum[0];
+    } else if constexpr (EPI == EPI_RESIDUAL) {
+      const uint32_t b = st.aux_use & 1;
+      mbar_wait(&aux_bar[b], (st.aux_use >> 1) & 1);
+      st.aux_use++;
+      uint4 outp[4];
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        float x[8];
+        uint32_t w[4];
+        unpack8(*reinterpret_cast<const uint4*>(aux_box + b * 2048 + box64_off(lane, q)), x);
+#pragma unroll
+        for (int j = 0; j < 8; j += 2) {
+          float f0 = __uint_as_float(v[q * 8 + j]), f1 = __uint_as_float(v[q * 8 + j + 1]);
+          bf16_round2(f0, f1);  // the projection's output is a bf16 tensor before the add
+          w[j >> 1] = pack_bf16x2(x[j] + f0, x[j + 1] + f1);
+        }
+        outp[q] = make_uint4(w[0], w[1], w[2], w[3]);
+      }
+      stage_acquire(lane, true);  // (also orders every lane's aux reads before the next request overwrites that box)
+#pragma unroll
+      for (int q = 0; q < 4; ++q) *reinterpret_cast<uint4*>(stage + box64_off(lane, q)) = outp[q];
+      stage_store(map_out0, stage, col0, slab_row0, lane);
+    } else if constexpr (EPI == EPI_DGATED) {
+      // Rows past M: their A rows and aux boxes are zero-filled, so every output is 0 (and the store clips them anyway).
+      const uint32_t b = st.aux_use & 1;
+      mbar_wait(&aux_bar[b], (st.aux_use >> 1) & 1);
+      st.aux_use++;
+      const uint8_t* a_box = aux_box + b * 4096;
+      uint4 out_a[4], out_b[4];
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        float av[8], bv[8];
+        uint32_t wa[4], wb[4];
+        unpack8(*reinterpret_cast<const uint4*>(a_box + box64_off(lane, q)), av);
+        unpack8(*reinterpret_cast<const uint4*>(a_box + 2048 + box64_off(lane, q)), bv);
+#pragma unroll
+        for (int j = 0; j < 8; j += 2) {
+          float t0 = __uint_as_float(v[q * 8 + j]), t1 = __uint_as_float(v[q * 8 + j + 1]);
+          bf16_round2(t0, t1);  // t = dL/dg, a bf16 tensor in autograd
+          float g0, g1;
+          const float d0 = gelu_tanh_grad(av[j], g0), d1 = gelu_tanh_grad(av[j + 1], g1);
+          bf16_round2(g0, g1);  // gelu(a) as the forward materialised it
+          wb[j >> 1] = pack_bf16x2(t0 * g0, t1 * g1);
+          float u0 = t0 * bv[j], u1 = t1 * bv[j + 1];
+          bf16_round2(u0, u1);  // dL/dgelu(a)
+          wa[j >> 1] = pack_bf16x2(u0 * d0, u1 * d1);
+        }
+        out_a[q] = make_uint4(wa[0], wa[1], wa[2], wa[3]);
+        out_b[q] = make_uint4(wb[0], wb[1], wb[2], wb[3]);
+      }
+      stage_acquire(lane, true);  // the previous pair's stores have read their boxes; orders the aux reads as above
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        *reinterpret_cast<uint4*>(stage + box64_off(lane, q)) = out_a[q];
+        *reinterpret_cast<uint4*>(stage + 2048 + box64_off(lane, q)) = out_b[q];
+      }
+      stage_store(map_out0, stage, 2 * col0, slab_row0, lane);
+      stage_store(map_out0, stage + 2048, 2 * col0 + 32, slab_row0, lane);
+    } else if constexpr (EPI == EPI_GATED) {
+      // chunk c even: a (wi_0 rows), keep bf16(gelu_tanh(a)); c odd: the matching b (wi_1 rows), emit g. N % 64 == 0 and
+      // ncol0 % 64 == 0, so an a chunk inside N is always followed by its b chunk.
+      const bool is_b = (c & 1) != 0;
+      uint4 o0[4];
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        uint32_t w0[4];
+#pragma unroll
+        for (int j = 0; j < 8; j += 2) w0[j >> 1] = pack_bf16x2(__uint_as_float(v[q * 8 + j]), __uint_as_float(v[q * 8 + j + 1]));
+        o0[q] = make_uint4(w0[0], w0[1], w0[2], w0[3]);
+      }
+      if (!is_b) {
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          float a[8];
+          unpack8(o0[q], a);
+#pragma unroll
+          for (int j = 0; j < 8; j += 2) {
+            float g0 = gelu_tanh(a[j]), g1 = gelu_tanh(a[j + 1]);
+            bf16_round2(g0, g1);
+            gate[q * 8 + j] = g0;
+            gate[q * 8 + j + 1] = g1;
+          }
+        }
+      }
+      if (p.out0 != nullptr) {  // inference skips saving a and b
+        uint8_t* box = stage + (st.box & 1) * 2048;
+        stage_acquire(lane, false);
+#pragma unroll
+        for (int q = 0; q < 4; ++q) *reinterpret_cast<uint4*>(box + box64_off(lane, q)) = o0[q];
+        stage_store(map_out0, box, col0, slab_row0, lane);
+        st.box++;
+      }
+      if (is_b) {
+        uint4 o1[4];
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          float b[8];
+          uint32_t w1[4];
+          unpack8(o0[q], b);
+#pragma unroll
+          for (int j = 0; j < 8; j += 2) w1[j >> 1] = pack_bf16x2(gate[q * 8 + j] * b[j], gate[q * 8 + j + 1] * b[j + 1]);
+          o1[q] = make_uint4(w1[0], w1[1], w1[2], w1[3]);
+        }
+        uint8_t* box = stage + (st.box & 1) * 2048;
+        stage_acquire(lane, false);
+#pragma unroll
+        for (int q = 0; q < 4; ++q) *reinterpret_cast<uint4*>(box + box64_off(lane, q)) = o1[q];
+        stage_store(map_out1, box, (col0 - 32) >> 1, slab_row0, lane);
+        st.box++;
+      }
     } else {
       // bias (bf16, same 32 columns for every thread of the warp -> broadcast loads)
       uint4 o0[4], o1[4];
@@ -523,8 +652,8 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
     tma_prefetch_desc(&tmap_b);
     if constexpr (EPI != EPI_F32_SCATTER) tma_prefetch_desc(&tmap_out0);
     else tma_prefetch_desc(&smaps.m[0]);
-    if constexpr (EPI == EPI_BIAS_GELU) tma_prefetch_desc(&tmap_out1);
-    if constexpr (EPI == EPI_DGELU) tma_prefetch_desc(&tmap_aux);
+    if constexpr (EPI == EPI_BIAS_GELU || EPI == EPI_GATED) tma_prefetch_desc(&tmap_out1);
+    if constexpr (EPI == EPI_DGELU || EPI == EPI_RESIDUAL || EPI == EPI_DGATED) tma_prefetch_desc(&tmap_aux);
     for (int s = 0; s < kStages; ++s) {
       mbar_init(&full_bar[s], 1);
       mbar_init(&empty_bar[s], 1);

@@ -349,6 +349,32 @@ __device__ __forceinline__ float gelu_grad_fast(float x) {
   return fmaf(x, pdf, cdf);
 }
 
+// gelu_new (transformers NewGELUActivation, T5's gated-gelu FFN): 0.5 x (1 + tanh u), u = sqrt(2/pi) (x + 0.044715 x^3). With
+// s = 0.5 (1 + tanh u) = 1 / (1 + e^{-2u}) this is x * s, and d/dx = s + x * 2 s (1 - s) u'. Both come from ONE exponential
+// e = e^{-2|u|} <= 1 and r = 1 / (1 + e): s = r for u >= 0, e r for u < 0, and s (1 - s) = e r^2 either way -- no cancellation and
+// no overflow at any x, |error| about 1e-7. (tanh.approx.f32 is only good to about 2^-11, close enough to half a bf16 ulp to flip
+// the rounding of the outputs.)
+__device__ __forceinline__ void gelu_tanh_gate(float x, float& s, float& ds) {
+  const float x2 = x * x;
+  const float u = 0.79788456080286535588f * fmaf(0.044715f * x2, x, x);
+  const float e = ex2_approx(-2.88539008177792681472f * fabsf(u));  // e^{-2|u|}
+  const float r = rcp_approx(1.0f + e);
+  s = u >= 0.f ? r : e * r;
+  ds = 2.0f * (e * r * r) * (0.79788456080286535588f * fmaf(3.0f * 0.044715f, x2, 1.0f));
+}
+__device__ __forceinline__ float gelu_tanh(float x) {
+  float s, ds;
+  gelu_tanh_gate(x, s, ds);
+  return x * s;
+}
+// Derivative of gelu_tanh at x; the value gelu_tanh(x) goes to `gelu` (the backward needs both).
+__device__ __forceinline__ float gelu_tanh_grad(float x, float& gelu) {
+  float s, ds;
+  gelu_tanh_gate(x, s, ds);
+  gelu = x * s;
+  return fmaf(x, ds, s);
+}
+
 // nn.GELU(approximate='none'): 0.5 x (1 + erf(x / sqrt 2)), and its derivative (libm-accurate forms).
 __device__ __forceinline__ float gelu_erf(float x) { return 0.5f * x * (1.0f + erff(x * 0.70710678118654752440f)); }
 __device__ __forceinline__ float gelu_erf_grad(float x) {

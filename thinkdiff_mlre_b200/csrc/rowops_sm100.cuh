@@ -274,14 +274,17 @@ rmsnorm_fwd_kernel(const __nv_bfloat16* __restrict__ h2, const float* __restrict
 //   dh2  = bf16( rstd * ghat - h2 * rstd^3 * s_r / D )
 //   dg_part[cta][col] += dy * h2 * rstd;  db2_part[cta][col] += dh2
 // Column sums stay in registers and are written once per CTA (deterministic two-level reduction).
+// RESIDUAL (a pre-norm sublayer with a frozen weight, T5LayerFF): dh2 = bf16(dres + rstd * ghat - h2 * rstd^3 * s_r / D), the
+// gradient that reaches the sublayer's input through the residual branch folded in; no dg / db2 partials.
 constexpr int kNormBwdThreads = 512;
 constexpr int kNormBwdRows = 2;
 
-template <bool DY_BF16>
+template <bool DY_BF16, bool RESIDUAL = false>
 __global__ void __launch_bounds__(kNormBwdThreads, 2)
 rmsnorm_bwd_kernel(const void* __restrict__ dy_in, const __nv_bfloat16* __restrict__ h2,
                    const float* __restrict__ rstd_in, const float* __restrict__ g, int M, int D, int rows_per_cta,
-                   __nv_bfloat16* __restrict__ dh2, float* __restrict__ dg_part, float* __restrict__ db2_part) {
+                   __nv_bfloat16* __restrict__ dh2, float* __restrict__ dg_part, float* __restrict__ db2_part,
+                   const __nv_bfloat16* __restrict__ dres = nullptr) {
   constexpr int R = kNormBwdRows;
   __shared__ float red[R][kNormBwdThreads / 32];
   __shared__ float tot[R];
@@ -346,11 +349,21 @@ rmsnorm_bwd_kernel(const void* __restrict__ dy_in, const __nv_bfloat16* __restri
         const float rstd = __ldg(rstd_in + row);
         const float c = tot[r] * inv_d * rstd * rstd * rstd;
         float o[8];
+        if constexpr (RESIDUAL) {
+          float rv[8];
+          const uint4 ru = ld_stream(reinterpret_cast<const uint4*>(dres + (long long)row * D) + t);
+          const uint32_t rw[4] = {ru.x, ru.y, ru.z, ru.w};
 #pragma unroll
-        for (int q = 0; q < 8; ++q) {
-          o[q] = bf16_round(rstd * gg[q] * dyv[r][q] - hv[r][q] * c);
-          adb[q] += o[q];
-          adg[q] = fmaf(dyv[r][q] * hv[r][q], rstd, adg[q]);
+          for (int q = 0; q < 4; ++q) { rv[2 * q] = bf16lo(rw[q]); rv[2 * q + 1] = bf16hi(rw[q]); }
+#pragma unroll
+          for (int q = 0; q < 8; ++q) o[q] = bf16_round(rv[q] + (rstd * gg[q] * dyv[r][q] - hv[r][q] * c));
+        } else {
+#pragma unroll
+          for (int q = 0; q < 8; ++q) {
+            o[q] = bf16_round(rstd * gg[q] * dyv[r][q] - hv[r][q] * c);
+            adb[q] += o[q];
+            adg[q] = fmaf(dyv[r][q] * hv[r][q], rstd, adg[q]);
+          }
         }
         st_stream(reinterpret_cast<uint4*>(dh2 + (long long)row * D) + t,
                   make_uint4(pack_bf16x2(o[0], o[1]), pack_bf16x2(o[2], o[3]), pack_bf16x2(o[4], o[5]),
@@ -360,7 +373,7 @@ rmsnorm_bwd_kernel(const void* __restrict__ dy_in, const __nv_bfloat16* __restri
     // `tot`/`red` are rewritten only after the next iteration's first __syncthreads(), which every thread
     // reaches after finishing its reads above.
   }
-  if (col_ok) {
+  if (!RESIDUAL && col_ok) {
     float4* pg = reinterpret_cast<float4*>(dg_part + (long long)blockIdx.x * D) + 2 * t;
     float4* pb = reinterpret_cast<float4*>(db2_part + (long long)blockIdx.x * D) + 2 * t;
     pg[0] = make_float4(adg[0], adg[1], adg[2], adg[3]);

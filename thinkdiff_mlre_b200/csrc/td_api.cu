@@ -258,21 +258,24 @@ int32_t td_cast_f32_to_bf16(const float* src, void* dst, int64_t n, td_stream_t 
 }
 
 // ------------------------------------------------------------------------------------------------ norm
+static int rmsnorm_fwd_launch(const void* x, const float* g, float eps, int64_t M, int32_t D, void* y, int32_t y_dtype,
+                              float* rstd, cudaStream_t st) {
+  const int grid = grid_for_rows(M, 8, 8);
+  if (y_dtype == TD_DTYPE_BF16)
+    rmsnorm_fwd_kernel<true><<<grid, 256, 0, st>>>(static_cast<const __nv_bfloat16*>(x), nullptr, 0, g, eps, int(M), D, y, rstd);
+  else
+    rmsnorm_fwd_kernel<false><<<grid, 256, 0, st>>>(static_cast<const __nv_bfloat16*>(x), nullptr, 0, g, eps, int(M), D, y, rstd);
+  TD_CUDA(cudaGetLastError());
+  return TD_OK;
+}
+
 int32_t td_rmsnorm_fwd(const void* x, const float* g, float eps, int64_t M, int32_t D, void* y, int32_t y_dtype,
                        float* rstd, td_stream_t stream) {
   TD_DEVICE_OR_RETURN();
   if (M < 0 || D <= 0 || D % 8 || D > 8 * 32 * kNormFwdMaxVec)
     TD_FAIL(TD_ERR_ARG, "td_rmsnorm_fwd: D=%d must be a positive multiple of 8, at most %d", D, 8 * 32 * kNormFwdMaxVec);
   if (M == 0) return TD_OK;
-  const int grid = grid_for_rows(M, 8, 8);
-  if (y_dtype == TD_DTYPE_BF16)
-    rmsnorm_fwd_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>(static_cast<const __nv_bfloat16*>(x), nullptr, 0, g,
-                                                                    eps, int(M), D, y, rstd);
-  else
-    rmsnorm_fwd_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>(static_cast<const __nv_bfloat16*>(x), nullptr, 0,
-                                                                     g, eps, int(M), D, y, rstd);
-  TD_CUDA(cudaGetLastError());
-  return TD_OK;
+  return rmsnorm_fwd_launch(x, g, eps, M, D, y, y_dtype, rstd, (cudaStream_t)stream);
 }
 
 int64_t td_rmsnorm_bwd_workspace_bytes(int64_t M, int32_t D) {
@@ -1334,6 +1337,119 @@ int32_t td_t5_attention_bwd(const void* dout, int64_t lddo, const void* q, int64
   rc = attn_launch(t5_attn_dkdv_kernel<false>, grid_k, kAttnThreads, smem_kv, st, c.p, "attn_bwd_dkdv", 4 * f);
   if (rc) return rc;
   return attn_launch(t5_attn_dq_kernel<false>, grid_q, kAttnThreads, smem_q, st, c.p, "attn_bwd_dq", 3 * f);
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------ T5 gated-GELU FFN (8 f-1)
+namespace {
+// Workspace of td_t5_ffn_fwd / _bwd: a [M, d] bf16 row buffer (xn forward, dxn backward), a [M, 2 d_ff] bf16 buffer (gated forward,
+// d_ab backward, each when the caller passes none) and the stream-K tail of the GEMMs, which run one after another on the stream.
+struct FfnWorkspace {
+  __nv_bfloat16* rows;
+  __nv_bfloat16* pairs;
+  void* sk;
+  size_t bytes;
+};
+FfnWorkspace carve_ffn(void* ws, int64_t M, int32_t d, int32_t d_ff) {
+  const size_t m = (size_t)(M > 0 ? M : 1);
+  Carver c(ws);
+  FfnWorkspace w;
+  w.rows = c.take<__nv_bfloat16>(m * (size_t)(d > 0 ? d : 1));
+  w.pairs = c.take<__nv_bfloat16>(m * 2 * (size_t)(d_ff > 0 ? d_ff : 1));
+  w.sk = c.take<uint8_t>(gemm_sk_workspace_bytes());
+  w.bytes = c.off;
+  return w;
+}
+
+int ffn_check_sizes(const char* fn, int64_t M, int32_t d, int32_t d_ff) {
+  if (M < 0 || d <= 0 || d_ff <= 0) TD_FAIL(TD_ERR_ARG, "%s: bad sizes (M=%lld d=%d d_ff=%d)", fn, (long long)M, d, d_ff);
+  if (d % 64 || d > 8 * kNormBwdThreads || d_ff % 32)
+    TD_FAIL(TD_ERR_UNSUPPORTED, "%s: need d %% 64 == 0, d <= %d and d_ff %% 32 == 0 (d=%d d_ff=%d)", fn, 8 * kNormBwdThreads, d, d_ff);
+  if (M > 0x7fffffffll / (2ll * d_ff)) TD_FAIL(TD_ERR_ARG, "%s: M=%lld out of range", fn, (long long)M);
+  return TD_OK;
+}
+int ffn_check_workspace(const char* fn, int64_t M, int32_t d, int32_t d_ff, void* ws, int64_t ws_bytes) {
+  if (!ws || ws_bytes < (int64_t)carve_ffn(nullptr, M, d, d_ff).bytes) TD_FAIL(TD_ERR_ARG, "%s: workspace too small", fn);
+  if (misaligned16(ws)) TD_FAIL(TD_ERR_ARG, "%s: the workspace must be 16-byte aligned", fn);
+  return TD_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int64_t td_t5_ffn_workspace_bytes(int64_t M, int32_t d, int32_t d_ff) { return (int64_t)carve_ffn(nullptr, M, d, d_ff).bytes; }
+
+int32_t td_t5_ffn_fwd(const void* x, int64_t M, int32_t d, int32_t d_ff, const float* ln_w, float eps, const void* wi, const void* wo,
+                      void* out, float* rstd, void* ab, void* gated, void* ws, int64_t ws_bytes, td_stream_t stream) {
+  TD_DEVICE_OR_RETURN();
+  int rc = ffn_check_sizes("td_t5_ffn_fwd", M, d, d_ff);
+  if (rc) return rc;
+  if (M == 0) return TD_OK;
+  rc = ffn_check_workspace("td_t5_ffn_fwd", M, d, d_ff, ws, ws_bytes);
+  if (rc) return rc;
+  if (!x || !ln_w || !wi || !wo || !out || !rstd) TD_FAIL(TD_ERR_ARG, "td_t5_ffn_fwd: null pointer");
+  if (misaligned16(x) || misaligned16(ln_w) || misaligned16(wi) || misaligned16(wo) || misaligned16(out) || misaligned16(ab) ||
+      misaligned16(gated))
+    TD_FAIL(TD_ERR_ARG, "td_t5_ffn_fwd: x / ln_w / wi / wo / out / ab / gated must be 16-byte aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  const FfnWorkspace w = carve_ffn(ws, M, d, d_ff);
+  __nv_bfloat16* xn = w.rows;
+  void* g = gated ? gated : w.pairs;
+  {
+    ProfScope prof("ffn_norm", double(M) * d * 4.0, st);
+    rc = rmsnorm_fwd_launch(x, ln_w, eps, M, d, xn, TD_DTYPE_BF16, rstd, st);
+  }
+  if (rc) return rc;
+  GemmParams p;
+  memset(&p, 0, sizeof(p));
+  p.M = int(M); p.N = 2 * d_ff; p.K = d;
+  p.out0 = ab; p.out1 = g; p.ld_out = 2 * d_ff; p.alpha = 1.f;
+  rc = launch_gemm<2, false, false, EPI_GATED>({xn, d, false}, {wi, d, false}, p, w.sk, st, "gemm_ffn_gate");
+  if (rc) return rc;
+  memset(&p, 0, sizeof(p));
+  p.M = int(M); p.N = d; p.K = d_ff;
+  p.out0 = out; p.aux0 = x; p.ld_out = d; p.alpha = 1.f;
+  return launch_gemm<2, false, false, EPI_RESIDUAL>({g, d_ff, false}, {wo, d_ff, false}, p, w.sk, st, "gemm_ffn_out");
+}
+
+int32_t td_t5_ffn_bwd(const void* dy, const void* x, const float* rstd, const float* ln_w, const void* ab, const void* wi, const void* wo,
+                      int64_t M, int32_t d, int32_t d_ff, void* dx, void* d_ab, void* ws, int64_t ws_bytes, td_stream_t stream) {
+  TD_DEVICE_OR_RETURN();
+  int rc = ffn_check_sizes("td_t5_ffn_bwd", M, d, d_ff);
+  if (rc) return rc;
+  if (M == 0) return TD_OK;
+  rc = ffn_check_workspace("td_t5_ffn_bwd", M, d, d_ff, ws, ws_bytes);
+  if (rc) return rc;
+  if (!dy || !x || !rstd || !ln_w || !ab || !wi || !wo || !dx) TD_FAIL(TD_ERR_ARG, "td_t5_ffn_bwd: null pointer");
+  if (misaligned16(dy) || misaligned16(x) || misaligned16(ab) || misaligned16(wi) || misaligned16(wo) || misaligned16(dx) ||
+      misaligned16(d_ab))
+    TD_FAIL(TD_ERR_ARG, "td_t5_ffn_bwd: dy / x / ab / wi / wo / dx / d_ab must be 16-byte aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  const FfnWorkspace w = carve_ffn(ws, M, d, d_ff);
+  void* dab = d_ab ? d_ab : w.pairs;
+  __nv_bfloat16* dxn = w.rows;
+  GemmParams p;
+  memset(&p, 0, sizeof(p));
+  p.M = int(M); p.N = d_ff; p.K = d;  // t = dy . wo, wo [d, d_ff] read MN-major in place
+  p.out0 = dab; p.aux0 = ab; p.ld_out = 2 * d_ff; p.alpha = 1.f;
+  rc = launch_gemm<2, false, true, EPI_DGATED>({dy, d, false}, {wo, d_ff, true}, p, w.sk, st, "gemm_ffn_dgate");
+  if (rc) return rc;
+  memset(&p, 0, sizeof(p));
+  p.M = int(M); p.N = d; p.K = 2 * d_ff;  // dxn = d_ab . wi, over the interleaved pair columns of both
+  p.out0 = dxn; p.ld_out = d; p.alpha = 1.f;
+  rc = launch_gemm<2, false, true, EPI_BF16>({dab, 2 * d_ff, false}, {wi, d, true}, p, w.sk, st, "gemm_ffn_dx");
+  if (rc) return rc;
+  int rpc;
+  const int grid = norm_bwd_grid(M, &rpc);
+  {
+    ProfScope prof("ffn_norm_bwd", double(M) * d * 8.0, st);
+    rmsnorm_bwd_kernel<true, true><<<grid, kNormBwdThreads, 0, st>>>(dxn, static_cast<const __nv_bfloat16*>(x), rstd, ln_w, int(M), d,
+                                                                     rpc, static_cast<__nv_bfloat16*>(dx), nullptr, nullptr,
+                                                                     static_cast<const __nv_bfloat16*>(dy));
+  }
+  TD_CUDA(cudaGetLastError());
+  return TD_OK;
 }
 
 }  // extern "C"

@@ -531,3 +531,61 @@ def t5_attention_bwd(dout, q, k, v, o, lse, cu_q, cu_k, max_len_q: int, max_len_
                                         L.ptr(dq), dq.stride(0), L.ptr(dk), dk.stride(0), L.ptr(dv), dv.stride(0), L.ptr(ws), ws_bytes,
                                         L.stream_ptr()), "td_t5_attention_bwd")
     return dq, dk, dv
+
+
+# ------------------------------------------------------------------------------------------------ T5 gated-GELU FFN (8 f-1)
+def _ffn_dims(x, wi, wo, ln_w):
+    _need_cuda(x, wi, wo, ln_w)
+    M, d = x.shape
+    d_ff = wo.shape[1]
+    if x.dtype != torch.bfloat16 or wi.dtype != torch.bfloat16 or wo.dtype != torch.bfloat16 or ln_w.dtype != torch.float32:
+        raise TypeError("t5_ffn: x, wi, wo must be bfloat16 and ln_w float32")
+    if tuple(wi.shape) != (2 * d_ff, d) or tuple(wo.shape) != (d, d_ff) or tuple(ln_w.shape) != (d,):
+        raise ValueError(f"t5_ffn: need wi [2 d_ff, d], wo [d, d_ff], ln_w [d]; got {tuple(wi.shape)}, {tuple(wo.shape)}, {tuple(ln_w.shape)}")
+    for t, n in ((x, "x"), (wi, "wi"), (wo, "wo"), (ln_w, "ln_w")):
+        _contig(t, n)
+    return M, d, d_ff
+
+
+def t5_ffn_fwd(x, wi, wo, ln_w, eps: float, want_ab: bool = True, want_gated: bool = False):
+    """T5LayerFF (gated-GELU) forward on packed rows: ``x [M, d]`` bf16, ``wi [2 d_ff, d]`` bf16 with wi_0 / wi_1 interleaved in
+    blocks of 32 rows (``t5.T5FeedForwardWeights``), ``wo [d, d_ff]`` bf16, ``ln_w [d]`` fp32. Returns ``(out [M, d] bf16, rstd [M]
+    fp32, ab [M, 2 d_ff] bf16 or None, gated [M, d_ff] bf16 or None)``: ``ab`` (a / b in wi's interleaved column order) is what the
+    backward needs; ``want_ab=False`` is the inference path. Three launches."""
+    M, d, d_ff = _ffn_dims(x, wi, wo, ln_w)
+    dev = x.device
+    out = torch.empty((M, d), dtype=torch.bfloat16, device=dev)
+    rstd = torch.empty((M,), dtype=torch.float32, device=dev)
+    ab = torch.empty((M, 2 * d_ff), dtype=torch.bfloat16, device=dev) if want_ab else None
+    gated = torch.empty((M, d_ff), dtype=torch.bfloat16, device=dev) if want_gated else None
+    ws_bytes = L.lib().td_t5_ffn_workspace_bytes(M, d, d_ff)
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+    L.launch_count += 3
+    L.check(L.lib().td_t5_ffn_fwd(L.ptr(x), M, d, d_ff, L.ptr(ln_w), eps, L.ptr(wi), L.ptr(wo), L.ptr(out), L.ptr(rstd), L.ptr(ab),
+                                  L.ptr(gated), L.ptr(ws), ws_bytes, L.stream_ptr()), "td_t5_ffn_fwd")
+    return out, rstd, ab, gated
+
+
+def t5_ffn_bwd(dy, x, rstd, ab, wi, wo, ln_w, want_d_ab: bool = False):
+    """Input gradient of ``t5_ffn_fwd`` (frozen weights): ``dy [M, d]`` bf16 and the forward's ``x``, ``rstd``, ``ab``. Returns
+    ``(dx [M, d] bf16, d_ab [M, 2 d_ff] bf16 or None)``; ``d_ab`` holds dL/da and dL/db in wi's interleaved column order. Three
+    launches; deterministic."""
+    M, d, d_ff = _ffn_dims(x, wi, wo, ln_w)
+    _need_cuda(dy, rstd, ab)
+    if dy.dtype != torch.bfloat16 or tuple(dy.shape) != (M, d):
+        raise TypeError(f"t5_ffn_bwd: dy must be bfloat16 [{M}, {d}]")
+    if ab is None or ab.dtype != torch.bfloat16 or tuple(ab.shape) != (M, 2 * d_ff):
+        raise TypeError(f"t5_ffn_bwd: ab must be the forward's bfloat16 [{M}, {2 * d_ff}] (run it with want_ab=True)")
+    if rstd.dtype != torch.float32 or rstd.numel() != M:
+        raise TypeError(f"t5_ffn_bwd: rstd must be float32 [{M}]")
+    for t, n in ((dy, "dy"), (ab, "ab"), (rstd, "rstd")):
+        _contig(t, n)
+    dev = x.device
+    dx = torch.empty((M, d), dtype=torch.bfloat16, device=dev)
+    d_ab = torch.empty((M, 2 * d_ff), dtype=torch.bfloat16, device=dev) if want_d_ab else None
+    ws_bytes = L.lib().td_t5_ffn_workspace_bytes(M, d, d_ff)
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+    L.launch_count += 3
+    L.check(L.lib().td_t5_ffn_bwd(L.ptr(dy), L.ptr(x), L.ptr(rstd), L.ptr(ln_w), L.ptr(ab), L.ptr(wi), L.ptr(wo), M, d, d_ff, L.ptr(dx),
+                                  L.ptr(d_ab), L.ptr(ws), ws_bytes, L.stream_ptr()), "td_t5_ffn_bwd")
+    return dx, d_ab
