@@ -342,6 +342,53 @@ int32_t td_t5_ffn_bwd(const void* dy, const void* x, const float* rstd, const fl
                       int64_t M, int32_t d, int32_t d_ff, void* dx, void* d_ab /* [M, 2 d_ff] or NULL */, void* workspace,
                       int64_t workspace_bytes, td_stream_t stream);
 
+/* ---- SURVEY section 8 f-1: the frozen T5 decoder's two attention sublayers on PACKED rows ------------------------------------
+ * transformers' T5LayerSelfAttention and T5LayerCrossAttention (pre-norm, attention, o projection, residual; dropout off), the
+ * model cast to bf16 and run under bf16 autocast, rounded where HF materialises a bf16 tensor and accumulated in fp32. inner = 64 H
+ * (d_kv = 64, the attention kernel's rule); the norm is the FFN's: rstd = rsqrt(mean(x^2) + eps), xn = bf16(bf16(ln_w) * bf16(x * rstd)).
+ *   self : qkv = bf16(xn . [Wq; Wk; Wv]^T) [M, 3 inner] (one GEMM)    o = attention(q, k, v), causal, bias_by_distance [H, n_dist]
+ *   cross: q = bf16(xn . Wq^T) [M, inner]   kv = bf16(enc . [Wk; Wv]^T) [Mk, 2 inner]   o = attention(q, k, v) over the aligner rows
+ *   both : out = bf16(x + bf16(o . Wo^T))
+ * q / k / v are read in place as column slices of qkv / kv (td_t5_attention_fwd). The backward gives the gradient to x, and for
+ * cross-attention to enc (the weights are frozen):
+ *   d_o = bf16(dy . Wo)   dq | dk | dv from the attention backward (bf16, written into one [M, 3 inner] / [Mk, 2 inner] buffer)
+ *   self : dxn = bf16(dqkv . [Wq; Wk; Wv])                 cross: dxn = bf16(dq . Wq)   d_enc = dkv . [Wk; Wv]   (fp32, overwritten)
+ *   dx = bf16(dy + rstd * ln_w * dxn - x * rstd^3 * mean(x * ln_w * dxn))
+ * d_enc deviates from HF on purpose: HF rounds dk . Wk and dv . Wv to bf16 separately and sums them in fp32; here one GEMM sums both
+ * in fp32 and never rounds, which is closer to fp32.
+ * x, out, dy, dx [M, d] bf16 (decoder rows, samples cu_q[b]..cu_q[b+1], cu_q[B] == M); enc [Mk, d] bf16 (aligner rows, cu_k[b]..
+ * cu_k[b+1], cu_k[B] == Mk); ln_w [d] fp32; w_qkv [3 inner, d], w_q [inner, d], w_kv [2 inner, d], wo [d, inner] bf16 (nn.Linear
+ * layout, Wq / Wk / Wv stacked by rows). max_len_* are host-known bounds of the samples' lengths, as for td_t5_attention_fwd.
+ * Forward intermediates the backward takes back: rstd [M] fp32, qkv [M, 3 inner] or q [M, inner] and kv [Mk, 2 inner], o [M, inner]
+ * bf16 and lse [H, Mq] fp32. Each of them may be NULL in the forward, which then keeps it in the workspace: with lse = NULL (inference)
+ * nothing beyond out needs to be kept. dqkv [M, 3 inner] (or NULL) receives the self-attention's dq | dk | dv. A cross sample with no
+ * aligner rows gets o = 0, so out = x exactly, and contributes no d_enc. Every buffer is 16-byte aligned; d % 64 == 0, d <= 4096,
+ * H >= 1; M == 0 does nothing. One workspace size serves the forward and the backward (self_attention = 1: Mk is ignored).
+ * Launches: self forward 4 (norm, QKV GEMM, attention, o GEMM with the residual in its epilogue), self backward 6 (d_o GEMM, three
+ * attention-backward launches, dxn GEMM, norm backward with the residual); cross forward 5 (norm, q GEMM, kv GEMM, attention, o GEMM),
+ * cross backward 7 (d_o GEMM, three attention-backward launches, dxn GEMM, fp32 d_enc GEMM, norm backward).
+ * Profiling tags: sa_norm, gemm_sa_qkv, gemm_sa_out, gemm_sa_do, gemm_sa_dx, sa_norm_bwd, ca_norm, gemm_ca_q, gemm_ca_kv, gemm_ca_out,
+ * gemm_ca_do, gemm_ca_dq, gemm_ca_denc, ca_norm_bwd; the attention launches keep attn_fwd / attn_bwd_*. */
+int64_t td_t5_attention_layer_workspace_bytes(int64_t M, int64_t Mk, int32_t d, int32_t H, int32_t self_attention);
+int32_t td_t5_self_attention_layer_fwd(const void* x, int64_t M, int32_t d, int32_t H, const int32_t* cu_q, int32_t B, int32_t max_len,
+                                       const float* ln_w, float eps, const void* w_qkv, const void* wo, const float* bias_by_distance,
+                                       int32_t n_dist, void* out, float* rstd /* or NULL */, void* qkv /* or NULL */, void* o /* or NULL */,
+                                       float* lse /* or NULL */, void* workspace, int64_t workspace_bytes, td_stream_t stream);
+int32_t td_t5_self_attention_layer_bwd(const void* dy, const void* x, const float* rstd, const float* ln_w, const void* qkv, const void* o,
+                                       const float* lse, const void* w_qkv, const void* wo, const float* bias_by_distance, int32_t n_dist,
+                                       const int32_t* cu_q, int32_t B, int32_t max_len, int64_t M, int32_t d, int32_t H, void* dx,
+                                       void* dqkv /* or NULL */, void* workspace, int64_t workspace_bytes, td_stream_t stream);
+int32_t td_t5_cross_attention_layer_fwd(const void* x, int64_t M, const void* enc, int64_t Mk, int32_t d, int32_t H, const int32_t* cu_q,
+                                        const int32_t* cu_k, int32_t B, int32_t max_len_q, int32_t max_len_k, const float* ln_w, float eps,
+                                        const void* w_q, const void* w_kv, const void* wo, void* out, float* rstd /* or NULL */,
+                                        void* q /* or NULL */, void* kv /* or NULL */, void* o /* or NULL */, float* lse /* or NULL */,
+                                        void* workspace, int64_t workspace_bytes, td_stream_t stream);
+int32_t td_t5_cross_attention_layer_bwd(const void* dy, const void* x, const float* rstd, const float* ln_w, const void* q, const void* kv,
+                                        const void* o, const float* lse, const void* w_q, const void* w_kv, const void* wo, const int32_t* cu_q,
+                                        const int32_t* cu_k, int32_t B, int32_t max_len_q, int32_t max_len_k, int64_t M, int64_t Mk, int32_t d,
+                                        int32_t H, void* dx, float* d_enc /* [Mk, d] fp32 */, void* workspace, int64_t workspace_bytes,
+                                        td_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -55,6 +55,15 @@ SIGNATURES = {
     "td_t5_ffn_workspace_bytes": (_i64, [_i64, _i32, _i32]),
     "td_t5_ffn_fwd": (_i32, [_vp, _i64, _i32, _i32, _vp, _f32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
     "td_t5_ffn_bwd": (_i32, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp, _i64, _vp]),
+    "td_t5_attention_layer_workspace_bytes": (_i64, [_i64, _i64, _i32, _i32, _i32]),
+    "td_t5_self_attention_layer_fwd": (_i32, [_vp, _i64, _i32, _i32, _vp, _i32, _i32, _vp, _f32, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp,
+                                              _vp, _i64, _vp]),
+    "td_t5_self_attention_layer_bwd": (_i32, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _i32, _i32, _i64, _i32, _i32, _vp,
+                                              _vp, _vp, _i64, _vp]),
+    "td_t5_cross_attention_layer_fwd": (_i32, [_vp, _i64, _vp, _i64, _i32, _i32, _vp, _vp, _i32, _i32, _i32, _vp, _f32, _vp, _vp, _vp, _vp, _vp,
+                                               _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
+    "td_t5_cross_attention_layer_bwd": (_i32, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i64, _i64,
+                                               _i32, _i32, _vp, _vp, _vp, _i64, _vp]),
     "td_gemm_bf16_f32out": (_i32, [_vp, _i64, _i32, _vp, _i64, _i32, _i64, _i32, _i64, _f32, _vp, _i32, _i32, _vp, _i64, _vp]),
     "td_adamw_step": (_i32, [_i32, _vp, _vp, _vp, _vp, _vp, C.POINTER(_i64), C.POINTER(_f32), _f32, _f32, _f32, _f32, _i64, _f32, _vp, _vp]),
     "td_step_ctl_bytes": (_i64, []),

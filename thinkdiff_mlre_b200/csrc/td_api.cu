@@ -1374,6 +1374,22 @@ int ffn_check_workspace(const char* fn, int64_t M, int32_t d, int32_t d_ff, void
   if (misaligned16(ws)) TD_FAIL(TD_ERR_ARG, "%s: the workspace must be 16-byte aligned", fn);
   return TD_OK;
 }
+
+// dx = bf16(dy + norm_bwd(dxn)): the backward of a T5 pre-norm sublayer's RMSNorm with the residual gradient folded in, one launch.
+// Shared by the FFN and both attention sublayers; ln_w is frozen, so no weight-gradient partials are formed.
+int residual_norm_bwd_launch(const __nv_bfloat16* dxn, const void* x, const float* rstd, const float* ln_w, int64_t M, int32_t d,
+                             const void* dy, void* dx, const char* tag, cudaStream_t st) {
+  int rpc;
+  const int grid = norm_bwd_grid(M, &rpc);
+  {
+    ProfScope prof(tag, double(M) * d * 8.0, st);
+    rmsnorm_bwd_kernel<true, true><<<grid, kNormBwdThreads, 0, st>>>(dxn, static_cast<const __nv_bfloat16*>(x), rstd, ln_w, int(M), d,
+                                                                     rpc, static_cast<__nv_bfloat16*>(dx), nullptr, nullptr,
+                                                                     static_cast<const __nv_bfloat16*>(dy));
+  }
+  TD_CUDA(cudaGetLastError());
+  return TD_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -1440,16 +1456,230 @@ int32_t td_t5_ffn_bwd(const void* dy, const void* x, const float* rstd, const fl
   p.out0 = dxn; p.ld_out = d; p.alpha = 1.f;
   rc = launch_gemm<2, false, true, EPI_BF16>({dab, 2 * d_ff, false}, {wi, d, true}, p, w.sk, st, "gemm_ffn_dx");
   if (rc) return rc;
-  int rpc;
-  const int grid = norm_bwd_grid(M, &rpc);
-  {
-    ProfScope prof("ffn_norm_bwd", double(M) * d * 8.0, st);
-    rmsnorm_bwd_kernel<true, true><<<grid, kNormBwdThreads, 0, st>>>(dxn, static_cast<const __nv_bfloat16*>(x), rstd, ln_w, int(M), d,
-                                                                     rpc, static_cast<__nv_bfloat16*>(dx), nullptr, nullptr,
-                                                                     static_cast<const __nv_bfloat16*>(dy));
-  }
-  TD_CUDA(cudaGetLastError());
+  return residual_norm_bwd_launch(dxn, x, rstd, ln_w, M, d, dy, dx, "ffn_norm_bwd", st);
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------ T5 attention sublayers (8 f-1)
+namespace {
+// Workspace of td_t5_{self,cross}_attention_layer_fwd / _bwd; every buffer serves the forward and then the backward:
+//   rows  [M, d] bf16             xn / dxn
+//   proj  [M, 3 inner] bf16       qkv / dqkv (self; when the caller passes none), or [Mk, 2 inner] kv / dkv (cross; kv when none given)
+//   q     [M, inner] bf16         cross only: q (when none given) / dq
+//   heads [M, inner] bf16         o (when none given) / d_o
+//   rstd  [M] fp32                when the caller passes none
+//   delta [H, M] fp32             the attention backward's row sums (td_t5_attention_workspace_bytes)
+// and the stream-K tail of the GEMMs, which run one after another on the stream.
+struct AttnLayerWorkspace {
+  __nv_bfloat16 *rows, *proj, *q, *heads;
+  float *rstd, *delta;
+  int64_t delta_bytes;
+  void* sk;
+  size_t bytes;
+};
+AttnLayerWorkspace carve_attn_layer(void* ws, int64_t M, int64_t Mk, int32_t d, int32_t H, bool self_attention) {
+  const size_t m = (size_t)(M > 0 ? M : 1), mk = (size_t)(Mk > 0 ? Mk : 1), dd = (size_t)(d > 0 ? d : 1);
+  const size_t inner = (size_t)kAttnDk * (H > 0 ? H : 1);
+  Carver c(ws);
+  AttnLayerWorkspace w;
+  w.rows = c.take<__nv_bfloat16>(m * dd);
+  w.proj = c.take<__nv_bfloat16>(self_attention ? m * 3 * inner : mk * 2 * inner);
+  w.q = self_attention ? nullptr : c.take<__nv_bfloat16>(m * inner);
+  w.heads = c.take<__nv_bfloat16>(m * inner);
+  w.rstd = c.take<float>(m);
+  w.delta_bytes = td_t5_attention_workspace_bytes(M, H);
+  w.delta = c.take<float>((size_t)w.delta_bytes / sizeof(float));
+  w.sk = c.take<uint8_t>(gemm_sk_workspace_bytes());
+  w.bytes = c.off;
+  return w;
+}
+
+int attn_layer_check(const char* fn, int64_t M, int64_t Mk, int32_t d, int32_t H, bool self_attention, void* ws, int64_t ws_bytes) {
+  if (M < 0 || Mk < 0 || d <= 0 || H <= 0 || H > 65535)
+    TD_FAIL(TD_ERR_ARG, "%s: bad sizes (M=%lld Mk=%lld d=%d H=%d)", fn, (long long)M, (long long)Mk, d, H);
+  if (d % 64 || d > 8 * kNormBwdThreads) TD_FAIL(TD_ERR_UNSUPPORTED, "%s: need d %% 64 == 0 and d <= %d (d=%d)", fn, 8 * kNormBwdThreads, d);
+  const long long widest = 3ll * kAttnDk * H > d ? 3ll * kAttnDk * H : (long long)d;
+  if (M > 0x7fffffffll / widest || Mk > 0x7fffffffll / widest)
+    TD_FAIL(TD_ERR_ARG, "%s: M=%lld / Mk=%lld out of range", fn, (long long)M, (long long)Mk);
+  if (M == 0) return TD_OK;
+  if (!ws || ws_bytes < (int64_t)carve_attn_layer(nullptr, M, Mk, d, H, self_attention).bytes)
+    TD_FAIL(TD_ERR_ARG, "%s: workspace too small", fn);
+  if (misaligned16(ws)) TD_FAIL(TD_ERR_ARG, "%s: the workspace must be 16-byte aligned", fn);
   return TD_OK;
+}
+
+// out = bf16(x + bf16(o . wo^T)), o [M, inner], wo [d, inner]: the closing projection of both attention sublayers
+int attn_out_gemm(const void* o, int32_t inner, const void* wo, const void* x, void* out, int64_t M, int32_t d, void* sk, cudaStream_t st,
+                  const char* tag) {
+  GemmParams p;
+  memset(&p, 0, sizeof(p));
+  p.M = int(M); p.N = d; p.K = inner;
+  p.out0 = out; p.aux0 = x; p.ld_out = d; p.alpha = 1.f;
+  return launch_gemm<2, false, false, EPI_RESIDUAL>({o, inner, false}, {wo, inner, false}, p, sk, st, tag);
+}
+
+// out [M, N] bf16 = bf16(a . w^T), w [N, K] read K-major (a projection)
+int proj_gemm(const void* a, int64_t M, int32_t K, const void* w, int32_t N, void* out, void* sk, cudaStream_t st, const char* tag) {
+  GemmParams p;
+  memset(&p, 0, sizeof(p));
+  p.M = int(M); p.N = N; p.K = K;
+  p.out0 = out; p.ld_out = N; p.alpha = 1.f;
+  return launch_gemm<2, false, false, EPI_BF16>({a, K, false}, {w, K, false}, p, sk, st, tag);
+}
+
+// out [M, N] = dy . w, dy [M, K], w [K, N] read MN-major in place (the input gradient of a projection): bf16, or fp32 when `f32`
+int proj_dx_gemm(const void* dy, int64_t M, int32_t K, const void* w, int32_t N, void* out, bool f32, void* sk, cudaStream_t st,
+                 const char* tag) {
+  GemmParams p;
+  memset(&p, 0, sizeof(p));
+  p.M = int(M); p.N = N; p.K = K;
+  p.out0 = out; p.ld_out = N; p.alpha = 1.f;
+  if (f32) return launch_gemm<2, false, true, EPI_F32>({dy, K, false}, {w, N, true}, p, sk, st, tag);
+  return launch_gemm<2, false, true, EPI_BF16>({dy, K, false}, {w, N, true}, p, sk, st, tag);
+}
+}  // namespace
+
+extern "C" {
+
+int64_t td_t5_attention_layer_workspace_bytes(int64_t M, int64_t Mk, int32_t d, int32_t H, int32_t self_attention) {
+  return (int64_t)carve_attn_layer(nullptr, M, Mk, d, H, self_attention != 0).bytes;
+}
+
+int32_t td_t5_self_attention_layer_fwd(const void* x, int64_t M, int32_t d, int32_t H, const int32_t* cu_q, int32_t B, int32_t max_len,
+                                       const float* ln_w, float eps, const void* w_qkv, const void* wo, const float* bias_by_distance,
+                                       int32_t n_dist, void* out, float* rstd, void* qkv, void* o, float* lse, void* ws, int64_t ws_bytes,
+                                       td_stream_t stream) {
+  TD_DEVICE_OR_RETURN();
+  const char* fn = "td_t5_self_attention_layer_fwd";
+  int rc = attn_layer_check(fn, M, 0, d, H, true, ws, ws_bytes);
+  if (rc || M == 0) return rc;
+  if (!x || !ln_w || !w_qkv || !wo || !out) TD_FAIL(TD_ERR_ARG, "%s: null pointer", fn);
+  if (misaligned16(x) || misaligned16(ln_w) || misaligned16(w_qkv) || misaligned16(wo) || misaligned16(out) || misaligned16(qkv) ||
+      misaligned16(o))
+    TD_FAIL(TD_ERR_ARG, "%s: x / ln_w / w_qkv / wo / out / qkv / o must be 16-byte aligned", fn);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int32_t inner = kAttnDk * H;
+  const AttnLayerWorkspace w = carve_attn_layer(ws, M, 0, d, H, true);
+  __nv_bfloat16* qkv_ = qkv ? static_cast<__nv_bfloat16*>(qkv) : w.proj;
+  void* o_ = o ? o : w.heads;
+  float* rstd_ = rstd ? rstd : w.rstd;
+  AttnCall c;  // the attention's own checks, before anything is enqueued
+  rc = attn_check(fn, qkv_, 3 * inner, qkv_ + inner, 3 * inner, qkv_ + 2 * inner, 3 * inner, cu_q, nullptr, B, H, inner, max_len, max_len, M,
+                  1, bias_by_distance, n_dist, c);
+  if (rc) return rc;
+  {
+    ProfScope prof("sa_norm", double(M) * d * 4.0, st);
+    rc = rmsnorm_fwd_launch(x, ln_w, eps, M, d, w.rows, TD_DTYPE_BF16, rstd_, st);
+  }
+  if (rc) return rc;
+  rc = proj_gemm(w.rows, M, d, w_qkv, 3 * inner, qkv_, w.sk, st, "gemm_sa_qkv");
+  if (rc) return rc;
+  rc = td_t5_attention_fwd(qkv_, 3 * inner, qkv_ + inner, 3 * inner, qkv_ + 2 * inner, 3 * inner, cu_q, nullptr, B, H, inner, max_len, max_len,
+                           M, 1, bias_by_distance, n_dist, o_, inner, lse, stream);
+  if (rc) return rc;
+  return attn_out_gemm(o_, inner, wo, x, out, M, d, w.sk, st, "gemm_sa_out");
+}
+
+int32_t td_t5_self_attention_layer_bwd(const void* dy, const void* x, const float* rstd, const float* ln_w, const void* qkv, const void* o,
+                                       const float* lse, const void* w_qkv, const void* wo, const float* bias_by_distance, int32_t n_dist,
+                                       const int32_t* cu_q, int32_t B, int32_t max_len, int64_t M, int32_t d, int32_t H, void* dx, void* dqkv,
+                                       void* ws, int64_t ws_bytes, td_stream_t stream) {
+  TD_DEVICE_OR_RETURN();
+  const char* fn = "td_t5_self_attention_layer_bwd";
+  int rc = attn_layer_check(fn, M, 0, d, H, true, ws, ws_bytes);
+  if (rc || M == 0) return rc;
+  if (!dy || !x || !rstd || !ln_w || !qkv || !o || !lse || !w_qkv || !wo || !dx) TD_FAIL(TD_ERR_ARG, "%s: null pointer", fn);
+  if (misaligned16(dy) || misaligned16(x) || misaligned16(ln_w) || misaligned16(qkv) || misaligned16(o) || misaligned16(w_qkv) ||
+      misaligned16(wo) || misaligned16(dx) || misaligned16(dqkv))
+    TD_FAIL(TD_ERR_ARG, "%s: dy / x / ln_w / qkv / o / w_qkv / wo / dx / dqkv must be 16-byte aligned", fn);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int32_t inner = kAttnDk * H;
+  const AttnLayerWorkspace w = carve_attn_layer(ws, M, 0, d, H, true);
+  const __nv_bfloat16* q = static_cast<const __nv_bfloat16*>(qkv);
+  __nv_bfloat16* dq = dqkv ? static_cast<__nv_bfloat16*>(dqkv) : w.proj;
+  AttnCall c;
+  rc = attn_check(fn, q, 3 * inner, q + inner, 3 * inner, q + 2 * inner, 3 * inner, cu_q, nullptr, B, H, inner, max_len, max_len, M, 1,
+                  bias_by_distance, n_dist, c);
+  if (rc) return rc;
+  rc = proj_dx_gemm(dy, M, d, wo, inner, w.heads, false, w.sk, st, "gemm_sa_do");
+  if (rc) return rc;
+  rc = td_t5_attention_bwd(w.heads, inner, q, 3 * inner, q + inner, 3 * inner, q + 2 * inner, 3 * inner, cu_q, nullptr, B, H, inner, max_len,
+                           max_len, M, 1, bias_by_distance, n_dist, o, inner, lse, dq, 3 * inner, dq + inner, 3 * inner, dq + 2 * inner,
+                           3 * inner, w.delta, w.delta_bytes, stream);
+  if (rc) return rc;
+  rc = proj_dx_gemm(dq, M, 3 * inner, w_qkv, d, w.rows, false, w.sk, st, "gemm_sa_dx");
+  if (rc) return rc;
+  return residual_norm_bwd_launch(w.rows, x, rstd, ln_w, M, d, dy, dx, "sa_norm_bwd", st);
+}
+
+int32_t td_t5_cross_attention_layer_fwd(const void* x, int64_t M, const void* enc, int64_t Mk, int32_t d, int32_t H, const int32_t* cu_q,
+                                        const int32_t* cu_k, int32_t B, int32_t max_len_q, int32_t max_len_k, const float* ln_w, float eps,
+                                        const void* w_q, const void* w_kv, const void* wo, void* out, float* rstd, void* q, void* kv, void* o,
+                                        float* lse, void* ws, int64_t ws_bytes, td_stream_t stream) {
+  TD_DEVICE_OR_RETURN();
+  const char* fn = "td_t5_cross_attention_layer_fwd";
+  int rc = attn_layer_check(fn, M, Mk, d, H, false, ws, ws_bytes);
+  if (rc || M == 0) return rc;
+  if (!x || (Mk > 0 && !enc) || !ln_w || !w_q || !w_kv || !wo || !out) TD_FAIL(TD_ERR_ARG, "%s: null pointer", fn);
+  if (misaligned16(x) || misaligned16(enc) || misaligned16(ln_w) || misaligned16(w_q) || misaligned16(w_kv) || misaligned16(wo) ||
+      misaligned16(out) || misaligned16(q) || misaligned16(kv) || misaligned16(o))
+    TD_FAIL(TD_ERR_ARG, "%s: x / enc / ln_w / w_q / w_kv / wo / out / q / kv / o must be 16-byte aligned", fn);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int32_t inner = kAttnDk * H;
+  const AttnLayerWorkspace w = carve_attn_layer(ws, M, Mk, d, H, false);
+  void* q_ = q ? q : w.q;
+  __nv_bfloat16* kv_ = kv ? static_cast<__nv_bfloat16*>(kv) : w.proj;
+  void* o_ = o ? o : w.heads;
+  float* rstd_ = rstd ? rstd : w.rstd;
+  AttnCall c;
+  rc = attn_check(fn, q_, inner, kv_, 2 * inner, kv_ + inner, 2 * inner, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, M, 0, nullptr, 0, c);
+  if (rc) return rc;
+  {
+    ProfScope prof("ca_norm", double(M) * d * 4.0, st);
+    rc = rmsnorm_fwd_launch(x, ln_w, eps, M, d, w.rows, TD_DTYPE_BF16, rstd_, st);
+  }
+  if (rc) return rc;
+  rc = proj_gemm(w.rows, M, d, w_q, inner, q_, w.sk, st, "gemm_ca_q");
+  if (rc) return rc;
+  rc = proj_gemm(enc, Mk, d, w_kv, 2 * inner, kv_, w.sk, st, "gemm_ca_kv");
+  if (rc) return rc;
+  rc = td_t5_attention_fwd(q_, inner, kv_, 2 * inner, kv_ + inner, 2 * inner, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, M, 0, nullptr, 0,
+                           o_, inner, lse, stream);
+  if (rc) return rc;
+  return attn_out_gemm(o_, inner, wo, x, out, M, d, w.sk, st, "gemm_ca_out");
+}
+
+int32_t td_t5_cross_attention_layer_bwd(const void* dy, const void* x, const float* rstd, const float* ln_w, const void* q, const void* kv,
+                                        const void* o, const float* lse, const void* w_q, const void* w_kv, const void* wo, const int32_t* cu_q,
+                                        const int32_t* cu_k, int32_t B, int32_t max_len_q, int32_t max_len_k, int64_t M, int64_t Mk, int32_t d,
+                                        int32_t H, void* dx, float* d_enc, void* ws, int64_t ws_bytes, td_stream_t stream) {
+  TD_DEVICE_OR_RETURN();
+  const char* fn = "td_t5_cross_attention_layer_bwd";
+  int rc = attn_layer_check(fn, M, Mk, d, H, false, ws, ws_bytes);
+  if (rc || M == 0) return rc;
+  if (!dy || !x || !rstd || !ln_w || !q || (Mk > 0 && !kv) || !o || !lse || !w_q || !w_kv || !wo || !dx || (Mk > 0 && !d_enc))
+    TD_FAIL(TD_ERR_ARG, "%s: null pointer", fn);
+  if (misaligned16(dy) || misaligned16(x) || misaligned16(ln_w) || misaligned16(q) || misaligned16(kv) || misaligned16(o) ||
+      misaligned16(w_q) || misaligned16(w_kv) || misaligned16(wo) || misaligned16(dx) || misaligned16(d_enc))
+    TD_FAIL(TD_ERR_ARG, "%s: dy / x / ln_w / q / kv / o / w_q / w_kv / wo / dx / d_enc must be 16-byte aligned", fn);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int32_t inner = kAttnDk * H;
+  const AttnLayerWorkspace w = carve_attn_layer(ws, M, Mk, d, H, false);
+  const __nv_bfloat16* k = kv ? static_cast<const __nv_bfloat16*>(kv) : w.proj;  // Mk == 0: no key is read
+  AttnCall c;
+  rc = attn_check(fn, q, inner, k, 2 * inner, k + inner, 2 * inner, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, M, 0, nullptr, 0, c);
+  if (rc) return rc;
+  rc = proj_dx_gemm(dy, M, d, wo, inner, w.heads, false, w.sk, st, "gemm_ca_do");
+  if (rc) return rc;
+  rc = td_t5_attention_bwd(w.heads, inner, q, inner, k, 2 * inner, k + inner, 2 * inner, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, M, 0,
+                           nullptr, 0, o, inner, lse, w.q, inner, w.proj, 2 * inner, w.proj + inner, 2 * inner, w.delta, w.delta_bytes, stream);
+  if (rc) return rc;
+  rc = proj_dx_gemm(w.q, M, inner, w_q, d, w.rows, false, w.sk, st, "gemm_ca_dq");
+  if (rc) return rc;
+  rc = proj_dx_gemm(w.proj, Mk, 2 * inner, w_kv, d, d_enc, true, w.sk, st, "gemm_ca_denc");
+  if (rc) return rc;
+  return residual_norm_bwd_launch(w.rows, x, rstd, ln_w, M, d, dy, dx, "ca_norm_bwd", st);
 }
 
 }  // extern "C"

@@ -311,15 +311,17 @@ def rmsnorm_fwd(x: torch.Tensor, g: torch.Tensor, eps: float = 1e-6, out_bf16: b
     return y, rstd
 
 
-def rmsnorm_bwd(dy, x, rstd, g):
+def rmsnorm_bwd(dy, x, rstd, g, want_dg: bool = True, want_dxsum: bool = True):
+    """Returns ``(dx, dg, dxsum)``; ``want_dg`` / ``want_dxsum`` False skip those column sums (None is returned): with both False, for a
+    frozen norm weight, the backward is one launch."""
     _need_cuda(dy, x, rstd, g)
     M, D = x.shape
     dx = torch.empty((M, D), dtype=torch.bfloat16, device=x.device)
-    dg = torch.empty((D,), dtype=torch.float32, device=x.device)
-    dxsum = torch.empty((D,), dtype=torch.float32, device=x.device)
+    dg = torch.empty((D,), dtype=torch.float32, device=x.device) if want_dg else None
+    dxsum = torch.empty((D,), dtype=torch.float32, device=x.device) if want_dxsum else None
     ws_bytes = L.lib().td_rmsnorm_bwd_workspace_bytes(M, D)
     ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=x.device)
-    L.launch_count += 3
+    L.launch_count += 3 if (want_dg or want_dxsum) else 1
     L.check(L.lib().td_rmsnorm_bwd(L.ptr(_contig(dy, "dy")), L.dtype_code(dy), L.ptr(x), L.ptr(rstd), L.ptr(g), M, D,
                                    L.ptr(dx), L.ptr(dg), L.ptr(dxsum), L.ptr(ws), ws_bytes, L.stream_ptr()), "td_rmsnorm_bwd")
     return dx, dg, dxsum
@@ -589,3 +591,152 @@ def t5_ffn_bwd(dy, x, rstd, ab, wi, wo, ln_w, want_d_ab: bool = False):
     L.check(L.lib().td_t5_ffn_bwd(L.ptr(dy), L.ptr(x), L.ptr(rstd), L.ptr(ln_w), L.ptr(ab), L.ptr(wi), L.ptr(wo), M, d, d_ff, L.ptr(dx),
                                   L.ptr(d_ab), L.ptr(ws), ws_bytes, L.stream_ptr()), "td_t5_ffn_bwd")
     return dx, d_ab
+
+
+# ------------------------------------------------------------------------------------------------ T5 attention sublayers (8 f-1)
+def _attn_layer_dims(x, ln_w, wo, n_heads):
+    _need_cuda(x, ln_w, wo)
+    M, d = x.shape
+    inner = 64 * n_heads
+    if x.dtype != torch.bfloat16 or wo.dtype != torch.bfloat16 or ln_w.dtype != torch.float32:
+        raise TypeError("t5 attention layer: x and the weights must be bfloat16, ln_w float32")
+    if tuple(wo.shape) != (d, inner) or tuple(ln_w.shape) != (d,):
+        raise ValueError(f"t5 attention layer: need wo [d, 64 H] = [{d}, {inner}] and ln_w [d]; got {tuple(wo.shape)}, {tuple(ln_w.shape)}")
+    for t, n in ((x, "x"), (ln_w, "ln_w"), (wo, "wo")):
+        _contig(t, n)
+    return M, d, inner
+
+
+def _proj_weight(w, rows, d, name):
+    if w.dtype != torch.bfloat16 or tuple(w.shape) != (rows, d):
+        raise TypeError(f"{name} must be bfloat16 [{rows}, {d}], got {w.dtype} {tuple(w.shape)}")
+    return _contig(w, name)
+
+
+def _layer_ws(M, Mk, d, n_heads, self_attention, dev):
+    n = L.lib().td_t5_attention_layer_workspace_bytes(M, Mk, d, n_heads, int(self_attention))
+    return torch.empty((n,), dtype=torch.uint8, device=dev), n
+
+
+def _saved(t, shape, dtype, name):
+    if t is None or t.dtype != dtype or tuple(t.shape) != tuple(shape):
+        raise TypeError(f"{name} must be the forward's {dtype} {list(shape)} (run the forward with want_saved=True)")
+    return _contig(t, name)
+
+
+def t5_self_attention_layer_fwd(x, w_qkv, wo, ln_w, eps: float, bias_by_distance, cu_q, max_len: int, n_heads: int,
+                                want_saved: bool = True):
+    """T5LayerSelfAttention forward on packed decoder rows (causal, relative position bias): ``x [M, d]`` bf16, ``w_qkv [3 inner, d]``
+    bf16 (``[Wq; Wk; Wv]``), ``wo [d, inner]`` bf16, ``ln_w [d]`` fp32, ``bias_by_distance [H, n_dist]`` fp32, ``cu_q`` int32 [B + 1]
+    with ``cu_q[B] == M``, inner = 64 H. Returns ``(out [M, d] bf16, rstd, qkv, o, lse)``; the last four are what the backward takes
+    and are None when ``want_saved=False`` (inference: nothing beyond ``out`` is kept). Four launches."""
+    M, d, inner = _attn_layer_dims(x, ln_w, wo, n_heads)
+    _proj_weight(w_qkv, 3 * inner, d, "w_qkv")
+    _need_cuda(cu_q, bias_by_distance)
+    if cu_q.dtype != torch.int32 or bias_by_distance is None or bias_by_distance.dtype != torch.float32 or bias_by_distance.dim() != 2:
+        raise TypeError("cu_q must be int32 and bias_by_distance float32 [H, n_dist]")
+    _contig(bias_by_distance, "bias_by_distance")
+    dev = x.device
+    out = torch.empty((M, d), dtype=torch.bfloat16, device=dev)
+    rstd = qkv = o = lse = None
+    if want_saved:
+        rstd = torch.empty((M,), dtype=torch.float32, device=dev)
+        qkv = torch.empty((M, 3 * inner), dtype=torch.bfloat16, device=dev)
+        o = torch.empty((M, inner), dtype=torch.bfloat16, device=dev)
+        lse = torch.empty((n_heads, M), dtype=torch.float32, device=dev)
+    ws, ws_bytes = _layer_ws(M, 0, d, n_heads, True, dev)
+    L.launch_count += 4
+    L.check(L.lib().td_t5_self_attention_layer_fwd(L.ptr(x), M, d, n_heads, L.ptr(cu_q), cu_q.numel() - 1, int(max_len), L.ptr(ln_w), eps,
+                                                   L.ptr(w_qkv), L.ptr(wo), L.ptr(bias_by_distance), bias_by_distance.shape[1], L.ptr(out),
+                                                   L.ptr(rstd), L.ptr(qkv), L.ptr(o), L.ptr(lse), L.ptr(ws), ws_bytes, L.stream_ptr()),
+            "td_t5_self_attention_layer_fwd")
+    return out, rstd, qkv, o, lse
+
+
+def t5_self_attention_layer_bwd(dy, x, rstd, qkv, o, lse, w_qkv, wo, ln_w, bias_by_distance, cu_q, max_len: int, n_heads: int,
+                                want_dqkv: bool = False):
+    """Input gradient of ``t5_self_attention_layer_fwd`` (frozen weights) from ``dy [M, d]`` bf16 and the forward's saved tensors.
+    Returns ``(dx [M, d] bf16, dqkv [M, 3 inner] bf16 or None)``. Six launches; deterministic."""
+    M, d, inner = _attn_layer_dims(x, ln_w, wo, n_heads)
+    _proj_weight(w_qkv, 3 * inner, d, "w_qkv")
+    _need_cuda(dy, cu_q, bias_by_distance)
+    _saved(dy, (M, d), torch.bfloat16, "dy")
+    _saved(rstd, (M,), torch.float32, "rstd")
+    _saved(qkv, (M, 3 * inner), torch.bfloat16, "qkv")
+    _saved(o, (M, inner), torch.bfloat16, "o")
+    _saved(lse, (n_heads, M), torch.float32, "lse")
+    dev = x.device
+    dx = torch.empty((M, d), dtype=torch.bfloat16, device=dev)
+    dqkv = torch.empty((M, 3 * inner), dtype=torch.bfloat16, device=dev) if want_dqkv else None
+    ws, ws_bytes = _layer_ws(M, 0, d, n_heads, True, dev)
+    L.launch_count += 6
+    L.check(L.lib().td_t5_self_attention_layer_bwd(L.ptr(dy), L.ptr(x), L.ptr(rstd), L.ptr(ln_w), L.ptr(qkv), L.ptr(o), L.ptr(lse),
+                                                   L.ptr(w_qkv), L.ptr(wo), L.ptr(bias_by_distance), bias_by_distance.shape[1], L.ptr(cu_q),
+                                                   cu_q.numel() - 1, int(max_len), M, d, n_heads, L.ptr(dx), L.ptr(dqkv), L.ptr(ws), ws_bytes,
+                                                   L.stream_ptr()), "td_t5_self_attention_layer_bwd")
+    return dx, dqkv
+
+
+def t5_cross_attention_layer_fwd(x, enc, w_q, w_kv, wo, ln_w, eps: float, cu_q, cu_k, max_len_q: int, max_len_k: int, n_heads: int,
+                                 want_saved: bool = True):
+    """T5LayerCrossAttention forward: decoder rows ``x [M, d]`` bf16 (samples ``cu_q``) attend to the packed aligner rows ``enc [Mk, d]``
+    bf16 (samples ``cu_k``, int32 [B + 1] like ``cu_q``). ``w_q [inner, d]``, ``w_kv [2 inner, d]`` (``[Wk; Wv]``), ``wo [d, inner]``
+    bf16, ``ln_w [d]`` fp32. Returns ``(out [M, d] bf16, rstd, q, kv, o, lse)``, the last five None when ``want_saved=False``.
+    Five launches."""
+    M, d, inner = _attn_layer_dims(x, ln_w, wo, n_heads)
+    _proj_weight(w_q, inner, d, "w_q")
+    _proj_weight(w_kv, 2 * inner, d, "w_kv")
+    _need_cuda(enc, cu_q, cu_k)
+    if enc.dtype != torch.bfloat16 or enc.dim() != 2 or enc.shape[1] != d:
+        raise TypeError(f"enc must be bfloat16 [Mk, {d}]")
+    _contig(enc, "enc")
+    if cu_q.dtype != torch.int32 or cu_k.dtype != torch.int32 or cu_k.numel() != cu_q.numel():
+        raise TypeError("cu_q / cu_k must be int32 [B + 1]")
+    Mk = enc.shape[0]
+    dev = x.device
+    out = torch.empty((M, d), dtype=torch.bfloat16, device=dev)
+    rstd = q = kv = o = lse = None
+    if want_saved:
+        rstd = torch.empty((M,), dtype=torch.float32, device=dev)
+        q = torch.empty((M, inner), dtype=torch.bfloat16, device=dev)
+        kv = torch.empty((Mk, 2 * inner), dtype=torch.bfloat16, device=dev)
+        o = torch.empty((M, inner), dtype=torch.bfloat16, device=dev)
+        lse = torch.empty((n_heads, M), dtype=torch.float32, device=dev)
+    ws, ws_bytes = _layer_ws(M, Mk, d, n_heads, False, dev)
+    L.launch_count += 5
+    L.check(L.lib().td_t5_cross_attention_layer_fwd(L.ptr(x), M, L.ptr(enc), Mk, d, n_heads, L.ptr(cu_q), L.ptr(cu_k),
+                                                    cu_q.numel() - 1, int(max_len_q), int(max_len_k), L.ptr(ln_w), eps, L.ptr(w_q),
+                                                    L.ptr(w_kv), L.ptr(wo), L.ptr(out), L.ptr(rstd), L.ptr(q), L.ptr(kv), L.ptr(o), L.ptr(lse),
+                                                    L.ptr(ws), ws_bytes, L.stream_ptr()), "td_t5_cross_attention_layer_fwd")
+    return out, rstd, q, kv, o, lse
+
+
+def t5_cross_attention_layer_bwd(dy, x, rstd, q, kv, o, lse, w_q, w_kv, wo, ln_w, cu_q, cu_k, max_len_q: int, max_len_k: int,
+                                 n_heads: int):
+    """Gradients of ``t5_cross_attention_layer_fwd`` (frozen weights) from ``dy [M, d]`` bf16 and the forward's saved tensors. Returns
+    ``(dx [M, d] bf16, d_enc [Mk, d] fp32)``: ``d_enc = dkv . [Wk; Wv]`` summed in fp32 and not rounded. Seven launches;
+    deterministic."""
+    M, d, inner = _attn_layer_dims(x, ln_w, wo, n_heads)
+    _proj_weight(w_q, inner, d, "w_q")
+    _proj_weight(w_kv, 2 * inner, d, "w_kv")
+    _need_cuda(dy, cu_q, cu_k)
+    if kv is None or kv.dim() != 2:
+        raise TypeError("kv must be the forward's bfloat16 [Mk, 2 inner] (run the forward with want_saved=True)")
+    Mk = kv.shape[0]
+    _saved(dy, (M, d), torch.bfloat16, "dy")
+    _saved(rstd, (M,), torch.float32, "rstd")
+    _saved(q, (M, inner), torch.bfloat16, "q")
+    _saved(kv, (Mk, 2 * inner), torch.bfloat16, "kv")
+    _saved(o, (M, inner), torch.bfloat16, "o")
+    _saved(lse, (n_heads, M), torch.float32, "lse")
+    dev = x.device
+    dx = torch.empty((M, d), dtype=torch.bfloat16, device=dev)
+    d_enc = torch.empty((Mk, d), dtype=torch.float32, device=dev)
+    ws, ws_bytes = _layer_ws(M, Mk, d, n_heads, False, dev)
+    L.launch_count += 7
+    L.check(L.lib().td_t5_cross_attention_layer_bwd(L.ptr(dy), L.ptr(x), L.ptr(rstd), L.ptr(ln_w), L.ptr(q), L.ptr(kv), L.ptr(o), L.ptr(lse),
+                                                    L.ptr(w_q), L.ptr(w_kv), L.ptr(wo), L.ptr(cu_q), L.ptr(cu_k), cu_q.numel() - 1,
+                                                    int(max_len_q), int(max_len_k), M, Mk, d, n_heads, L.ptr(dx),
+                                                    L.ptr(d_enc), L.ptr(ws), ws_bytes, L.stream_ptr()),
+            "td_t5_cross_attention_layer_bwd")
+    return dx, d_enc

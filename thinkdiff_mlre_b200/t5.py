@@ -1,6 +1,7 @@
-"""The frozen T5 decoder's attention and feed-forward sublayers on packed rows (SURVEY section 8 f-1): host plumbing for the
-relative position bias and the gated FFN's weight layout, and the autograd boundaries of their tcgen05 kernels. The attention
-composes with ``frozen_linear`` for the Q / K / V / O projections."""
+"""The frozen T5 decoder on packed rows (SURVEY section 8 f-1): host plumbing for the relative position bias and the gated FFN's
+weight layout, the autograd boundaries of the attention core and of the three sublayers (self-attention, cross-attention,
+feed-forward), and their composition into a decoder block and the decoder stack. The attention core also composes with
+``frozen_linear`` for hand-built projections."""
 from __future__ import annotations
 
 import math
@@ -170,3 +171,221 @@ def t5_layer_ff(x: torch.Tensor, weights: T5FeedForwardWeights) -> torch.Tensor:
     bf16 autocast, dropout off (DESIGN.md section 7). ``x [..., d]``; returns bf16 of the same shape. The weights are frozen: the
     gradient flows to ``x`` only. Saves ``x``, ``rstd`` and ``ab`` ([rows, 2 d_ff] bf16) for the backward."""
     return _T5LayerFF.apply(x, weights)
+
+
+# ------------------------------------------------------------------------------------------------ attention sublayers, block, stack
+def _frozen(named):
+    for n, t in named:
+        if t.requires_grad:
+            raise NotImplementedError(f"T5 decoder weights: {n} must not require grad (the T5 decoder is frozen in ThinkDiff)")
+
+
+class T5DecoderBlockWeights:
+    """Frozen weights of one decoder ``T5Block`` in the layout the sublayer kernels read: the three pre-norm weights ``ln_self``,
+    ``ln_cross`` (fp32 [d]) and ``ffn.ln_weight``; ``w_qkv`` [3 inner, d] (``[Wq; Wk; Wv]`` of the self-attention, one GEMM),
+    ``wo_self`` [d, inner], ``w_q`` [inner, d], ``w_kv`` [2 inner, d] (``[Wk; Wv]`` of the cross-attention) and ``wo_cross`` [d, inner]
+    (bf16); ``ffn`` (``T5FeedForwardWeights``); ``n_heads`` and ``eps``. inner = 64 n_heads: d_kv must be 64."""
+
+    def __init__(self, ln_self, wq, wk, wv, wo_self, ln_cross, cq, ck, cv, wo_cross, ffn: T5FeedForwardWeights, n_heads: int,
+                 eps: float = 1e-6):
+        _frozen((("layer.0.layer_norm.weight", ln_self), ("SelfAttention.q", wq), ("SelfAttention.k", wk), ("SelfAttention.v", wv),
+                 ("SelfAttention.o", wo_self), ("layer.1.layer_norm.weight", ln_cross), ("EncDecAttention.q", cq),
+                 ("EncDecAttention.k", ck), ("EncDecAttention.v", cv), ("EncDecAttention.o", wo_cross)))
+        inner, d = wq.shape
+        if n_heads < 1 or inner != 64 * n_heads:
+            raise NotImplementedError(f"T5DecoderBlockWeights: d_kv = {inner / max(n_heads, 1):g} (inner {inner}, {n_heads} heads); the "
+                                      "attention kernels need d_kv = 64")
+        for t, shape, n in ((wk, (inner, d), "k"), (wv, (inner, d), "v"), (cq, (inner, d), "cross q"), (ck, (inner, d), "cross k"),
+                            (cv, (inner, d), "cross v"), (wo_self, (d, inner), "o"), (wo_cross, (d, inner), "cross o"),
+                            (ln_self, (d,), "layer.0.layer_norm"), (ln_cross, (d,), "layer.1.layer_norm")):
+            if tuple(t.shape) != shape:
+                raise ValueError(f"T5DecoderBlockWeights: {n} must be {list(shape)}, got {list(t.shape)}")
+        if ffn.d != d:
+            raise ValueError(f"T5DecoderBlockWeights: the FFN's d = {ffn.d} differs from the attention's d = {d}")
+
+        def bf(*ts):
+            return torch.cat([t.detach().to(torch.bfloat16) for t in ts]).contiguous()
+
+        self.d, self.n_heads, self.eps = d, int(n_heads), float(eps)
+        self.ln_self, self.ln_cross = ln_self.detach().float().contiguous(), ln_cross.detach().float().contiguous()
+        self.w_qkv, self.wo_self = bf(wq, wk, wv), bf(wo_self)
+        self.w_q, self.w_kv, self.wo_cross = bf(cq), bf(ck, cv), bf(wo_cross)
+        self.ffn = ffn
+
+    @classmethod
+    def from_module(cls, block) -> "T5DecoderBlockWeights":
+        """From a live transformers decoder ``T5Block`` whose parameters are frozen (``requires_grad_(False)``)."""
+        sa, ca = block.layer[0], block.layer[1]
+        a, c = sa.SelfAttention, ca.EncDecAttention
+        if a.key_value_proj_dim != 64 or c.key_value_proj_dim != 64:
+            raise NotImplementedError(f"T5DecoderBlockWeights: d_kv = {a.key_value_proj_dim}; the attention kernels need d_kv = 64")
+        return cls(sa.layer_norm.weight, a.q.weight, a.k.weight, a.v.weight, a.o.weight, ca.layer_norm.weight, c.q.weight, c.k.weight,
+                   c.v.weight, c.o.weight, T5FeedForwardWeights.from_module(block.layer[2]), a.n_heads, sa.layer_norm.variance_epsilon)
+
+    @classmethod
+    def from_state_dict(cls, sd: dict, n_heads: int, eps: float = 1e-6, prefix: str = "") -> "T5DecoderBlockWeights":
+        """From a ``T5Block`` state dict (``layer.0.SelfAttention.q.weight``, ..., behind ``prefix``, e.g. ``"block.3."``)."""
+        s, c = prefix + "layer.0.", prefix + "layer.1."
+        return cls(sd[s + "layer_norm.weight"], *(sd[s + f"SelfAttention.{n}.weight"] for n in "qkvo"), sd[c + "layer_norm.weight"],
+                   *(sd[c + f"EncDecAttention.{n}.weight"] for n in "qkvo"),
+                   T5FeedForwardWeights.from_state_dict(sd, eps, prefix=prefix + "layer.2."), n_heads, eps)
+
+    def to(self, device) -> "T5DecoderBlockWeights":
+        for n in ("ln_self", "ln_cross", "w_qkv", "wo_self", "w_q", "w_kv", "wo_cross"):
+            setattr(self, n, getattr(self, n).to(device))
+        self.ffn.to(device)
+        return self
+
+
+class T5DecoderWeights:
+    """Frozen weights of a decoder ``T5Stack``: ``blocks`` (``T5DecoderBlockWeights``), ``final_ln`` (fp32 [d]), ``eps``, and
+    ``position_bias``, block 0's relative attention bias table turned once into the per-distance table the self-attention kernels
+    read (``t5_position_bias_by_distance``, [H, max_distance] fp32), shared by every block as in HF."""
+
+    def __init__(self, blocks, final_ln: torch.Tensor, bias_table: torch.Tensor, eps: float = 1e-6, num_buckets: int = 32,
+                 max_distance: int = 128):
+        _frozen((("final_layer_norm.weight", final_ln), ("relative_attention_bias.weight", bias_table)))
+        self.blocks = list(blocks)
+        if not self.blocks:
+            raise ValueError("T5DecoderWeights: no blocks")
+        self.final_ln = final_ln.detach().float().contiguous()
+        self.position_bias = t5_position_bias_by_distance(bias_table, num_buckets, max_distance)
+        if self.position_bias.shape[0] != self.blocks[0].n_heads:
+            raise ValueError(f"T5DecoderWeights: the bias table has {self.position_bias.shape[0]} heads, the blocks {self.blocks[0].n_heads}")
+        self.eps = float(eps)
+
+    @classmethod
+    def from_module(cls, stack) -> "T5DecoderWeights":
+        """From a live transformers decoder ``T5Stack`` whose parameters are frozen."""
+        cfg = stack.config
+        return cls([T5DecoderBlockWeights.from_module(b) for b in stack.block], stack.final_layer_norm.weight,
+                   stack.block[0].layer[0].SelfAttention.relative_attention_bias.weight, stack.final_layer_norm.variance_epsilon,
+                   cfg.relative_attention_num_buckets, cfg.relative_attention_max_distance)
+
+    @classmethod
+    def from_state_dict(cls, sd: dict, n_heads: int, eps: float = 1e-6, prefix: str = "", num_buckets: int = 32,
+                        max_distance: int = 128) -> "T5DecoderWeights":
+        """From a decoder ``T5Stack`` state dict (``block.{i}.layer...``, ``final_layer_norm.weight``, behind ``prefix``)."""
+        n_blocks = 1 + max(int(k[len(prefix):].split(".")[1]) for k in sd if k.startswith(prefix + "block."))
+        blocks = [T5DecoderBlockWeights.from_state_dict(sd, n_heads, eps, prefix=f"{prefix}block.{i}.") for i in range(n_blocks)]
+        return cls(blocks, sd[prefix + "final_layer_norm.weight"], sd[prefix + "block.0.layer.0.SelfAttention.relative_attention_bias.weight"],
+                   eps, num_buckets, max_distance)
+
+    def to(self, device) -> "T5DecoderWeights":
+        for b in self.blocks:
+            b.to(device)
+        self.final_ln, self.position_bias = self.final_ln.to(device), self.position_bias.to(device)
+        return self
+
+
+class _T5LayerSelfAttention(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, cu_q, max_len, weights, bias):
+        w = weights
+        x2 = x.reshape(-1, x.shape[-1]).to(torch.bfloat16).contiguous()
+        need_grad = ctx.needs_input_grad[0]
+        out, rstd, qkv, o, lse = ops.t5_self_attention_layer_fwd(x2, w.w_qkv, w.wo_self, w.ln_self, w.eps, bias, cu_q, max_len, w.n_heads,
+                                                                 want_saved=need_grad)
+        if need_grad:
+            ctx.save_for_backward(x2, rstd, qkv, o, lse, cu_q, bias)
+            ctx.weights, ctx.max_len = w, max_len
+        ctx.shape, ctx.dtype = x.shape, x.dtype
+        return out.view(x.shape)
+
+    @staticmethod
+    def backward(ctx, dy):
+        x2, rstd, qkv, o, lse, cu_q, bias = ctx.saved_tensors
+        w = ctx.weights
+        dy2 = dy.reshape(x2.shape).to(torch.bfloat16).contiguous()
+        dx, _ = ops.t5_self_attention_layer_bwd(dy2, x2, rstd, qkv, o, lse, w.w_qkv, w.wo_self, w.ln_self, bias, cu_q, ctx.max_len, w.n_heads)
+        return dx.view(ctx.shape).to(ctx.dtype), None, None, None, None
+
+
+def t5_layer_self_attention(x: torch.Tensor, cu_q: torch.Tensor, max_len_q: int, weights: T5DecoderBlockWeights,
+                            position_bias: torch.Tensor) -> torch.Tensor:
+    """transformers' ``T5LayerSelfAttention`` of a decoder block on packed rows, forward and input gradient on the library's kernels:
+    ``x + o(attention(q(norm(x)), k(norm(x)), v(norm(x))))``, causal within each sample ``cu_q[b]:cu_q[b+1]`` (covering every row),
+    with ``position_bias`` from ``T5DecoderWeights.position_bias`` (or ``t5_position_bias_by_distance``), rounded as the bf16 model
+    under bf16 autocast (DESIGN.md section 7). ``x [rows, d]``; returns bf16. The weights are frozen: the gradient flows to ``x``.
+    Saves ``x``, ``rstd``, ``qkv``, ``o`` and ``lse`` when ``x`` needs a gradient, nothing otherwise."""
+    if position_bias is None or position_bias.requires_grad:
+        raise NotImplementedError("t5_layer_self_attention: pass the frozen per-distance bias table (t5_position_bias_by_distance)")
+    return _T5LayerSelfAttention.apply(x, cu_q, int(max_len_q), weights, position_bias)
+
+
+class _T5LayerCrossAttention(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, enc, cu_q, cu_k, max_len_q, max_len_k, weights):
+        w = weights
+        x2 = x.reshape(-1, x.shape[-1]).to(torch.bfloat16).contiguous()
+        e2 = enc.reshape(-1, enc.shape[-1]).to(torch.bfloat16).contiguous()  # autocast's cast, once per use as in HF
+        need_grad = any(ctx.needs_input_grad[:2])
+        out, rstd, q, kv, o, lse = ops.t5_cross_attention_layer_fwd(x2, e2, w.w_q, w.w_kv, w.wo_cross, w.ln_cross, w.eps, cu_q, cu_k,
+                                                                    max_len_q, max_len_k, w.n_heads, want_saved=need_grad)
+        if need_grad:
+            ctx.save_for_backward(x2, rstd, q, kv, o, lse, cu_q, cu_k)
+            ctx.weights, ctx.max_lens = w, (max_len_q, max_len_k)
+        ctx.shapes, ctx.dtypes = (x.shape, enc.shape), (x.dtype, enc.dtype)
+        return out.view(x.shape)
+
+    @staticmethod
+    def backward(ctx, dy):
+        x2, rstd, q, kv, o, lse, cu_q, cu_k = ctx.saved_tensors
+        w = ctx.weights
+        dy2 = dy.reshape(x2.shape).to(torch.bfloat16).contiguous()
+        dx, d_enc = ops.t5_cross_attention_layer_bwd(dy2, x2, rstd, q, kv, o, lse, w.w_q, w.w_kv, w.wo_cross, w.ln_cross, cu_q, cu_k,
+                                                     *ctx.max_lens, w.n_heads)
+        # d_enc is fp32: returned in enc's dtype, so autograd sums the blocks' contributions in fp32 when enc is fp32
+        d_enc = d_enc.view(ctx.shapes[1]).to(ctx.dtypes[1]) if ctx.needs_input_grad[1] else None
+        dx = dx.view(ctx.shapes[0]).to(ctx.dtypes[0]) if ctx.needs_input_grad[0] else None
+        return dx, d_enc, None, None, None, None, None
+
+
+def t5_layer_cross_attention(x: torch.Tensor, enc: torch.Tensor, cu_q: torch.Tensor, cu_k: torch.Tensor, max_len_q: int, max_len_k: int,
+                             weights: T5DecoderBlockWeights) -> torch.Tensor:
+    """transformers' ``T5LayerCrossAttention`` on packed rows: decoder rows ``x`` (samples ``cu_q``) attend to the packed aligner rows
+    ``enc [Mk, d]`` (samples ``cu_k``), ``x + o(attention(q(norm(x)), k(enc), v(enc)))``. ``enc`` may be fp32 (the aligner's output in
+    training) or bf16; it is cast to bf16 inside, and its gradient, summed in fp32 by one GEMM, comes back in ``enc``'s dtype. A sample
+    without aligner rows passes ``x`` through unchanged. Returns bf16 of ``x``'s shape."""
+    return _T5LayerCrossAttention.apply(x, enc, cu_q, cu_k, int(max_len_q), int(max_len_k), weights)
+
+
+def t5_decoder_block(x: torch.Tensor, enc: torch.Tensor, cu_q: torch.Tensor, cu_k: torch.Tensor, max_len_q: int, max_len_k: int,
+                     weights: T5DecoderBlockWeights, position_bias: torch.Tensor) -> torch.Tensor:
+    """One decoder ``T5Block`` on packed rows: causal self-attention with the relative position bias, cross-attention to the packed
+    aligner rows, gated-GELU FFN, each pre-norm with its residual, on the library's kernels (15 launches forward, 19 backward)."""
+    h = t5_layer_self_attention(x, cu_q, max_len_q, weights, position_bias)
+    h = t5_layer_cross_attention(h, enc, cu_q, cu_k, max_len_q, max_len_k, weights)
+    return t5_layer_ff(h, weights.ffn)
+
+
+class _T5FinalNorm(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, weight, eps):
+        x2 = x.reshape(-1, x.shape[-1]).to(torch.bfloat16).contiguous()
+        y, rstd = ops.rmsnorm_fwd(x2, weight, eps, out_bf16=True)
+        if ctx.needs_input_grad[0]:
+            ctx.save_for_backward(x2, rstd, weight)
+        ctx.shape, ctx.dtype = x.shape, x.dtype
+        return y.view(x.shape)
+
+    @staticmethod
+    def backward(ctx, dy):
+        x2, rstd, weight = ctx.saved_tensors
+        dy2 = dy.reshape(x2.shape).to(torch.bfloat16).contiguous()
+        dx, _, _ = ops.rmsnorm_bwd(dy2, x2, rstd, weight, want_dg=False, want_dxsum=False)
+        return dx.view(ctx.shape).to(ctx.dtype), None, None
+
+
+def t5_decoder_stack(dec_rows: torch.Tensor, enc: torch.Tensor, cu_q: torch.Tensor, cu_k: torch.Tensor, max_len_q: int, max_len_k: int,
+                     weights: T5DecoderWeights) -> torch.Tensor:
+    """The frozen decoder ``T5Stack`` of ``T5ForDecoder.forward`` (thinkdiff/models/mllama_vllm_t5_embed_decoder_2.py:211-224) on packed
+    rows: every block in order (``t5_decoder_block``), then the frozen final norm (bf16 out; its backward skips the weight gradient).
+    ``dec_rows [Mq, d]`` are the decoder input embeddings packed with ``cu_q``; ``enc [Mk, d]`` the aligner rows packed with ``cu_k``
+    (fp32 or bf16; the gradient reaching it is summed over the blocks in its dtype). With right-padded labels and no decoder mask, as
+    in the reference, a valid position never sees a pad position under the causal mask, so packing only the valid decoder rows is exact
+    for the loss. The output feeds ``lm_head_cross_entropy`` unchanged."""
+    h = dec_rows
+    for bw in weights.blocks:
+        h = t5_decoder_block(h, enc, cu_q, cu_k, max_len_q, max_len_k, bw, weights.position_bias)
+    return _T5FinalNorm.apply(h, weights.final_ln, weights.eps)
