@@ -44,10 +44,10 @@ struct Profiler {
 };
 struct ProfScope {
   cudaStream_t st; cudaEvent_t e1 = nullptr;
-  // `work` = algorithmic FLOPs (GEMMs) or bytes (row kernels) of this launch, for the roofline report
+  // `work` = algorithmic FLOPs (GEMMs) or bytes (row kernels) of this launch, for the roofline report; a null tag records nothing
   ProfScope(const char* tag, double work, cudaStream_t s) : st(s) {
     Profiler& p = Profiler::get();
-    if (!p.on.load(std::memory_order_relaxed)) return;
+    if (!tag || !p.on.load(std::memory_order_relaxed)) return;
     ProfRecord r{tag, nullptr, nullptr, work, s};
     cudaEventCreate(&r.e0); cudaEventCreate(&r.e1);
     cudaEventRecord(r.e0, st);
@@ -257,6 +257,13 @@ inline void plan_schedule(GemmParams& p, int max_workers, bool stream_k) {
   }
 }
 
+// The tile grid of a GEMM whose clusters are CTAS CTAs wide: each tile is CTAS * kBlockM rows by kBlockN columns, kBlockK deep.
+inline void set_tile_grid(GemmParams& p, int ctas) {
+  p.num_m_blocks = (p.M + kBlockM * ctas - 1) / (kBlockM * ctas);
+  p.num_n_blocks = (p.N + kBlockN - 1) / kBlockN;
+  p.num_k_blocks = (p.K + kBlockK - 1) / kBlockK;
+}
+
 // `ws` (optional, gemm_sk_workspace_bytes()) enables the stream-K tail.
 template <int CTAS, bool A_MN, bool B_MN, int EPI>
 int launch_gemm(GemmOperand a, GemmOperand b, GemmParams p, void* ws, cudaStream_t stream, const char* tag = "gemm") {
@@ -299,9 +306,7 @@ int launch_gemm(GemmOperand a, GemmOperand b, GemmParams p, void* ws, cudaStream
     rc = make_epilogue_map(&maux, p.aux0, p.M, out_cols, p.ld_out, false);
     if (rc) return rc;
   }
-  p.num_m_blocks = (p.M + kBlockM * CTAS - 1) / (kBlockM * CTAS);
-  p.num_n_blocks = (p.N + kBlockN - 1) / kBlockN;
-  p.num_k_blocks = (p.K + kBlockK - 1) / kBlockK;
+  set_tile_grid(p, CTAS);
   plan_schedule(p, device_sm_count() / CTAS, ws != nullptr);
   p.sk_partials = static_cast<float*>(ws);
   p.sched_counter = next_sched_counter();

@@ -9,6 +9,7 @@
 #include "attn_sm100.cuh"
 
 #include <cmath>
+#include <initializer_list>
 
 using namespace td;
 
@@ -77,19 +78,10 @@ struct PdlConfig {
   PdlConfig(const PdlConfig&) = delete;  // cfg points at attr
 };
 
-inline int norm_bwd_grid(long long M, int* rows_per_cta) {
-  // one slab of rows per CTA, a multiple of the R rows it walks at a time
-  int ctas = device_sm_count() * 2;
-  long long rpc = (M + ctas - 1) / ctas;
-  rpc = (rpc + kNormBwdRows - 1) / kNormBwdRows * kNormBwdRows;
-  if (rpc < kNormBwdRows) rpc = kNormBwdRows;
-  *rows_per_cta = int(rpc);
-  return int((M + rpc - 1) / rpc);
-}
-
-inline int norm_mse_grid(long long M, int* rows_per_cta) {
-  // fused norm + MSE + norm-backward: one 512-thread CTA per SM, each with one contiguous slab of rows
-  int ctas = device_sm_count();
+// Grid of the norm-backward kernels: up to `ctas_per_sm` CTAs per SM (2 for the plain backward, 1 for the fused norm + MSE +
+// norm-backward), each with one contiguous slab of rows, a multiple of the kNormBwdRows rows it walks at a time.
+inline int norm_grid(long long M, int ctas_per_sm, int* rows_per_cta) {
+  int ctas = device_sm_count() * ctas_per_sm;
   long long rpc = (M + ctas - 1) / ctas;
   rpc = (rpc + kNormBwdRows - 1) / kNormBwdRows * kNormBwdRows;
   if (rpc < kNormBwdRows) rpc = kNormBwdRows;
@@ -98,6 +90,52 @@ inline int norm_mse_grid(long long M, int* rows_per_cta) {
 }
 
 inline bool dims_ok(int Din, int D) { return Din > 0 && D > 0 && Din % 64 == 0 && D % 64 == 0 && D <= 8 * kNormBwdThreads; }
+
+// A pointer argument of an entry point, by name, and what it must be: non-null and 16-byte aligned (the default), 16-byte aligned
+// when given (an optional buffer), or only non-null.
+enum PtrRule { kNonNullAligned, kOptionalAligned, kNonNull };
+struct Arg {
+  const char* name;
+  const void* ptr;
+  PtrRule rule = kNonNullAligned;
+};
+
+// Fails with the entry's name and the first offending argument; every null check comes before the alignment checks.
+int check_pointers(const char* fn, std::initializer_list<Arg> args) {
+  for (const Arg& a : args)
+    if (a.rule != kOptionalAligned && !a.ptr) TD_FAIL(TD_ERR_ARG, "%s: null pointer (%s)", fn, a.name);
+  for (const Arg& a : args)
+    if (a.rule != kNonNull && (reinterpret_cast<uintptr_t>(a.ptr) & 15)) TD_FAIL(TD_ERR_ARG, "%s: %s must be 16-byte aligned", fn, a.name);
+  return TD_OK;
+}
+
+// Zeroed GEMM parameters for an [M, N] output (row pitch N) over a K-long contraction, alpha = 1.
+GemmParams gemm_params(int64_t M, int32_t N, int64_t K) {
+  GemmParams p;
+  memset(&p, 0, sizeof(p));
+  p.M = int(M); p.N = N; p.K = int(K);
+  p.ld_out = N; p.alpha = 1.f;
+  return p;
+}
+
+// The pack entries: rows = total_rows (varlen) or B * L_max (padded), each row_bytes long, copied by pack_rows_kernel<PADDED>.
+template <bool PADDED>
+int pack_launch(const char* fn, std::initializer_list<Arg> ptrs, const void* src, const void* src2, const int64_t* src_row_start,
+                const int32_t* cu, int32_t B, int64_t rows, int32_t L_max, int64_t row_bytes, void* dst, int64_t* mask,
+                int64_t* src_row_out, cudaStream_t st) {
+  if (B < 0 || rows < 0 || L_max < 0 || row_bytes <= 0 || row_bytes % 16)
+    TD_FAIL(TD_ERR_ARG, "%s: row_bytes=%lld must be a positive multiple of 16", fn, (long long)row_bytes);
+  if (rows == 0 || B == 0) return TD_OK;
+  int rc = check_pointers(fn, ptrs);
+  if (rc) return rc;
+  ProfScope prof(PADDED ? "pack_padded" : "pack_varlen", 2.0 * double(rows) * double(row_bytes), st);
+  PdlConfig l(grid_for_rows(rows, 8, 8), 256, st);
+  TD_CUDA(cudaLaunchKernelEx(&l.cfg, pack_rows_kernel<PADDED>, static_cast<const uint4*>(src),
+                             reinterpret_cast<const long long*>(src_row_start), cu, B, (long long)rows, L_max, int(row_bytes / 16),
+                             static_cast<uint4*>(dst), reinterpret_cast<long long*>(mask),
+                             reinterpret_cast<long long*>(src_row_out), static_cast<const uint4*>(src2)));
+  return TD_OK;
+}
 
 }  // namespace
 
@@ -183,62 +221,24 @@ int32_t td_pack_varlen(const void* src, const int64_t* src_row_start, const int3
 int32_t td_pack_varlen_indexed(const void* src, const int64_t* src_row_start, const int32_t* cu, int32_t B,
                                int64_t total_rows, int64_t row_bytes, void* dst, int64_t* src_row_out, td_stream_t stream) {
   TD_DEVICE_OR_RETURN();
-  if (B < 0 || total_rows < 0 || row_bytes <= 0 || row_bytes % 16)
-    TD_FAIL(TD_ERR_ARG, "td_pack_varlen: row_bytes=%lld must be a positive multiple of 16", (long long)row_bytes);
-  if (total_rows == 0 || B == 0) return TD_OK;
-  if (!src || !src_row_start || !cu || !dst) TD_FAIL(TD_ERR_ARG, "td_pack_varlen: null pointer");
-  if ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst)) & 15)
-    TD_FAIL(TD_ERR_ARG, "td_pack_varlen: buffers must be 16-byte aligned");
-  const int grid = grid_for_rows(total_rows, 8, 8);
-  {
-    ProfScope prof("pack_varlen", 2.0 * double(total_rows) * double(row_bytes), (cudaStream_t)stream);
-    PdlConfig l(grid, 256, (cudaStream_t)stream);
-    TD_CUDA(cudaLaunchKernelEx(&l.cfg, pack_rows_kernel<false>, static_cast<const uint4*>(src),
-                               reinterpret_cast<const long long*>(src_row_start), cu, B, total_rows, 0, int(row_bytes / 16),
-                               static_cast<uint4*>(dst), nullptr, reinterpret_cast<long long*>(src_row_out), nullptr));
-  }
-  return TD_OK;
+  return pack_launch<false>("td_pack_varlen", {{"src", src}, {"src_row_start", src_row_start, kNonNull}, {"cu", cu, kNonNull}, {"dst", dst}},
+                            src, nullptr, src_row_start, cu, B, total_rows, 0, row_bytes, dst, nullptr, src_row_out, (cudaStream_t)stream);
 }
 
 int32_t td_pack_varlen2(const void* src, const void* src2, const int64_t* src_row_start, const int32_t* cu, int32_t B,
                         int64_t total_rows, int64_t row_bytes, void* dst, td_stream_t stream) {
   TD_DEVICE_OR_RETURN();
-  if (B < 0 || total_rows < 0 || row_bytes <= 0 || row_bytes % 16)
-    TD_FAIL(TD_ERR_ARG, "td_pack_varlen2: row_bytes=%lld must be a positive multiple of 16", (long long)row_bytes);
-  if (total_rows == 0 || B == 0) return TD_OK;
-  if (!src || !src2 || !src_row_start || !cu || !dst) TD_FAIL(TD_ERR_ARG, "td_pack_varlen2: null pointer");
-  if ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(src2) | reinterpret_cast<uintptr_t>(dst)) & 15)
-    TD_FAIL(TD_ERR_ARG, "td_pack_varlen2: buffers must be 16-byte aligned");
-  const int grid = grid_for_rows(total_rows, 8, 8);
-  {
-    ProfScope prof("pack_varlen", 2.0 * double(total_rows) * double(row_bytes), (cudaStream_t)stream);
-    PdlConfig l(grid, 256, (cudaStream_t)stream);
-    TD_CUDA(cudaLaunchKernelEx(&l.cfg, pack_rows_kernel<false>, static_cast<const uint4*>(src),
-                               reinterpret_cast<const long long*>(src_row_start), cu, B, total_rows, 0, int(row_bytes / 16),
-                               static_cast<uint4*>(dst), nullptr, nullptr, static_cast<const uint4*>(src2)));
-  }
-  return TD_OK;
+  return pack_launch<false>("td_pack_varlen2",
+                            {{"src", src}, {"src2", src2}, {"src_row_start", src_row_start, kNonNull}, {"cu", cu, kNonNull}, {"dst", dst}},
+                            src, src2, src_row_start, cu, B, total_rows, 0, row_bytes, dst, nullptr, nullptr, (cudaStream_t)stream);
 }
 
 int32_t td_pack_padded(const void* src, const int64_t* src_row_start, const int32_t* cu, int32_t B, int32_t L_max,
                        int64_t row_bytes, void* dst, int64_t* mask, td_stream_t stream) {
   TD_DEVICE_OR_RETURN();
-  if (B < 0 || L_max < 0 || row_bytes <= 0 || row_bytes % 16)
-    TD_FAIL(TD_ERR_ARG, "td_pack_padded: row_bytes=%lld must be a positive multiple of 16", (long long)row_bytes);
-  if (B == 0 || L_max == 0) return TD_OK;
-  if (!src_row_start || !cu || !dst) TD_FAIL(TD_ERR_ARG, "td_pack_padded: null pointer");
-  if ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst)) & 15)
-    TD_FAIL(TD_ERR_ARG, "td_pack_padded: buffers must be 16-byte aligned");
-  const long long rows = (long long)B * L_max;
-  const int grid = grid_for_rows(rows, 8, 8);
-  {
-    ProfScope prof("pack_padded", 2.0 * double(rows) * double(row_bytes), (cudaStream_t)stream);
-    PdlConfig l(grid, 256, (cudaStream_t)stream);
-    TD_CUDA(cudaLaunchKernelEx(&l.cfg, pack_rows_kernel<true>, static_cast<const uint4*>(src),
-                               reinterpret_cast<const long long*>(src_row_start), cu, B, rows, L_max, int(row_bytes / 16),
-                               static_cast<uint4*>(dst), reinterpret_cast<long long*>(mask), nullptr, nullptr));
-  }
-  return TD_OK;
+  return pack_launch<true>("td_pack_padded", {{"src", src, kOptionalAligned}, {"src_row_start", src_row_start, kNonNull}, {"cu", cu, kNonNull},
+                           {"dst", dst}}, src, nullptr, src_row_start, cu, B, (int64_t)B * L_max, L_max, row_bytes, dst, mask, nullptr,
+                           (cudaStream_t)stream);
 }
 
 // ------------------------------------------------------------------------------------------------ casts
@@ -258,13 +258,19 @@ int32_t td_cast_f32_to_bf16(const float* src, void* dst, int64_t n, td_stream_t 
 }
 
 // ------------------------------------------------------------------------------------------------ norm
-static int rmsnorm_fwd_launch(const void* x, const float* g, float eps, int64_t M, int32_t D, void* y, int32_t y_dtype,
-                              float* rstd, cudaStream_t st) {
+// y (bf16 or fp32) = x * rstd * g. With `ssq_part`, each row's sum of squares comes from the `nparts` partials the GEMM that wrote
+// x left behind instead of from x itself. A null tag launches unprofiled.
+static int rmsnorm_fwd_launch(const void* x, const float* ssq_part, int nparts, const float* g, float eps, int64_t M, int32_t D,
+                              void* y, int32_t y_dtype, float* rstd, const char* tag, cudaStream_t st) {
   const int grid = grid_for_rows(M, 8, 8);
-  if (y_dtype == TD_DTYPE_BF16)
-    rmsnorm_fwd_kernel<true><<<grid, 256, 0, st>>>(static_cast<const __nv_bfloat16*>(x), nullptr, 0, g, eps, int(M), D, y, rstd);
-  else
-    rmsnorm_fwd_kernel<false><<<grid, 256, 0, st>>>(static_cast<const __nv_bfloat16*>(x), nullptr, 0, g, eps, int(M), D, y, rstd);
+  const __nv_bfloat16* xb = static_cast<const __nv_bfloat16*>(x);
+  {
+    ProfScope prof(tag, double(M) * D * (y_dtype == TD_DTYPE_BF16 ? 4.0 : 6.0), st);
+    if (y_dtype == TD_DTYPE_BF16)
+      rmsnorm_fwd_kernel<true><<<grid, 256, 0, st>>>(xb, ssq_part, nparts, g, eps, int(M), D, y, rstd);
+    else
+      rmsnorm_fwd_kernel<false><<<grid, 256, 0, st>>>(xb, ssq_part, nparts, g, eps, int(M), D, y, rstd);
+  }
   TD_CUDA(cudaGetLastError());
   return TD_OK;
 }
@@ -275,12 +281,12 @@ int32_t td_rmsnorm_fwd(const void* x, const float* g, float eps, int64_t M, int3
   if (M < 0 || D <= 0 || D % 8 || D > 8 * 32 * kNormFwdMaxVec)
     TD_FAIL(TD_ERR_ARG, "td_rmsnorm_fwd: D=%d must be a positive multiple of 8, at most %d", D, 8 * 32 * kNormFwdMaxVec);
   if (M == 0) return TD_OK;
-  return rmsnorm_fwd_launch(x, g, eps, M, D, y, y_dtype, rstd, (cudaStream_t)stream);
+  return rmsnorm_fwd_launch(x, nullptr, 0, g, eps, M, D, y, y_dtype, rstd, nullptr, (cudaStream_t)stream);
 }
 
 int64_t td_rmsnorm_bwd_workspace_bytes(int64_t M, int32_t D) {
   int rpc;
-  const int grid = norm_bwd_grid(M > 0 ? M : 1, &rpc);
+  const int grid = norm_grid(M > 0 ? M : 1, 2, &rpc);
   return (int64_t)(2 * align_up(sizeof(float) * (size_t)grid * D, 256));
 }
 
@@ -288,7 +294,7 @@ static int rmsnorm_bwd_impl(const void* dy, int32_t dy_dtype, const __nv_bfloat1
                             int64_t M, int32_t D, __nv_bfloat16* dx, float* dg, float* dxsum, float scale, void* ws,
                             cudaStream_t st) {
   int rpc;
-  const int grid = norm_bwd_grid(M, &rpc);
+  const int grid = norm_grid(M, 2, &rpc);
   Carver c(ws);
   float* dg_part = c.take<float>((size_t)grid * D);
   float* db_part = c.take<float>((size_t)grid * D);
@@ -300,12 +306,11 @@ static int rmsnorm_bwd_impl(const void* dy, int32_t dy_dtype, const __nv_bfloat1
     rmsnorm_bwd_kernel<false><<<grid, kNormBwdThreads, 0, st>>>(dy, x, rstd, g, int(M), D, rpc, dx, dg_part, db_part);
   }
   TD_CUDA(cudaGetLastError());
-  if (dg && dxsum)
-    colsum_finish_kernel<<<dim3((D + 31) / 32, 2), 256, 0, st>>>(dg_part, dg, db_part, dxsum, grid, D, scale);
-  else if (dg)
-    colsum_finish_kernel<<<dim3((D + 31) / 32, 1), 256, 0, st>>>(dg_part, dg, nullptr, nullptr, grid, D, scale);
-  else if (dxsum)
-    colsum_finish_kernel<<<dim3((D + 31) / 32, 1), 256, 0, st>>>(db_part, dxsum, nullptr, nullptr, grid, D, scale);
+  if (dg || dxsum) {  // one column-sum job per requested output (grid.y)
+    const bool both = dg && dxsum;
+    colsum_finish_kernel<<<dim3((D + 31) / 32, both ? 2 : 1), 256, 0, st>>>(dg ? dg_part : db_part, dg ? dg : dxsum,
+                                                                          both ? db_part : nullptr, both ? dxsum : nullptr, grid, D, scale);
+  }
   TD_CUDA(cudaGetLastError());
   return TD_OK;
 }
@@ -331,6 +336,49 @@ int64_t td_gemm_workspace_bytes(void) { return (int64_t)align_up(gemm_sk_workspa
 namespace {
 // the stream-K workspace is optional at the test / utility entries: without it the leftover tiles run as a last partial wave
 inline void* sk_ws_or_null(void* ws, int64_t ws_bytes) { return (ws && ws_bytes >= td_gemm_workspace_bytes()) ? ws : nullptr; }
+
+// The GEMM shapes the entries share. `a` [M, K] is K-major throughout; `sk` is the optional stream-K workspace.
+
+// out [M, N] bf16 = bf16(a . w^T (+ bias)), w [N, K] K-major: a linear layer
+int gemm_linear(const void* a, int64_t M, int32_t K, const void* w, int32_t N, const void* bias, void* out, void* sk, cudaStream_t st,
+                const char* tag) {
+  GemmParams p = gemm_params(M, N, K);
+  p.out0 = out; p.bias = static_cast<const __nv_bfloat16*>(bias);
+  return launch_gemm<2, false, false, EPI_BF16>({a, K, false}, {w, K, false}, p, sk, st, tag);
+}
+
+// out [M, N] = a . w, w [K, N] read MN-major in place (the input gradient of a linear layer): bf16, or fp32 when `f32`
+int gemm_linear_dx(const void* a, int64_t M, int64_t K, const void* w, int32_t N, void* out, bool f32, void* sk, cudaStream_t st,
+                   const char* tag) {
+  GemmParams p = gemm_params(M, N, K);
+  p.out0 = out;
+  if (f32) return launch_gemm<2, false, true, EPI_F32>({a, K, false}, {w, N, true}, p, sk, st, tag);
+  return launch_gemm<2, false, true, EPI_BF16>({a, K, false}, {w, N, true}, p, sk, st, tag);
+}
+
+// out [M, N] bf16 = bf16(x + bf16(a . w^T)), w [N, K] K-major: the closing projection of a residual sublayer
+int gemm_residual(const void* a, int64_t M, int32_t K, const void* w, int32_t N, const void* x, void* out, void* sk, cudaStream_t st,
+                  const char* tag) {
+  GemmParams p = gemm_params(M, N, K);
+  p.out0 = out; p.aux0 = x;
+  return launch_gemm<2, false, false, EPI_RESIDUAL>({a, K, false}, {w, K, false}, p, sk, st, tag);
+}
+
+// The aligner's Linear1: h0 = x . W1^T + b1 [M, D] and h1 = bf16(gelu(h0))
+int gemm_fwd1(const void* x, int64_t M, int32_t Din, const void* W1, int32_t D, const void* b1, void* h0, void* h1, void* sk,
+              cudaStream_t st) {
+  GemmParams p = gemm_params(M, D, Din);
+  p.out0 = h0; p.out1 = h1; p.bias = static_cast<const __nv_bfloat16*>(b1);
+  return launch_gemm<2, false, false, EPI_BIAS_GELU>({x, Din, false}, {W1, Din, false}, p, sk, st, "gemm_fwd1_bias_gelu");
+}
+
+// The aligner's Linear2: h2 = bf16(h1 . W2^T + b2) [M, D], with per-row sum-of-squares partials in ssq_part for the norm after it
+int gemm_fwd2(const void* h1, int64_t M, int32_t D, const void* W2, const void* b2, void* h2, float* ssq_part, void* sk,
+              cudaStream_t st) {
+  GemmParams p = gemm_params(M, D, D);
+  p.out0 = h2; p.bias = static_cast<const __nv_bfloat16*>(b2); p.red0 = ssq_part;
+  return launch_gemm<2, false, false, EPI_BIAS_SSQ>({h1, D, false}, {W2, D, false}, p, sk, st, "gemm_fwd2_bias_ssq");
+}
 }  // namespace
 
 int32_t td_linear_bf16(const void* x, int64_t M, int32_t K, const void* W, int32_t N, const void* bias, void* out, void* ws,
@@ -338,11 +386,7 @@ int32_t td_linear_bf16(const void* x, int64_t M, int32_t K, const void* W, int32
   TD_DEVICE_OR_RETURN();
   if (M < 0 || K <= 0 || N <= 0 || K % 8 || N % 32) TD_FAIL(TD_ERR_UNSUPPORTED, "td_linear_bf16: need K %% 8 == 0, N %% 32 == 0");
   if (M == 0) return TD_OK;
-  GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.M = int(M); p.N = N; p.K = K;
-  p.out0 = out; p.ld_out = N; p.bias = static_cast<const __nv_bfloat16*>(bias); p.alpha = 1.f;
-  return launch_gemm<2, false, false, EPI_BF16>({x, K, false}, {W, K, false}, p, sk_ws_or_null(ws, ws_bytes), (cudaStream_t)stream, "gemm_linear");
+  return gemm_linear(x, M, K, W, N, bias, out, sk_ws_or_null(ws, ws_bytes), (cudaStream_t)stream, "gemm_linear");
 }
 
 int32_t td_linear_bf16_dx(const void* dy, int64_t M, int32_t N, const void* W, int32_t K, void* dx, void* ws, int64_t ws_bytes,
@@ -350,11 +394,8 @@ int32_t td_linear_bf16_dx(const void* dy, int64_t M, int32_t N, const void* W, i
   TD_DEVICE_OR_RETURN();
   if (M < 0 || K <= 0 || N <= 0 || N % 8 || K % 64) TD_FAIL(TD_ERR_UNSUPPORTED, "td_linear_bf16_dx: need N %% 8 == 0, K %% 64 == 0");
   if (M == 0) return TD_OK;
-  GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.M = int(M); p.N = K; p.K = N;  // output [M, K]; the contraction runs over the N rows of W
-  p.out0 = dx; p.ld_out = K; p.alpha = 1.f;
-  return launch_gemm<2, false, true, EPI_BF16>({dy, N, false}, {W, K, true}, p, sk_ws_or_null(ws, ws_bytes), (cudaStream_t)stream, "gemm_linear_dx");
+  // output [M, K]; the contraction runs over the N rows of W
+  return gemm_linear_dx(dy, M, N, W, K, dx, false, sk_ws_or_null(ws, ws_bytes), (cudaStream_t)stream, "gemm_linear_dx");
 }
 
 int32_t td_gemm_bf16_f32out(const void* A, int64_t lda, int32_t a_mn, const void* B, int64_t ldb, int32_t b_mn, int64_t M,
@@ -362,10 +403,8 @@ int32_t td_gemm_bf16_f32out(const void* A, int64_t lda, int32_t a_mn, const void
                             int64_t ws_bytes, td_stream_t stream) {
   TD_DEVICE_OR_RETURN();
   if (M <= 0 || N <= 0 || K <= 0) TD_FAIL(TD_ERR_ARG, "td_gemm_bf16_f32out: empty problem");
-  GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.M = int(M); p.N = N; p.K = int(K);
-  p.out0 = out; p.ld_out = N; p.alpha = alpha; p.accumulate = accumulate != 0;
+  GemmParams p = gemm_params(M, N, K);
+  p.out0 = out; p.alpha = alpha; p.accumulate = accumulate != 0;
   cudaStream_t st = (cudaStream_t)stream;
   void* sk = sk_ws_or_null(ws, ws_bytes);
   GemmOperand a{A, lda, a_mn != 0}, b{B, ldb, b_mn != 0};
@@ -419,29 +458,11 @@ int32_t td_aligner_fwd(const void* x, int64_t M, int32_t Din, int32_t D, const v
   // sum-of-squares partials: one per 128-column half tile that exists (the last N tile may be half empty)
   const int nblk = (D + kEpiColsPerWarp - 1) / kEpiColsPerWarp;
 
-  GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.M = int(M); p.N = D; p.K = Din; p.ld_out = D; p.alpha = 1.f;
-  p.out0 = h0; p.out1 = h1; p.bias = static_cast<const __nv_bfloat16*>(b1);
-  int rc = launch_gemm<2, false, false, EPI_BIAS_GELU>({x, Din, false}, {W1, Din, false}, p, w.sk, st, "gemm_fwd1_bias_gelu");
+  int rc = gemm_fwd1(x, M, Din, W1, D, b1, h0, h1, w.sk, st);
   if (rc) return rc;
-
-  memset(&p, 0, sizeof(p));
-  p.M = int(M); p.N = D; p.K = D; p.ld_out = D; p.alpha = 1.f;
-  p.out0 = h2; p.bias = static_cast<const __nv_bfloat16*>(b2); p.red0 = w.ssq_part;
-  rc = launch_gemm<2, false, false, EPI_BIAS_SSQ>({h1, D, false}, {W2, D, false}, p, w.sk, st, "gemm_fwd2_bias_ssq");
+  rc = gemm_fwd2(h1, M, D, W2, b2, h2, w.ssq_part, w.sk, st);
   if (rc) return rc;
-
-  const int grid = grid_for_rows(M, 8, 8);
-  ProfScope prof("rmsnorm_fwd", double(M) * D * (y_dtype == TD_DTYPE_BF16 ? 4.0 : 6.0), st);
-  if (y_dtype == TD_DTYPE_BF16)
-    rmsnorm_fwd_kernel<true><<<grid, 256, 0, st>>>(static_cast<const __nv_bfloat16*>(h2), w.ssq_part, nblk, g, eps, int(M),
-                                                   D, y, rstd);
-  else
-    rmsnorm_fwd_kernel<false><<<grid, 256, 0, st>>>(static_cast<const __nv_bfloat16*>(h2), w.ssq_part, nblk, g, eps, int(M),
-                                                    D, y, rstd);
-  TD_CUDA(cudaGetLastError());
-  return TD_OK;
+  return rmsnorm_fwd_launch(h2, w.ssq_part, nblk, g, eps, M, D, y, y_dtype, rstd, "rmsnorm_fwd", st);
 }
 
 // ------------------------------------------------------------------------------------------------ aligner backward
@@ -479,7 +500,7 @@ struct NormPartials {
 };
 NormPartials carve_norm_partials(void* buf, int64_t M, int32_t D) {
   NormPartials n;
-  n.grid = norm_mse_grid(M > 0 ? M : 1, &n.rows_per_cta);
+  n.grid = norm_grid(M > 0 ? M : 1, 1, &n.rows_per_cta);
   Carver c(buf);
   n.dg_part = c.take<float>((size_t)n.grid * D);
   n.db_part = c.take<float>((size_t)n.grid * D);
@@ -543,14 +564,13 @@ int launch_dw_gemm(GemmOperand a, GemmOperand b, GemmParams& p, float* const* ds
 int bwd_from_dh2(const __nv_bfloat16* dh2, const void* x, const void* h0, const void* h1, const void* W2, int64_t M,
                  int32_t Din, int32_t D, float scale, const float* scale_ptr, float* dW1, float* db1, float* dW2, float* db2,
                  float* dg, BwdWorkspace& w, int32_t phases, cudaStream_t st, const ScatterDst* sc, const BwdExtras& ex) {
-  GemmParams p;
   const int world = sc ? sc->world : 0;
   const bool do_gelu = (phases & (TD_BWD_PHASE_GELU_W1 | TD_BWD_PHASE_GELU_ONLY)) != 0;
   const bool do_small2 = ex.np != nullptr && (phases & (TD_BWD_PHASE_NORM_W2 | TD_BWD_PHASE_SMALL2_ONLY)) != 0;
   if (do_gelu) {
     // dh0 = bf16( bf16(scale_ptr * dh2 . W2) * gelu'(h0) ), plus per-slab column sums for db1
-    memset(&p, 0, sizeof(p));
-    p.M = int(M); p.N = D; p.K = D; p.ld_out = D; p.alpha = 1.f; p.alpha_ptr = scale_ptr;
+    GemmParams p = gemm_params(M, D, D);
+    p.alpha_ptr = scale_ptr;
     p.out0 = w.dh0; p.aux0 = h0; p.red0 = w.db1_part;
     int rc = launch_gemm<2, false, true, EPI_DGELU>({dh2, D, false}, {W2, D, true}, p, w.sk, st, "gemm_dh0_dgelu");
     if (rc) return rc;
@@ -584,8 +604,8 @@ int bwd_from_dh2(const __nv_bfloat16* dh2, const void* x, const void* h0, const 
   }
   if (phases & (TD_BWD_PHASE_GELU_W1 | TD_BWD_PHASE_W1_ONLY)) {
     // dW1[D, Din] = scale * dh0^T . x   (dh0 already carries the upstream scalar; W1_ONLY: dh0 is in the workspace from a GELU_ONLY call)
-    memset(&p, 0, sizeof(p));
-    p.M = D; p.N = Din; p.K = int(M); p.ld_out = Din; p.alpha = scale; p.out0 = dW1; p.stats = ex.stats; p.accumulate = ex.accumulate;
+    GemmParams p = gemm_params(D, Din, M);
+    p.alpha = scale; p.out0 = dW1; p.stats = ex.stats; p.accumulate = ex.accumulate;
     const bool last = !(phases & (TD_BWD_PHASE_NORM_W2 | TD_BWD_PHASE_W2_ONLY));  // the call's last GEMM carries the signal
     int rc = launch_dw_gemm({w.dh0, D, true}, {x, Din, true}, p, sc ? sc->dW1 : nullptr, world, sc ? sc->rank : -1, w.sk, st,
                             world ? "gemm_dW1_scatter" : "gemm_dW1", last ? sc : nullptr);
@@ -593,8 +613,8 @@ int bwd_from_dh2(const __nv_bfloat16* dh2, const void* x, const void* h0, const 
   }
   if (phases & (TD_BWD_PHASE_NORM_W2 | TD_BWD_PHASE_W2_ONLY)) {
     // dW2[D, D] = scale * dh2^T . h1  (contraction over tokens; both operands MN-major)
-    memset(&p, 0, sizeof(p));
-    p.M = D; p.N = D; p.K = int(M); p.ld_out = D; p.alpha = scale; p.alpha_ptr = scale_ptr; p.out0 = dW2; p.stats = ex.stats;
+    GemmParams p = gemm_params(D, D, M);
+    p.alpha = scale; p.alpha_ptr = scale_ptr; p.out0 = dW2; p.stats = ex.stats;
     p.accumulate = ex.accumulate;
     int rc = launch_dw_gemm({dh2, D, true}, {h1, D, true}, p, sc ? sc->dW2 : nullptr, world, sc ? sc->rank : -1, w.sk, st,
                             world ? "gemm_dW2_scatter" : "gemm_dW2", sc);
@@ -673,20 +693,13 @@ int32_t td_aligner_mse_fwd(const void* x, int64_t M, int32_t Din, int32_t D, con
   __nv_bfloat16* h2 = c.take<__nv_bfloat16>((size_t)M * D);
   NormPartials np = carve_norm_partials(norm_partials, M, D);  // consumed by td_aligner_bwd_dh2
 
-  GemmParams p;
   int rc;
   if (stages & TD_FWD_STAGE_LINEAR1) {  // Linear1 + GELU (reads W1, b1 only)
-    memset(&p, 0, sizeof(p));
-    p.M = int(M); p.N = D; p.K = Din; p.ld_out = D; p.alpha = 1.f;
-    p.out0 = h0; p.out1 = h1; p.bias = static_cast<const __nv_bfloat16*>(b1);
-    rc = launch_gemm<2, false, false, EPI_BIAS_GELU>({x, Din, false}, {W1, Din, false}, p, w.sk, st, "gemm_fwd1_bias_gelu");
+    rc = gemm_fwd1(x, M, Din, W1, D, b1, h0, h1, w.sk, st);
     if (rc) return rc;
   }
   if (!(stages & TD_FWD_STAGE_REST)) return TD_OK;
-  memset(&p, 0, sizeof(p));
-  p.M = int(M); p.N = D; p.K = D; p.ld_out = D; p.alpha = 1.f;
-  p.out0 = h2; p.bias = static_cast<const __nv_bfloat16*>(b2); p.red0 = w.ssq_part;
-  rc = launch_gemm<2, false, false, EPI_BIAS_SSQ>({h1, D, false}, {W2, D, false}, p, w.sk, st, "gemm_fwd2_bias_ssq");
+  rc = gemm_fwd2(h1, M, D, W2, b2, h2, w.ssq_part, w.sk, st);
   if (rc) return rc;
   const float dy_coef = 2.0f / (float(M) * float(D));
   const long long* tri = reinterpret_cast<const long long*>(target_row_index);
@@ -1051,12 +1064,8 @@ extern "C" {
 int32_t td_gemm_schedule(int64_t M, int32_t N, int64_t K, int32_t workers, int32_t stream_k, int32_t* out, int32_t max_segments) {
   // host arithmetic only: plan_schedule() + for_each_segment(), the code the launch and the kernel run
   if (M <= 0 || N <= 0 || K <= 0 || workers < 1 || M > 0x7fffffffll || K > 0x7fffffffll || (max_segments > 0 && !out)) return -1;
-  GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.M = int(M); p.N = N; p.K = int(K);
-  p.num_m_blocks = (p.M + 2 * kBlockM - 1) / (2 * kBlockM);
-  p.num_n_blocks = (p.N + kBlockN - 1) / kBlockN;
-  p.num_k_blocks = (p.K + kBlockK - 1) / kBlockK;
+  GemmParams p = gemm_params(M, N, K);
+  set_tile_grid(p, 2);  // a CTA-pair GEMM, as every composite entry launches
   plan_schedule(p, workers, stream_k != 0);
   int n = 0;
   const int units = num_units(p);
@@ -1067,11 +1076,8 @@ int32_t td_gemm_schedule(int64_t M, int32_t N, int64_t K, int32_t workers, int32
 int32_t td_scatter_tile_owner(int32_t tile, int32_t M, int32_t N, int32_t world, int32_t rank, int32_t* m_blk_out, int32_t* n_blk_out) {
   // host arithmetic only (no device needed): the same tile_coords() the kernel runs, with the raster launch_dw_gemm sets up
   if (M <= 0 || N <= 0 || world < 1 || world > kMaxPeers || M % world || (M / world) % 32 || rank >= world) return -1;
-  GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.M = M; p.N = N;
-  p.num_m_blocks = (M + 2 * kBlockM - 1) / (2 * kBlockM);
-  p.num_n_blocks = (N + kBlockN - 1) / kBlockN;
+  GemmParams p = gemm_params(M, N, 0);
+  set_tile_grid(p, 2);  // launch_dw_gemm runs CTA pairs
   if (tile < 0 || tile >= p.num_m_blocks * p.num_n_blocks) return -1;
   set_scatter_raster(p, world, rank);
   int m_blk = 0, n_blk = 0;
@@ -1087,9 +1093,8 @@ int32_t td_gemm_tn_scatter(const void* A, int64_t lda, const void* B, int64_t ld
   if (rank >= world) TD_FAIL(TD_ERR_ARG, "td_gemm_tn_scatter: rank=%d outside world=%d", rank, world);
   if (world < 1 || world > kMaxPeers || M % world) TD_FAIL(TD_ERR_ARG, "td_gemm_tn_scatter: world=%d must be 1..%d and divide M", world, kMaxPeers);
   if (M <= 0 || M > 0x7fffffffll || K <= 0 || K > 0x7fffffffll) TD_FAIL(TD_ERR_ARG, "td_gemm_tn_scatter: size out of range");
-  GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.M = int(M); p.N = N; p.K = int(K); p.ld_out = N; p.alpha = alpha;
+  GemmParams p = gemm_params(M, N, K);
+  p.alpha = alpha;
   for (int o = 0; o < world; ++o) {
     if (!dst || !dst[o]) TD_FAIL(TD_ERR_ARG, "td_gemm_tn_scatter: null destination for rank %d", o);
   }
@@ -1204,8 +1209,6 @@ struct AttnCall {
   AttnParams p;
 };
 
-inline bool misaligned16(const void* ptr) { return (reinterpret_cast<uintptr_t>(ptr) & 15) != 0; }
-
 // Host checks shared by the forward and the backward; fills the kernel parameters that both use.
 int attn_check(const char* fn, const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv, const int32_t* cu_q,
                const int32_t* cu_k, int32_t B, int32_t H, int32_t inner, int32_t max_len_q, int32_t max_len_k, int64_t Mq,
@@ -1213,8 +1216,9 @@ int attn_check(const char* fn, const void* q, int64_t ldq, const void* k, int64_
   if (B < 0 || B > 65535 || H <= 0 || H > 65535 || max_len_q < 0 || max_len_k < 0 || Mq < 0)
     TD_FAIL(TD_ERR_ARG, "%s: bad sizes (B=%d H=%d max_len_q=%d max_len_k=%d Mq=%lld)", fn, B, H, max_len_q, max_len_k, (long long)Mq);
   if (inner != kAttnDk * H) TD_FAIL(TD_ERR_UNSUPPORTED, "%s: inner=%d must be 64 * H = %d (d_kv = 64 only)", fn, inner, kAttnDk * H);
-  if (!q || !k || !v || !cu_q || (!self_attention && !cu_k)) TD_FAIL(TD_ERR_ARG, "%s: null pointer", fn);
-  if (misaligned16(q) || misaligned16(k) || misaligned16(v)) TD_FAIL(TD_ERR_ARG, "%s: q / k / v must be 16-byte aligned", fn);
+  // (self-attention reads cu_q for its keys too)
+  int rc = check_pointers(fn, {{"q", q}, {"k", k}, {"v", v}, {"cu_q", cu_q, kNonNull}, {"cu_k", self_attention ? cu_q : cu_k, kNonNull}});
+  if (rc) return rc;
   if (ldq % 8 || ldk % 8 || ldv % 8 || ldq < inner || ldk < inner || ldv < inner)
     TD_FAIL(TD_ERR_ARG, "%s: row pitches must be multiples of 8 and >= inner (ldq=%lld ldk=%lld ldv=%lld)", fn, (long long)ldq,
             (long long)ldk, (long long)ldv);
@@ -1269,12 +1273,75 @@ int attn_launch(K kernel, dim3 grid, int threads, int smem, cudaStream_t st, con
 inline unsigned attn_tiles(int max_len) { return unsigned((max_len + kAttnTile - 1) / kAttnTile); }
 }  // namespace
 
-extern "C" {
-
-int64_t td_t5_attention_workspace_bytes(int64_t Mq, int32_t H) {
+extern "C" int64_t td_t5_attention_workspace_bytes(int64_t Mq, int32_t H) {
   const size_t rows = (size_t)(Mq > 0 ? Mq : 1), heads = (size_t)(H > 0 ? H : 1);
   return (int64_t)align_up(sizeof(float) * rows * heads, 256);  // Delta [H, Mq]
 }
+
+namespace {
+// Every check of the forward (attn_check and the output), run before anything is enqueued; attn_fwd_run then only launches.
+int attn_fwd_check(const char* fn, const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv, const int32_t* cu_q,
+                   const int32_t* cu_k, int32_t B, int32_t H, int32_t inner, int32_t max_len_q, int32_t max_len_k, int64_t Mq,
+                   int32_t self_attention, const float* bias, int32_t n_dist, void* o, int64_t ldo, float* lse, AttnCall& c) {
+  int rc = attn_check(fn, q, ldq, k, ldk, v, ldv, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, Mq, self_attention, bias, n_dist, c);
+  if (rc) return rc;
+  rc = check_pointers(fn, {{"o", o}});
+  if (rc) return rc;
+  if (ldo % 8 || ldo < inner) TD_FAIL(TD_ERR_ARG, "%s: o's row pitch must be a multiple of 8 and >= inner (ldo=%lld)", fn, (long long)ldo);
+  c.p.out = static_cast<__nv_bfloat16*>(o); c.p.ld_out = ldo; c.p.lse = lse;
+  return TD_OK;
+}
+
+int attn_fwd_run(const AttnCall& c, cudaStream_t st) {
+  const double flops = 4.0 * kAttnDk * c.H * attn_visible_pairs(c, st);
+  const dim3 grid(attn_tiles(c.max_len_q), c.H, c.B);
+  const int smem = attn_smem_bytes(AttnFwdSmem::kBias, c.p.n_dist);
+  return attn_launch(c.causal ? t5_attn_fwd_kernel<true> : t5_attn_fwd_kernel<false>, grid, kAttnThreads, smem, st, c.p, "attn_fwd", flops);
+}
+
+// Every check of the backward; attn_bwd_run then launches the row sums of dO * O, dK / dV and dQ.
+int attn_bwd_check(const char* fn, const void* dout, int64_t lddo, const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v,
+                   int64_t ldv, const int32_t* cu_q, const int32_t* cu_k, int32_t B, int32_t H, int32_t inner, int32_t max_len_q,
+                   int32_t max_len_k, int64_t Mq, int32_t self_attention, const float* bias, int32_t n_dist, const void* o,
+                   int64_t ldo, const float* lse, void* dq, int64_t lddq, void* dk, int64_t lddk, void* dv, int64_t lddv,
+                   void* ws, int64_t ws_bytes, AttnCall& c) {
+  int rc = attn_check(fn, q, ldq, k, ldk, v, ldv, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, Mq, self_attention, bias, n_dist, c);
+  if (rc) return rc;
+  rc = check_pointers(fn, {{"dout", dout}, {"o", o}, {"lse", lse, kNonNull}, {"dq", dq}, {"dk", dk}, {"dv", dv}});
+  if (rc) return rc;
+  if (lddo % 8 || ldo % 8 || lddq % 8 || lddk % 8 || lddv % 8 || lddo < inner || ldo < inner || lddq < inner || lddk < inner || lddv < inner)
+    TD_FAIL(TD_ERR_ARG, "%s: row pitches must be multiples of 8 and >= inner", fn);
+  if (!ws || ws_bytes < td_t5_attention_workspace_bytes(Mq, H)) TD_FAIL(TD_ERR_ARG, "%s: workspace too small", fn);
+  c.p.dout = static_cast<const __nv_bfloat16*>(dout); c.p.lddo = lddo;
+  c.p.o = static_cast<const __nv_bfloat16*>(o); c.p.ldo = ldo;
+  c.p.lse = const_cast<float*>(lse);
+  c.p.delta = static_cast<float*>(ws);
+  c.p.dq = static_cast<__nv_bfloat16*>(dq); c.p.lddq = lddq;
+  c.p.dk = static_cast<__nv_bfloat16*>(dk); c.p.lddk = lddk;
+  c.p.dv = static_cast<__nv_bfloat16*>(dv); c.p.lddv = lddv;
+  return TD_OK;
+}
+
+int attn_bwd_run(const AttnCall& c, cudaStream_t st) {
+  if (c.B == 0) return TD_OK;
+  const int H = c.H;
+  const long long Mq = c.p.Mq;
+  const double pairs = attn_visible_pairs(c, st);
+  const long long delta_threads = Mq * H * 8;
+  int rc = attn_launch(t5_attn_delta_kernel, dim3(unsigned((delta_threads + 255) / 256)), 256, 0, st, c.p, "attn_bwd_delta",
+                       double(Mq) * H * (4.0 * kAttnDk + 4.0));
+  if (rc) return rc;
+  const dim3 grid_k(attn_tiles(c.max_len_k), H, c.B), grid_q(attn_tiles(c.max_len_q), H, c.B);
+  const int smem_kv = attn_smem_bytes(AttnDkdvSmem::kBias, c.p.n_dist), smem_q = attn_smem_bytes(AttnDqSmem::kBias, c.p.n_dist);
+  const double f = 2.0 * kAttnDk * H * pairs;
+  rc = attn_launch(c.causal ? t5_attn_dkdv_kernel<true> : t5_attn_dkdv_kernel<false>, c.causal ? grid_q : grid_k, kAttnThreads, smem_kv, st,
+                   c.p, "attn_bwd_dkdv", 4 * f);
+  if (rc) return rc;
+  return attn_launch(c.causal ? t5_attn_dq_kernel<true> : t5_attn_dq_kernel<false>, grid_q, kAttnThreads, smem_q, st, c.p, "attn_bwd_dq", 3 * f);
+}
+}  // namespace
+
+extern "C" {
 
 int32_t td_t5_attention_fwd(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv, const int32_t* cu_q,
                             const int32_t* cu_k, int32_t B, int32_t H, int32_t inner, int32_t max_len_q, int32_t max_len_k, int64_t Mq,
@@ -1282,18 +1349,9 @@ int32_t td_t5_attention_fwd(const void* q, int64_t ldq, const void* k, int64_t l
                             td_stream_t stream) {
   TD_DEVICE_OR_RETURN();
   AttnCall c;
-  int rc = attn_check("td_t5_attention_fwd", q, ldq, k, ldk, v, ldv, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, Mq, self_attention,
-                      bias, n_dist, c);
-  if (rc) return rc;
-  if (!o) TD_FAIL(TD_ERR_ARG, "td_t5_attention_fwd: null pointer (o)");
-  if (misaligned16(o) || ldo % 8 || ldo < inner) TD_FAIL(TD_ERR_ARG, "td_t5_attention_fwd: o must be 16-byte aligned with a pitch that is a multiple of 8 and >= inner");
-  c.p.out = static_cast<__nv_bfloat16*>(o); c.p.ld_out = ldo; c.p.lse = lse;
-  cudaStream_t st = (cudaStream_t)stream;
-  const double flops = 4.0 * kAttnDk * H * attn_visible_pairs(c, st);
-  const dim3 grid(attn_tiles(max_len_q), H, B);
-  const int smem = attn_smem_bytes(AttnFwdSmem::kBias, c.p.n_dist);
-  return c.causal ? attn_launch(t5_attn_fwd_kernel<true>, grid, kAttnThreads, smem, st, c.p, "attn_fwd", flops)
-                  : attn_launch(t5_attn_fwd_kernel<false>, grid, kAttnThreads, smem, st, c.p, "attn_fwd", flops);
+  int rc = attn_fwd_check("td_t5_attention_fwd", q, ldq, k, ldk, v, ldv, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, Mq,
+                          self_attention, bias, n_dist, o, ldo, lse, c);
+  return rc ? rc : attn_fwd_run(c, (cudaStream_t)stream);
 }
 
 int32_t td_t5_attention_bwd(const void* dout, int64_t lddo, const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v,
@@ -1303,40 +1361,9 @@ int32_t td_t5_attention_bwd(const void* dout, int64_t lddo, const void* q, int64
                             void* ws, int64_t ws_bytes, td_stream_t stream) {
   TD_DEVICE_OR_RETURN();
   AttnCall c;
-  int rc = attn_check("td_t5_attention_bwd", q, ldq, k, ldk, v, ldv, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, Mq, self_attention,
-                      bias, n_dist, c);
-  if (rc) return rc;
-  if (!dout || !o || !lse || !dq || !dk || !dv) TD_FAIL(TD_ERR_ARG, "td_t5_attention_bwd: null pointer");
-  if (misaligned16(dout) || misaligned16(o) || misaligned16(dq) || misaligned16(dk) || misaligned16(dv))
-    TD_FAIL(TD_ERR_ARG, "td_t5_attention_bwd: dout / o / dq / dk / dv must be 16-byte aligned");
-  if (lddo % 8 || ldo % 8 || lddq % 8 || lddk % 8 || lddv % 8 || lddo < inner || ldo < inner || lddq < inner || lddk < inner || lddv < inner)
-    TD_FAIL(TD_ERR_ARG, "td_t5_attention_bwd: row pitches must be multiples of 8 and >= inner");
-  if (!ws || ws_bytes < td_t5_attention_workspace_bytes(Mq, H)) TD_FAIL(TD_ERR_ARG, "td_t5_attention_bwd: workspace too small");
-  c.p.dout = static_cast<const __nv_bfloat16*>(dout); c.p.lddo = lddo;
-  c.p.o = static_cast<const __nv_bfloat16*>(o); c.p.ldo = ldo;
-  c.p.lse = const_cast<float*>(lse);
-  c.p.delta = static_cast<float*>(ws);
-  c.p.dq = static_cast<__nv_bfloat16*>(dq); c.p.lddq = lddq;
-  c.p.dk = static_cast<__nv_bfloat16*>(dk); c.p.lddk = lddk;
-  c.p.dv = static_cast<__nv_bfloat16*>(dv); c.p.lddv = lddv;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (B == 0) return TD_OK;
-  const double pairs = attn_visible_pairs(c, st);
-  const long long delta_threads = Mq * H * 8;
-  rc = attn_launch(t5_attn_delta_kernel, dim3(unsigned((delta_threads + 255) / 256)), 256, 0, st, c.p, "attn_bwd_delta",
-                   double(Mq) * H * (4.0 * kAttnDk + 4.0));
-  if (rc) return rc;
-  const dim3 grid_k(attn_tiles(max_len_k), H, B), grid_q(attn_tiles(max_len_q), H, B);
-  const int smem_kv = attn_smem_bytes(AttnDkdvSmem::kBias, c.p.n_dist), smem_q = attn_smem_bytes(AttnDqSmem::kBias, c.p.n_dist);
-  const double f = 2.0 * kAttnDk * H * pairs;
-  if (c.causal) {
-    rc = attn_launch(t5_attn_dkdv_kernel<true>, grid_q, kAttnThreads, smem_kv, st, c.p, "attn_bwd_dkdv", 4 * f);
-    if (rc) return rc;
-    return attn_launch(t5_attn_dq_kernel<true>, grid_q, kAttnThreads, smem_q, st, c.p, "attn_bwd_dq", 3 * f);
-  }
-  rc = attn_launch(t5_attn_dkdv_kernel<false>, grid_k, kAttnThreads, smem_kv, st, c.p, "attn_bwd_dkdv", 4 * f);
-  if (rc) return rc;
-  return attn_launch(t5_attn_dq_kernel<false>, grid_q, kAttnThreads, smem_q, st, c.p, "attn_bwd_dq", 3 * f);
+  int rc = attn_bwd_check("td_t5_attention_bwd", dout, lddo, q, ldq, k, ldk, v, ldv, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, Mq,
+                          self_attention, bias, n_dist, o, ldo, lse, dq, lddq, dk, lddk, dv, lddv, ws, ws_bytes, c);
+  return rc ? rc : attn_bwd_run(c, (cudaStream_t)stream);
 }
 
 }  // extern "C"
@@ -1371,8 +1398,7 @@ int ffn_check_sizes(const char* fn, int64_t M, int32_t d, int32_t d_ff) {
 }
 int ffn_check_workspace(const char* fn, int64_t M, int32_t d, int32_t d_ff, void* ws, int64_t ws_bytes) {
   if (!ws || ws_bytes < (int64_t)carve_ffn(nullptr, M, d, d_ff).bytes) TD_FAIL(TD_ERR_ARG, "%s: workspace too small", fn);
-  if (misaligned16(ws)) TD_FAIL(TD_ERR_ARG, "%s: the workspace must be 16-byte aligned", fn);
-  return TD_OK;
+  return check_pointers(fn, {{"the workspace", ws, kOptionalAligned}});
 }
 
 // dx = bf16(dy + norm_bwd(dxn)): the backward of a T5 pre-norm sublayer's RMSNorm with the residual gradient folded in, one launch.
@@ -1380,7 +1406,7 @@ int ffn_check_workspace(const char* fn, int64_t M, int32_t d, int32_t d_ff, void
 int residual_norm_bwd_launch(const __nv_bfloat16* dxn, const void* x, const float* rstd, const float* ln_w, int64_t M, int32_t d,
                              const void* dy, void* dx, const char* tag, cudaStream_t st) {
   int rpc;
-  const int grid = norm_bwd_grid(M, &rpc);
+  const int grid = norm_grid(M, 2, &rpc);
   {
     ProfScope prof(tag, double(M) * d * 8.0, st);
     rmsnorm_bwd_kernel<true, true><<<grid, kNormBwdThreads, 0, st>>>(dxn, static_cast<const __nv_bfloat16*>(x), rstd, ln_w, int(M), d,
@@ -1404,29 +1430,20 @@ int32_t td_t5_ffn_fwd(const void* x, int64_t M, int32_t d, int32_t d_ff, const f
   if (M == 0) return TD_OK;
   rc = ffn_check_workspace("td_t5_ffn_fwd", M, d, d_ff, ws, ws_bytes);
   if (rc) return rc;
-  if (!x || !ln_w || !wi || !wo || !out || !rstd) TD_FAIL(TD_ERR_ARG, "td_t5_ffn_fwd: null pointer");
-  if (misaligned16(x) || misaligned16(ln_w) || misaligned16(wi) || misaligned16(wo) || misaligned16(out) || misaligned16(ab) ||
-      misaligned16(gated))
-    TD_FAIL(TD_ERR_ARG, "td_t5_ffn_fwd: x / ln_w / wi / wo / out / ab / gated must be 16-byte aligned");
+  rc = check_pointers("td_t5_ffn_fwd", {{"x", x}, {"ln_w", ln_w}, {"wi", wi}, {"wo", wo}, {"out", out}, {"rstd", rstd, kNonNull},
+                                        {"ab", ab, kOptionalAligned}, {"gated", gated, kOptionalAligned}});
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const FfnWorkspace w = carve_ffn(ws, M, d, d_ff);
   __nv_bfloat16* xn = w.rows;
   void* g = gated ? gated : w.pairs;
-  {
-    ProfScope prof("ffn_norm", double(M) * d * 4.0, st);
-    rc = rmsnorm_fwd_launch(x, ln_w, eps, M, d, xn, TD_DTYPE_BF16, rstd, st);
-  }
+  rc = rmsnorm_fwd_launch(x, nullptr, 0, ln_w, eps, M, d, xn, TD_DTYPE_BF16, rstd, "ffn_norm", st);
   if (rc) return rc;
-  GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.M = int(M); p.N = 2 * d_ff; p.K = d;
-  p.out0 = ab; p.out1 = g; p.ld_out = 2 * d_ff; p.alpha = 1.f;
+  GemmParams p = gemm_params(M, 2 * d_ff, d);
+  p.out0 = ab; p.out1 = g;
   rc = launch_gemm<2, false, false, EPI_GATED>({xn, d, false}, {wi, d, false}, p, w.sk, st, "gemm_ffn_gate");
   if (rc) return rc;
-  memset(&p, 0, sizeof(p));
-  p.M = int(M); p.N = d; p.K = d_ff;
-  p.out0 = out; p.aux0 = x; p.ld_out = d; p.alpha = 1.f;
-  return launch_gemm<2, false, false, EPI_RESIDUAL>({g, d_ff, false}, {wo, d_ff, false}, p, w.sk, st, "gemm_ffn_out");
+  return gemm_residual(g, M, d_ff, wo, d, x, out, w.sk, st, "gemm_ffn_out");
 }
 
 int32_t td_t5_ffn_bwd(const void* dy, const void* x, const float* rstd, const float* ln_w, const void* ab, const void* wi, const void* wo,
@@ -1437,24 +1454,19 @@ int32_t td_t5_ffn_bwd(const void* dy, const void* x, const float* rstd, const fl
   if (M == 0) return TD_OK;
   rc = ffn_check_workspace("td_t5_ffn_bwd", M, d, d_ff, ws, ws_bytes);
   if (rc) return rc;
-  if (!dy || !x || !rstd || !ln_w || !ab || !wi || !wo || !dx) TD_FAIL(TD_ERR_ARG, "td_t5_ffn_bwd: null pointer");
-  if (misaligned16(dy) || misaligned16(x) || misaligned16(ab) || misaligned16(wi) || misaligned16(wo) || misaligned16(dx) ||
-      misaligned16(d_ab))
-    TD_FAIL(TD_ERR_ARG, "td_t5_ffn_bwd: dy / x / ab / wi / wo / dx / d_ab must be 16-byte aligned");
+  rc = check_pointers("td_t5_ffn_bwd", {{"dy", dy}, {"x", x}, {"rstd", rstd, kNonNull}, {"ln_w", ln_w, kNonNull}, {"ab", ab}, {"wi", wi},
+                                        {"wo", wo}, {"dx", dx}, {"d_ab", d_ab, kOptionalAligned}});
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const FfnWorkspace w = carve_ffn(ws, M, d, d_ff);
   void* dab = d_ab ? d_ab : w.pairs;
   __nv_bfloat16* dxn = w.rows;
-  GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.M = int(M); p.N = d_ff; p.K = d;  // t = dy . wo, wo [d, d_ff] read MN-major in place
-  p.out0 = dab; p.aux0 = ab; p.ld_out = 2 * d_ff; p.alpha = 1.f;
+  GemmParams p = gemm_params(M, d_ff, d);  // t = dy . wo, wo [d, d_ff] read MN-major in place
+  p.out0 = dab; p.aux0 = ab; p.ld_out = 2 * d_ff;
   rc = launch_gemm<2, false, true, EPI_DGATED>({dy, d, false}, {wo, d_ff, true}, p, w.sk, st, "gemm_ffn_dgate");
   if (rc) return rc;
-  memset(&p, 0, sizeof(p));
-  p.M = int(M); p.N = d; p.K = 2 * d_ff;  // dxn = d_ab . wi, over the interleaved pair columns of both
-  p.out0 = dxn; p.ld_out = d; p.alpha = 1.f;
-  rc = launch_gemm<2, false, true, EPI_BF16>({dab, 2 * d_ff, false}, {wi, d, true}, p, w.sk, st, "gemm_ffn_dx");
+  // dxn = d_ab . wi, over the interleaved pair columns of both
+  rc = gemm_linear_dx(dab, M, 2 * d_ff, wi, d, dxn, false, w.sk, st, "gemm_ffn_dx");
   if (rc) return rc;
   return residual_norm_bwd_launch(dxn, x, rstd, ln_w, M, d, dy, dx, "ffn_norm_bwd", st);
 }
@@ -1505,38 +1517,7 @@ int attn_layer_check(const char* fn, int64_t M, int64_t Mk, int32_t d, int32_t H
   if (M == 0) return TD_OK;
   if (!ws || ws_bytes < (int64_t)carve_attn_layer(nullptr, M, Mk, d, H, self_attention).bytes)
     TD_FAIL(TD_ERR_ARG, "%s: workspace too small", fn);
-  if (misaligned16(ws)) TD_FAIL(TD_ERR_ARG, "%s: the workspace must be 16-byte aligned", fn);
-  return TD_OK;
-}
-
-// out = bf16(x + bf16(o . wo^T)), o [M, inner], wo [d, inner]: the closing projection of both attention sublayers
-int attn_out_gemm(const void* o, int32_t inner, const void* wo, const void* x, void* out, int64_t M, int32_t d, void* sk, cudaStream_t st,
-                  const char* tag) {
-  GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.M = int(M); p.N = d; p.K = inner;
-  p.out0 = out; p.aux0 = x; p.ld_out = d; p.alpha = 1.f;
-  return launch_gemm<2, false, false, EPI_RESIDUAL>({o, inner, false}, {wo, inner, false}, p, sk, st, tag);
-}
-
-// out [M, N] bf16 = bf16(a . w^T), w [N, K] read K-major (a projection)
-int proj_gemm(const void* a, int64_t M, int32_t K, const void* w, int32_t N, void* out, void* sk, cudaStream_t st, const char* tag) {
-  GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.M = int(M); p.N = N; p.K = K;
-  p.out0 = out; p.ld_out = N; p.alpha = 1.f;
-  return launch_gemm<2, false, false, EPI_BF16>({a, K, false}, {w, K, false}, p, sk, st, tag);
-}
-
-// out [M, N] = dy . w, dy [M, K], w [K, N] read MN-major in place (the input gradient of a projection): bf16, or fp32 when `f32`
-int proj_dx_gemm(const void* dy, int64_t M, int32_t K, const void* w, int32_t N, void* out, bool f32, void* sk, cudaStream_t st,
-                 const char* tag) {
-  GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.M = int(M); p.N = N; p.K = K;
-  p.out0 = out; p.ld_out = N; p.alpha = 1.f;
-  if (f32) return launch_gemm<2, false, true, EPI_F32>({dy, K, false}, {w, N, true}, p, sk, st, tag);
-  return launch_gemm<2, false, true, EPI_BF16>({dy, K, false}, {w, N, true}, p, sk, st, tag);
+  return check_pointers(fn, {{"the workspace", ws, kOptionalAligned}});
 }
 }  // namespace
 
@@ -1554,10 +1535,9 @@ int32_t td_t5_self_attention_layer_fwd(const void* x, int64_t M, int32_t d, int3
   const char* fn = "td_t5_self_attention_layer_fwd";
   int rc = attn_layer_check(fn, M, 0, d, H, true, ws, ws_bytes);
   if (rc || M == 0) return rc;
-  if (!x || !ln_w || !w_qkv || !wo || !out) TD_FAIL(TD_ERR_ARG, "%s: null pointer", fn);
-  if (misaligned16(x) || misaligned16(ln_w) || misaligned16(w_qkv) || misaligned16(wo) || misaligned16(out) || misaligned16(qkv) ||
-      misaligned16(o))
-    TD_FAIL(TD_ERR_ARG, "%s: x / ln_w / w_qkv / wo / out / qkv / o must be 16-byte aligned", fn);
+  rc = check_pointers(fn, {{"x", x}, {"ln_w", ln_w}, {"w_qkv", w_qkv}, {"wo", wo}, {"out", out}, {"qkv", qkv, kOptionalAligned},
+                           {"o", o, kOptionalAligned}});
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const int32_t inner = kAttnDk * H;
   const AttnLayerWorkspace w = carve_attn_layer(ws, M, 0, d, H, true);
@@ -1565,20 +1545,16 @@ int32_t td_t5_self_attention_layer_fwd(const void* x, int64_t M, int32_t d, int3
   void* o_ = o ? o : w.heads;
   float* rstd_ = rstd ? rstd : w.rstd;
   AttnCall c;  // the attention's own checks, before anything is enqueued
-  rc = attn_check(fn, qkv_, 3 * inner, qkv_ + inner, 3 * inner, qkv_ + 2 * inner, 3 * inner, cu_q, nullptr, B, H, inner, max_len, max_len, M,
-                  1, bias_by_distance, n_dist, c);
+  rc = attn_fwd_check(fn, qkv_, 3 * inner, qkv_ + inner, 3 * inner, qkv_ + 2 * inner, 3 * inner, cu_q, nullptr, B, H, inner, max_len,
+                      max_len, M, 1, bias_by_distance, n_dist, o_, inner, lse, c);
   if (rc) return rc;
-  {
-    ProfScope prof("sa_norm", double(M) * d * 4.0, st);
-    rc = rmsnorm_fwd_launch(x, ln_w, eps, M, d, w.rows, TD_DTYPE_BF16, rstd_, st);
-  }
+  rc = rmsnorm_fwd_launch(x, nullptr, 0, ln_w, eps, M, d, w.rows, TD_DTYPE_BF16, rstd_, "sa_norm", st);
   if (rc) return rc;
-  rc = proj_gemm(w.rows, M, d, w_qkv, 3 * inner, qkv_, w.sk, st, "gemm_sa_qkv");
+  rc = gemm_linear(w.rows, M, d, w_qkv, 3 * inner, nullptr, qkv_, w.sk, st, "gemm_sa_qkv");
   if (rc) return rc;
-  rc = td_t5_attention_fwd(qkv_, 3 * inner, qkv_ + inner, 3 * inner, qkv_ + 2 * inner, 3 * inner, cu_q, nullptr, B, H, inner, max_len, max_len,
-                           M, 1, bias_by_distance, n_dist, o_, inner, lse, stream);
+  rc = attn_fwd_run(c, st);
   if (rc) return rc;
-  return attn_out_gemm(o_, inner, wo, x, out, M, d, w.sk, st, "gemm_sa_out");
+  return gemm_residual(o_, M, inner, wo, d, x, out, w.sk, st, "gemm_sa_out");
 }
 
 int32_t td_t5_self_attention_layer_bwd(const void* dy, const void* x, const float* rstd, const float* ln_w, const void* qkv, const void* o,
@@ -1589,26 +1565,24 @@ int32_t td_t5_self_attention_layer_bwd(const void* dy, const void* x, const floa
   const char* fn = "td_t5_self_attention_layer_bwd";
   int rc = attn_layer_check(fn, M, 0, d, H, true, ws, ws_bytes);
   if (rc || M == 0) return rc;
-  if (!dy || !x || !rstd || !ln_w || !qkv || !o || !lse || !w_qkv || !wo || !dx) TD_FAIL(TD_ERR_ARG, "%s: null pointer", fn);
-  if (misaligned16(dy) || misaligned16(x) || misaligned16(ln_w) || misaligned16(qkv) || misaligned16(o) || misaligned16(w_qkv) ||
-      misaligned16(wo) || misaligned16(dx) || misaligned16(dqkv))
-    TD_FAIL(TD_ERR_ARG, "%s: dy / x / ln_w / qkv / o / w_qkv / wo / dx / dqkv must be 16-byte aligned", fn);
+  rc = check_pointers(fn, {{"dy", dy}, {"x", x}, {"rstd", rstd, kNonNull}, {"ln_w", ln_w}, {"qkv", qkv}, {"o", o}, {"lse", lse, kNonNull},
+                           {"w_qkv", w_qkv}, {"wo", wo}, {"dx", dx}, {"dqkv", dqkv, kOptionalAligned}});
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const int32_t inner = kAttnDk * H;
   const AttnLayerWorkspace w = carve_attn_layer(ws, M, 0, d, H, true);
   const __nv_bfloat16* q = static_cast<const __nv_bfloat16*>(qkv);
   __nv_bfloat16* dq = dqkv ? static_cast<__nv_bfloat16*>(dqkv) : w.proj;
   AttnCall c;
-  rc = attn_check(fn, q, 3 * inner, q + inner, 3 * inner, q + 2 * inner, 3 * inner, cu_q, nullptr, B, H, inner, max_len, max_len, M, 1,
-                  bias_by_distance, n_dist, c);
+  rc = attn_bwd_check(fn, w.heads, inner, q, 3 * inner, q + inner, 3 * inner, q + 2 * inner, 3 * inner, cu_q, nullptr, B, H, inner, max_len,
+                      max_len, M, 1, bias_by_distance, n_dist, o, inner, lse, dq, 3 * inner, dq + inner, 3 * inner, dq + 2 * inner,
+                      3 * inner, w.delta, w.delta_bytes, c);
   if (rc) return rc;
-  rc = proj_dx_gemm(dy, M, d, wo, inner, w.heads, false, w.sk, st, "gemm_sa_do");
+  rc = gemm_linear_dx(dy, M, d, wo, inner, w.heads, false, w.sk, st, "gemm_sa_do");
   if (rc) return rc;
-  rc = td_t5_attention_bwd(w.heads, inner, q, 3 * inner, q + inner, 3 * inner, q + 2 * inner, 3 * inner, cu_q, nullptr, B, H, inner, max_len,
-                           max_len, M, 1, bias_by_distance, n_dist, o, inner, lse, dq, 3 * inner, dq + inner, 3 * inner, dq + 2 * inner,
-                           3 * inner, w.delta, w.delta_bytes, stream);
+  rc = attn_bwd_run(c, st);
   if (rc) return rc;
-  rc = proj_dx_gemm(dq, M, 3 * inner, w_qkv, d, w.rows, false, w.sk, st, "gemm_sa_dx");
+  rc = gemm_linear_dx(dq, M, 3 * inner, w_qkv, d, w.rows, false, w.sk, st, "gemm_sa_dx");
   if (rc) return rc;
   return residual_norm_bwd_launch(w.rows, x, rstd, ln_w, M, d, dy, dx, "sa_norm_bwd", st);
 }
@@ -1621,10 +1595,10 @@ int32_t td_t5_cross_attention_layer_fwd(const void* x, int64_t M, const void* en
   const char* fn = "td_t5_cross_attention_layer_fwd";
   int rc = attn_layer_check(fn, M, Mk, d, H, false, ws, ws_bytes);
   if (rc || M == 0) return rc;
-  if (!x || (Mk > 0 && !enc) || !ln_w || !w_q || !w_kv || !wo || !out) TD_FAIL(TD_ERR_ARG, "%s: null pointer", fn);
-  if (misaligned16(x) || misaligned16(enc) || misaligned16(ln_w) || misaligned16(w_q) || misaligned16(w_kv) || misaligned16(wo) ||
-      misaligned16(out) || misaligned16(q) || misaligned16(kv) || misaligned16(o))
-    TD_FAIL(TD_ERR_ARG, "%s: x / enc / ln_w / w_q / w_kv / wo / out / q / kv / o must be 16-byte aligned", fn);
+  rc = check_pointers(fn, {{"x", x}, {"enc", enc, Mk > 0 ? kNonNullAligned : kOptionalAligned}, {"ln_w", ln_w}, {"w_q", w_q},
+                           {"w_kv", w_kv}, {"wo", wo}, {"out", out}, {"q", q, kOptionalAligned}, {"kv", kv, kOptionalAligned},
+                           {"o", o, kOptionalAligned}});
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const int32_t inner = kAttnDk * H;
   const AttnLayerWorkspace w = carve_attn_layer(ws, M, Mk, d, H, false);
@@ -1633,21 +1607,18 @@ int32_t td_t5_cross_attention_layer_fwd(const void* x, int64_t M, const void* en
   void* o_ = o ? o : w.heads;
   float* rstd_ = rstd ? rstd : w.rstd;
   AttnCall c;
-  rc = attn_check(fn, q_, inner, kv_, 2 * inner, kv_ + inner, 2 * inner, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, M, 0, nullptr, 0, c);
+  rc = attn_fwd_check(fn, q_, inner, kv_, 2 * inner, kv_ + inner, 2 * inner, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, M, 0, nullptr,
+                      0, o_, inner, lse, c);
   if (rc) return rc;
-  {
-    ProfScope prof("ca_norm", double(M) * d * 4.0, st);
-    rc = rmsnorm_fwd_launch(x, ln_w, eps, M, d, w.rows, TD_DTYPE_BF16, rstd_, st);
-  }
+  rc = rmsnorm_fwd_launch(x, nullptr, 0, ln_w, eps, M, d, w.rows, TD_DTYPE_BF16, rstd_, "ca_norm", st);
   if (rc) return rc;
-  rc = proj_gemm(w.rows, M, d, w_q, inner, q_, w.sk, st, "gemm_ca_q");
+  rc = gemm_linear(w.rows, M, d, w_q, inner, nullptr, q_, w.sk, st, "gemm_ca_q");
   if (rc) return rc;
-  rc = proj_gemm(enc, Mk, d, w_kv, 2 * inner, kv_, w.sk, st, "gemm_ca_kv");
+  rc = gemm_linear(enc, Mk, d, w_kv, 2 * inner, nullptr, kv_, w.sk, st, "gemm_ca_kv");
   if (rc) return rc;
-  rc = td_t5_attention_fwd(q_, inner, kv_, 2 * inner, kv_ + inner, 2 * inner, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, M, 0, nullptr, 0,
-                           o_, inner, lse, stream);
+  rc = attn_fwd_run(c, st);
   if (rc) return rc;
-  return attn_out_gemm(o_, inner, wo, x, out, M, d, w.sk, st, "gemm_ca_out");
+  return gemm_residual(o_, M, inner, wo, d, x, out, w.sk, st, "gemm_ca_out");
 }
 
 int32_t td_t5_cross_attention_layer_bwd(const void* dy, const void* x, const float* rstd, const float* ln_w, const void* q, const void* kv,
@@ -1658,26 +1629,25 @@ int32_t td_t5_cross_attention_layer_bwd(const void* dy, const void* x, const flo
   const char* fn = "td_t5_cross_attention_layer_bwd";
   int rc = attn_layer_check(fn, M, Mk, d, H, false, ws, ws_bytes);
   if (rc || M == 0) return rc;
-  if (!dy || !x || !rstd || !ln_w || !q || (Mk > 0 && !kv) || !o || !lse || !w_q || !w_kv || !wo || !dx || (Mk > 0 && !d_enc))
-    TD_FAIL(TD_ERR_ARG, "%s: null pointer", fn);
-  if (misaligned16(dy) || misaligned16(x) || misaligned16(ln_w) || misaligned16(q) || misaligned16(kv) || misaligned16(o) ||
-      misaligned16(w_q) || misaligned16(w_kv) || misaligned16(wo) || misaligned16(dx) || misaligned16(d_enc))
-    TD_FAIL(TD_ERR_ARG, "%s: dy / x / ln_w / q / kv / o / w_q / w_kv / wo / dx / d_enc must be 16-byte aligned", fn);
+  const PtrRule enc_rule = Mk > 0 ? kNonNullAligned : kOptionalAligned;  // Mk == 0: no key is read, no encoder gradient written
+  rc = check_pointers(fn, {{"dy", dy}, {"x", x}, {"rstd", rstd, kNonNull}, {"ln_w", ln_w}, {"q", q}, {"kv", kv, enc_rule}, {"o", o},
+                           {"lse", lse, kNonNull}, {"w_q", w_q}, {"w_kv", w_kv}, {"wo", wo}, {"dx", dx}, {"d_enc", d_enc, enc_rule}});
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const int32_t inner = kAttnDk * H;
   const AttnLayerWorkspace w = carve_attn_layer(ws, M, Mk, d, H, false);
   const __nv_bfloat16* k = kv ? static_cast<const __nv_bfloat16*>(kv) : w.proj;  // Mk == 0: no key is read
   AttnCall c;
-  rc = attn_check(fn, q, inner, k, 2 * inner, k + inner, 2 * inner, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, M, 0, nullptr, 0, c);
+  rc = attn_bwd_check(fn, w.heads, inner, q, inner, k, 2 * inner, k + inner, 2 * inner, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, M, 0,
+                      nullptr, 0, o, inner, lse, w.q, inner, w.proj, 2 * inner, w.proj + inner, 2 * inner, w.delta, w.delta_bytes, c);
   if (rc) return rc;
-  rc = proj_dx_gemm(dy, M, d, wo, inner, w.heads, false, w.sk, st, "gemm_ca_do");
+  rc = gemm_linear_dx(dy, M, d, wo, inner, w.heads, false, w.sk, st, "gemm_ca_do");
   if (rc) return rc;
-  rc = td_t5_attention_bwd(w.heads, inner, q, inner, k, 2 * inner, k + inner, 2 * inner, cu_q, cu_k, B, H, inner, max_len_q, max_len_k, M, 0,
-                           nullptr, 0, o, inner, lse, w.q, inner, w.proj, 2 * inner, w.proj + inner, 2 * inner, w.delta, w.delta_bytes, stream);
+  rc = attn_bwd_run(c, st);
   if (rc) return rc;
-  rc = proj_dx_gemm(w.q, M, inner, w_q, d, w.rows, false, w.sk, st, "gemm_ca_dq");
+  rc = gemm_linear_dx(w.q, M, inner, w_q, d, w.rows, false, w.sk, st, "gemm_ca_dq");
   if (rc) return rc;
-  rc = proj_dx_gemm(w.proj, Mk, 2 * inner, w_kv, d, d_enc, true, w.sk, st, "gemm_ca_denc");
+  rc = gemm_linear_dx(w.proj, Mk, 2 * inner, w_kv, d, d_enc, true, w.sk, st, "gemm_ca_denc");
   if (rc) return rc;
   return residual_norm_bwd_launch(w.rows, x, rstd, ln_w, M, d, dy, dx, "ca_norm_bwd", st);
 }
