@@ -388,6 +388,27 @@ int32_t td_t5_cross_attention_layer_bwd(const void* dy, const void* x, const flo
                                         const int32_t* cu_k, int32_t B, int32_t max_len_q, int32_t max_len_k, int64_t M, int64_t Mk, int32_t d,
                                         int32_t H, void* dx, float* d_enc /* [Mk, d] fp32 */, void* workspace, int64_t workspace_bytes,
                                         td_stream_t stream);
+/* The same backward with d_enc ADDED to instead of overwritten (d_enc += dkv . [Wk; Wv], one fp32 TMA reduce-add per output tile
+ * of the d_enc GEMM): the encoder gradient of a decoder stack summed over its blocks in one [Mk, d] buffer, the last block (the first
+ * one run backward) overwriting it with td_t5_cross_attention_layer_bwd and every earlier block adding into it. Same arguments,
+ * launches and profiling tags. */
+int32_t td_t5_cross_attention_layer_bwd_accumulate(const void* dy, const void* x, const float* rstd, const float* ln_w, const void* q,
+                                                   const void* kv, const void* o, const float* lse, const void* w_q, const void* w_kv,
+                                                   const void* wo, const int32_t* cu_q, const int32_t* cu_k, int32_t B, int32_t max_len_q,
+                                                   int32_t max_len_k, int64_t M, int64_t Mk, int32_t d, int32_t H, void* dx,
+                                                   float* d_enc /* [Mk, d] fp32, added to */, void* workspace, int64_t workspace_bytes,
+                                                   td_stream_t stream);
+
+/* ---- the T5 decoder's inputs from the labels, on PACKED rows ---------------------------------------------------------------------
+ * transformers' T5 `_shift_right(labels)` followed by `embed_tokens` (T5ForConditionalGeneration.forward with labels and no
+ * decoder_input_ids), per sample: row r of sample b (r in [cu_q[b], cu_q[b+1]), cu_q[B] == Mq) is embed[id] with
+ *   id = decoder_start_token_id if r == cu_q[b], else labels[r - 1];   id == -100 -> pad_token_id.
+ * labels int64 [Mq] (the packed labels, -100 = ignored by the loss), embed bf16 [V, d], rows bf16 [Mq, d]; d % 8 == 0, buffers
+ * 16-byte aligned (labels and cu_q: non-null). An id outside [0, V) gives a zero row: the table is never read out of bounds (the
+ * Python layer rejects such labels before they get here). One launch (programmatic dependent launch); profiling tag
+ * t5_decoder_inputs (bytes). Mq == 0 does nothing. */
+int32_t td_t5_decoder_inputs(const int64_t* labels, const int32_t* cu_q, int32_t B, int64_t Mq, const void* embed, int64_t V, int32_t d,
+                             int64_t decoder_start_token_id, int64_t pad_token_id, void* rows, td_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -12,12 +12,13 @@ from . import ops  # noqa: E402
 from .aligner import FUSED_TYPE, ThinkDiffAligner, build_vision_projector  # noqa: E402
 from .loss import frozen_linear, lm_head_cross_entropy, masked_cross_entropy, masked_mse  # noqa: E402
 from .pack import FlatBatch, FlatCollater, PackedBatch, compose_image_text, kept_lengths, pack_batch, pack_device  # noqa: E402
-from .train_step import AlignerTrainStep, synthetic_lvlm_batch  # noqa: E402
+from .train_step import AlignerT5TrainStep, AlignerTrainStep, synthetic_lvlm_batch  # noqa: E402
 from .optim import DeviceGradScaler, FusedAdamW  # noqa: E402
 from .shards import EmbedShardReader, EmbedShardSet, EmbedShardWriter, convert_webdataset_shards, iter_webdataset_samples  # noqa: E402
 from .lr_schedule import LinearWarmupCosineLRScheduler, LinearWarmupStepLRScheduler, get_lr_scheduler_class  # noqa: E402
-from .t5 import (T5DecoderBlockWeights, T5DecoderWeights, T5FeedForwardWeights, t5_attention, t5_decoder_block, t5_decoder_stack,  # noqa: E402
-                 t5_layer_cross_attention, t5_layer_ff, t5_layer_self_attention, t5_position_bias_by_distance)
+from .t5 import (T5DecoderBlockWeights, T5DecoderWeights, T5FeedForwardWeights, T5ForDecoderWeights, pack_labels, t5_attention,  # noqa: E402
+                 t5_decoder_block, t5_decoder_loss, t5_decoder_stack, t5_layer_cross_attention, t5_layer_ff, t5_layer_self_attention,
+                 t5_position_bias_by_distance)
 
 __all__ = [
     "ops", "ThinkDiffAligner", "build_vision_projector", "FUSED_TYPE", "masked_mse", "masked_cross_entropy", "lm_head_cross_entropy", "frozen_linear",
@@ -25,5 +26,5 @@ __all__ = [
     "synthetic_lvlm_batch", "FusedAdamW", "DeviceGradScaler", "EmbedShardReader", "EmbedShardSet", "EmbedShardWriter", "convert_webdataset_shards", "iter_webdataset_samples", "LinearWarmupCosineLRScheduler",
     "LinearWarmupStepLRScheduler", "get_lr_scheduler_class", "t5_attention", "t5_position_bias_by_distance", "t5_layer_ff",
     "T5FeedForwardWeights", "T5DecoderBlockWeights", "T5DecoderWeights", "t5_layer_self_attention", "t5_layer_cross_attention",
-    "t5_decoder_block", "t5_decoder_stack",
+    "t5_decoder_block", "t5_decoder_stack", "T5ForDecoderWeights", "pack_labels", "t5_decoder_loss", "AlignerT5TrainStep",
 ]

@@ -64,6 +64,9 @@ SIGNATURES = {
                                                _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
     "td_t5_cross_attention_layer_bwd": (_i32, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i64, _i64,
                                                _i32, _i32, _vp, _vp, _vp, _i64, _vp]),
+    "td_t5_cross_attention_layer_bwd_accumulate": (_i32, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32,
+                                                          _i64, _i64, _i32, _i32, _vp, _vp, _vp, _i64, _vp]),
+    "td_t5_decoder_inputs": (_i32, [_vp, _vp, _i32, _i64, _vp, _i64, _i32, _i64, _i64, _vp, _vp]),
     "td_gemm_bf16_f32out": (_i32, [_vp, _i64, _i32, _vp, _i64, _i32, _i64, _i32, _i64, _f32, _vp, _i32, _i32, _vp, _i64, _vp]),
     "td_adamw_step": (_i32, [_i32, _vp, _vp, _vp, _vp, _vp, C.POINTER(_i64), C.POINTER(_f32), _f32, _f32, _f32, _f32, _i64, _f32, _vp, _vp]),
     "td_step_ctl_bytes": (_i64, []),

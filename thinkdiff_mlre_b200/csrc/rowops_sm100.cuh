@@ -178,6 +178,58 @@ pack_rows_kernel(const uint4* __restrict__ src, const long long* __restrict__ sr
   }
 }
 
+// ------------------------------------------------------------------------------------------ T5 decoder inputs
+// transformers' T5 `_shift_right` followed by `embed_tokens`, on packed rows: destination row r of sample i (r in [cu[i], cu[i+1]))
+// <- embed[id], id = start_id if r == cu[i] else labels[r - 1], with -100 (the loss's ignore index) replaced by pad_id. The
+// launch shape is pack_rows_kernel's: one warp per row, 128-bit accesses, 8 loads in flight per lane. An id outside [0, V) gives a
+// zero row: the table is never read out of bounds (the host layer rejects such ids before they arrive).
+__global__ void __launch_bounds__(256)
+t5_decoder_inputs_kernel(const long long* __restrict__ labels, const int* __restrict__ cu, int B, long long rows,
+                         const uint4* __restrict__ embed, long long V, int vec_per_row, long long start_id, long long pad_id,
+                         uint4* __restrict__ dst) {
+  grid_dependency_wait();  // launched with programmatic dependent launch: nothing global before this
+  grid_launch_dependents();
+  __shared__ int s_cu[kPackMaxStagedSeqs + 1];
+  const bool staged = B <= kPackMaxStagedSeqs;
+  if (staged) {
+    for (int i = threadIdx.x; i <= B; i += blockDim.x) s_cu[i] = cu[i];
+    __syncthreads();
+  }
+  const int* cu_t = staged ? s_cu : cu;
+  const int lane = threadIdx.x & 31;
+  const long long warp0 = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const long long nwarps = (long long)gridDim.x * (blockDim.x >> 5);
+  for (long long r = warp0; r < rows; r += nwarps) {
+    int lo = 0, hi = B;  // largest i with cu[i] <= r
+    while (hi - lo > 1) {
+      const int mid = (lo + hi) >> 1;
+      if ((long long)cu_t[mid] <= r) lo = mid; else hi = mid;
+    }
+    long long id = r == (long long)cu_t[lo] ? start_id : labels[r - 1];
+    if (id == -100) id = pad_id;
+    uint4* d = dst + r * vec_per_row;
+    if (id >= 0 && id < V) {
+      const uint4* s = embed + id * vec_per_row;
+      for (int v0 = 0; v0 < vec_per_row; v0 += 256) {
+        uint4 t[8];
+#pragma unroll
+        for (int u = 0; u < 8; ++u) {
+          const int v = v0 + u * 32 + lane;
+          if (v < vec_per_row) t[u] = __ldg(s + v);
+        }
+#pragma unroll
+        for (int u = 0; u < 8; ++u) {
+          const int v = v0 + u * 32 + lane;
+          if (v < vec_per_row) d[v] = t[u];
+        }
+      }
+    } else {
+      const uint4 z = make_uint4(0, 0, 0, 0);
+      for (int v = lane; v < vec_per_row; v += 32) d[v] = z;
+    }
+  }
+}
+
 // ------------------------------------------------------------------------------------------ casts
 __global__ void __launch_bounds__(256)
 cast_f32_to_bf16_kernel(const float* __restrict__ src, __nv_bfloat16* __restrict__ dst, long long n) {

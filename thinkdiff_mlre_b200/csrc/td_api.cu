@@ -347,11 +347,12 @@ int gemm_linear(const void* a, int64_t M, int32_t K, const void* w, int32_t N, c
   return launch_gemm<2, false, false, EPI_BF16>({a, K, false}, {w, K, false}, p, sk, st, tag);
 }
 
-// out [M, N] = a . w, w [K, N] read MN-major in place (the input gradient of a linear layer): bf16, or fp32 when `f32`
+// out [M, N] = a . w, w [K, N] read MN-major in place (the input gradient of a linear layer): bf16, or fp32 when `f32`;
+// `accumulate` (fp32 only): out += a . w by TMA reduce-add
 int gemm_linear_dx(const void* a, int64_t M, int64_t K, const void* w, int32_t N, void* out, bool f32, void* sk, cudaStream_t st,
-                   const char* tag) {
+                   const char* tag, bool accumulate = false) {
   GemmParams p = gemm_params(M, N, K);
-  p.out0 = out;
+  p.out0 = out; p.accumulate = accumulate;
   if (f32) return launch_gemm<2, false, true, EPI_F32>({a, K, false}, {w, N, true}, p, sk, st, tag);
   return launch_gemm<2, false, true, EPI_BF16>({a, K, false}, {w, N, true}, p, sk, st, tag);
 }
@@ -1621,12 +1622,15 @@ int32_t td_t5_cross_attention_layer_fwd(const void* x, int64_t M, const void* en
   return gemm_residual(o_, M, inner, wo, d, x, out, w.sk, st, "gemm_ca_out");
 }
 
-int32_t td_t5_cross_attention_layer_bwd(const void* dy, const void* x, const float* rstd, const float* ln_w, const void* q, const void* kv,
-                                        const void* o, const float* lse, const void* w_q, const void* w_kv, const void* wo, const int32_t* cu_q,
-                                        const int32_t* cu_k, int32_t B, int32_t max_len_q, int32_t max_len_k, int64_t M, int64_t Mk, int32_t d,
-                                        int32_t H, void* dx, float* d_enc, void* ws, int64_t ws_bytes, td_stream_t stream) {
+}  // extern "C"
+
+namespace {
+// The two cross-attention backward entries: `accumulate` adds the encoder gradient into d_enc instead of overwriting it.
+int cross_attention_layer_bwd(const char* fn, bool accumulate, const void* dy, const void* x, const float* rstd, const float* ln_w,
+                              const void* q, const void* kv, const void* o, const float* lse, const void* w_q, const void* w_kv, const void* wo,
+                              const int32_t* cu_q, const int32_t* cu_k, int32_t B, int32_t max_len_q, int32_t max_len_k, int64_t M, int64_t Mk,
+                              int32_t d, int32_t H, void* dx, float* d_enc, void* ws, int64_t ws_bytes, td_stream_t stream) {
   TD_DEVICE_OR_RETURN();
-  const char* fn = "td_t5_cross_attention_layer_bwd";
   int rc = attn_layer_check(fn, M, Mk, d, H, false, ws, ws_bytes);
   if (rc || M == 0) return rc;
   const PtrRule enc_rule = Mk > 0 ? kNonNullAligned : kOptionalAligned;  // Mk == 0: no key is read, no encoder gradient written
@@ -1647,9 +1651,49 @@ int32_t td_t5_cross_attention_layer_bwd(const void* dy, const void* x, const flo
   if (rc) return rc;
   rc = gemm_linear_dx(w.q, M, inner, w_q, d, w.rows, false, w.sk, st, "gemm_ca_dq");
   if (rc) return rc;
-  rc = gemm_linear_dx(w.proj, Mk, 2 * inner, w_kv, d, d_enc, true, w.sk, st, "gemm_ca_denc");
+  rc = gemm_linear_dx(w.proj, Mk, 2 * inner, w_kv, d, d_enc, true, w.sk, st, "gemm_ca_denc", accumulate);
   if (rc) return rc;
   return residual_norm_bwd_launch(w.rows, x, rstd, ln_w, M, d, dy, dx, "ca_norm_bwd", st);
+}
+}  // namespace
+
+extern "C" {
+
+int32_t td_t5_cross_attention_layer_bwd(const void* dy, const void* x, const float* rstd, const float* ln_w, const void* q, const void* kv,
+                                        const void* o, const float* lse, const void* w_q, const void* w_kv, const void* wo, const int32_t* cu_q,
+                                        const int32_t* cu_k, int32_t B, int32_t max_len_q, int32_t max_len_k, int64_t M, int64_t Mk, int32_t d,
+                                        int32_t H, void* dx, float* d_enc, void* ws, int64_t ws_bytes, td_stream_t stream) {
+  return cross_attention_layer_bwd("td_t5_cross_attention_layer_bwd", false, dy, x, rstd, ln_w, q, kv, o, lse, w_q, w_kv, wo, cu_q, cu_k, B,
+                                   max_len_q, max_len_k, M, Mk, d, H, dx, d_enc, ws, ws_bytes, stream);
+}
+
+int32_t td_t5_cross_attention_layer_bwd_accumulate(const void* dy, const void* x, const float* rstd, const float* ln_w, const void* q,
+                                                   const void* kv, const void* o, const float* lse, const void* w_q, const void* w_kv,
+                                                   const void* wo, const int32_t* cu_q, const int32_t* cu_k, int32_t B, int32_t max_len_q,
+                                                   int32_t max_len_k, int64_t M, int64_t Mk, int32_t d, int32_t H, void* dx, float* d_enc,
+                                                   void* ws, int64_t ws_bytes, td_stream_t stream) {
+  return cross_attention_layer_bwd("td_t5_cross_attention_layer_bwd_accumulate", true, dy, x, rstd, ln_w, q, kv, o, lse, w_q, w_kv, wo, cu_q,
+                                   cu_k, B, max_len_q, max_len_k, M, Mk, d, H, dx, d_enc, ws, ws_bytes, stream);
+}
+
+// ------------------------------------------------------------------------------------------------ T5 decoder inputs
+int32_t td_t5_decoder_inputs(const int64_t* labels, const int32_t* cu_q, int32_t B, int64_t Mq, const void* embed, int64_t V, int32_t d,
+                             int64_t decoder_start_token_id, int64_t pad_token_id, void* rows, td_stream_t stream) {
+  TD_DEVICE_OR_RETURN();
+  const char* fn = "td_t5_decoder_inputs";
+  if (B < 0 || Mq < 0 || V <= 0 || d <= 0 || d % 8)
+    TD_FAIL(TD_ERR_ARG, "%s: bad sizes (B=%d Mq=%lld V=%lld d=%d; d must be a positive multiple of 8)", fn, B, (long long)Mq, (long long)V, d);
+  if (Mq == 0) return TD_OK;
+  if (B == 0) TD_FAIL(TD_ERR_ARG, "%s: Mq=%lld rows but no sample", fn, (long long)Mq);
+  int rc = check_pointers(fn, {{"labels", labels, kNonNull}, {"cu_q", cu_q, kNonNull}, {"embed", embed}, {"rows", rows}});
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  ProfScope prof("t5_decoder_inputs", 4.0 * double(Mq) * d + 8.0 * double(Mq), st);
+  PdlConfig l(grid_for_rows(Mq, 8, 8), 256, st);
+  TD_CUDA(cudaLaunchKernelEx(&l.cfg, t5_decoder_inputs_kernel, reinterpret_cast<const long long*>(labels), cu_q, B, (long long)Mq,
+                             static_cast<const uint4*>(embed), (long long)V, d / 8, (long long)decoder_start_token_id,
+                             (long long)pad_token_id, static_cast<uint4*>(rows)));
+  return TD_OK;
 }
 
 }  // extern "C"

@@ -712,10 +712,11 @@ def t5_cross_attention_layer_fwd(x, enc, w_q, w_kv, wo, ln_w, eps: float, cu_q, 
 
 
 def t5_cross_attention_layer_bwd(dy, x, rstd, q, kv, o, lse, w_q, w_kv, wo, ln_w, cu_q, cu_k, max_len_q: int, max_len_k: int,
-                                 n_heads: int):
+                                 n_heads: int, d_enc_accumulate=None):
     """Gradients of ``t5_cross_attention_layer_fwd`` (frozen weights) from ``dy [M, d]`` bf16 and the forward's saved tensors. Returns
-    ``(dx [M, d] bf16, d_enc [Mk, d] fp32)``: ``d_enc = dkv . [Wk; Wv]`` summed in fp32 and not rounded. Seven launches;
-    deterministic."""
+    ``(dx [M, d] bf16, d_enc [Mk, d] fp32)``: ``d_enc = dkv . [Wk; Wv]`` summed in fp32 and not rounded. ``d_enc_accumulate`` (fp32
+    [Mk, d]): add ``d_enc`` into this buffer (one fp32 reduce-add per element) and return it, instead of a fresh one -- the encoder
+    gradient of a stack summed over its blocks. Seven launches; deterministic."""
     M, d, inner = _attn_layer_dims(x, ln_w, wo, n_heads)
     _proj_weight(w_q, inner, d, "w_q")
     _proj_weight(w_kv, 2 * inner, d, "w_kv")
@@ -731,12 +732,90 @@ def t5_cross_attention_layer_bwd(dy, x, rstd, q, kv, o, lse, w_q, w_kv, wo, ln_w
     _saved(lse, (n_heads, M), torch.float32, "lse")
     dev = x.device
     dx = torch.empty((M, d), dtype=torch.bfloat16, device=dev)
-    d_enc = torch.empty((Mk, d), dtype=torch.float32, device=dev)
+    if d_enc_accumulate is None:
+        d_enc, entry = torch.empty((Mk, d), dtype=torch.float32, device=dev), "td_t5_cross_attention_layer_bwd"
+    else:
+        _need_cuda(d_enc_accumulate)
+        d_enc, entry = _saved(d_enc_accumulate, (Mk, d), torch.float32, "d_enc_accumulate"), "td_t5_cross_attention_layer_bwd_accumulate"
     ws, ws_bytes = _layer_ws(M, Mk, d, n_heads, False, dev)
     L.launch_count += 7
-    L.check(L.lib().td_t5_cross_attention_layer_bwd(L.ptr(dy), L.ptr(x), L.ptr(rstd), L.ptr(ln_w), L.ptr(q), L.ptr(kv), L.ptr(o), L.ptr(lse),
-                                                    L.ptr(w_q), L.ptr(w_kv), L.ptr(wo), L.ptr(cu_q), L.ptr(cu_k), cu_q.numel() - 1,
-                                                    int(max_len_q), int(max_len_k), M, Mk, d, n_heads, L.ptr(dx),
-                                                    L.ptr(d_enc), L.ptr(ws), ws_bytes, L.stream_ptr()),
-            "td_t5_cross_attention_layer_bwd")
+    L.check(getattr(L.lib(), entry)(L.ptr(dy), L.ptr(x), L.ptr(rstd), L.ptr(ln_w), L.ptr(q), L.ptr(kv), L.ptr(o), L.ptr(lse), L.ptr(w_q),
+                                    L.ptr(w_kv), L.ptr(wo), L.ptr(cu_q), L.ptr(cu_k), cu_q.numel() - 1, int(max_len_q), int(max_len_k), M, Mk,
+                                    d, n_heads, L.ptr(dx), L.ptr(d_enc), L.ptr(ws), ws_bytes, L.stream_ptr()), entry)
     return dx, d_enc
+
+
+# ------------------------------------------------------------------------------------------------ T5 objective (decoder inputs -> CE)
+def t5_decoder_inputs(labels, cu_q, embed, decoder_start_token_id: int, pad_token_id: int):
+    """The decoder's input rows from the packed labels: transformers' ``_shift_right`` + ``embed_tokens`` per sample. ``labels`` int64
+    [Mq] (-100 = ignored), ``cu_q`` int32 [B + 1] with ``cu_q[B] == Mq``, ``embed`` bf16 [V, d]. Returns bf16 [Mq, d]: row ``cu_q[b]``
+    is ``embed[decoder_start_token_id]``, row r > cu_q[b] is ``embed[labels[r - 1]]``, -100 read as ``pad_token_id``. An id outside
+    [0, V) gives a zero row (``t5.pack_labels`` rejects such labels). One launch."""
+    _need_cuda(labels, cu_q, embed)
+    if labels.dtype != torch.int64 or labels.dim() != 1 or cu_q.dtype != torch.int32:
+        raise TypeError("t5_decoder_inputs: labels must be int64 [Mq] and cu_q int32 [B + 1]")
+    if embed.dtype != torch.bfloat16 or embed.dim() != 2:
+        raise TypeError("t5_decoder_inputs: embed must be bfloat16 [V, d]")
+    _contig(labels, "labels")
+    _contig(cu_q, "cu_q")
+    _contig(embed, "embed")
+    V, d = embed.shape
+    Mq = labels.numel()
+    rows = torch.empty((Mq, d), dtype=torch.bfloat16, device=embed.device)
+    L.launch_count += 1
+    L.check(L.lib().td_t5_decoder_inputs(L.ptr(labels), L.ptr(cu_q), cu_q.numel() - 1, Mq, L.ptr(embed), V, d, int(decoder_start_token_id),
+                                         int(pad_token_id), L.ptr(rows), L.stream_ptr()), "td_t5_decoder_inputs")
+    return rows
+
+
+def t5_decoder_loss_fwd_bwd(enc, cu_k, max_len_k: int, labels, cu_q, max_len_q: int, weights, grad_scale: float = 1.0,
+                            want_grad: bool = True):
+    """The reference's objective (``T5ForDecoder.forward``, thinkdiff/models/mllama_vllm_t5_embed_decoder_2.py:211-246) on packed rows,
+    forward and the gradient into the aligner rows as one direct call sequence, without autograd. ``enc`` [Mk, d] fp32 or bf16 (the
+    aligner output, samples ``cu_k``), ``labels`` int64 [Mq] packed by ``t5.pack_labels`` (samples ``cu_q``), ``weights`` a
+    ``t5.T5ForDecoderWeights``. Returns ``(loss fp32 scalar, d_enc fp32 [Mk, d] or None)``, ``d_enc`` being the gradient of the loss with
+    respect to ``enc`` times ``grad_scale`` -- which ``lm_head_ce`` folds into its softmax exponent, so a scale other than 1 also moves
+    roundings of the logits' gradient (an exact power-of-two loss scale belongs after this call, as in ``AlignerT5TrainStep``).
+
+    Order: ``enc`` cast to bf16 once; decoder inputs; every block forward, keeping what its backward takes (block 0's self-attention
+    keeps nothing: its input gradient would only reach the frozen embedding); final norm; ``lm_head_ce``; final-norm backward; the
+    blocks in reverse, each block's saved tensors dropped once its backward is enqueued. The blocks' encoder gradients are summed in
+    one fp32 buffer: the last block overwrites it and every earlier block adds into it, last to first."""
+    dec = weights.decoder
+    _need_cuda(enc, cu_k, labels, cu_q)
+    if enc.dim() != 2 or enc.shape[1] != dec.blocks[0].d or enc.dtype not in (torch.float32, torch.bfloat16):
+        raise TypeError(f"enc must be float32 or bfloat16 [Mk, {dec.blocks[0].d}], got {enc.dtype} {tuple(enc.shape)}")
+    if labels.numel() == 0:
+        raise ValueError("t5_decoder_loss: no decoder rows (every label is -100); the loss is undefined")
+    e2 = cast_to_bf16(_contig(enc, "enc")) if enc.dtype == torch.float32 else _contig(enc, "enc")
+    bias = dec.position_bias
+    h = t5_decoder_inputs(labels, cu_q, weights.embed, weights.decoder_start_token_id, weights.pad_token_id)
+    saved = []
+    for i, bw in enumerate(dec.blocks):
+        sa_saved = want_grad and i > 0
+        h1, *sa = t5_self_attention_layer_fwd(h, bw.w_qkv, bw.wo_self, bw.ln_self, bw.eps, bias, cu_q, max_len_q, bw.n_heads,
+                                              want_saved=sa_saved)
+        h2, *ca = t5_cross_attention_layer_fwd(h1, e2, bw.w_q, bw.w_kv, bw.wo_cross, bw.ln_cross, bw.eps, cu_q, cu_k, max_len_q, max_len_k,
+                                               bw.n_heads, want_saved=want_grad)
+        h3, rstd, ab, _ = t5_ffn_fwd(h2, bw.ffn.wi, bw.ffn.wo, bw.ffn.ln_weight, bw.ffn.eps, want_ab=want_grad)
+        if want_grad:
+            saved.append((h if sa_saved else None, sa, h1, ca, h2, rstd, ab))
+        h = h3
+    seq, rstd_f = rmsnorm_fwd(h, dec.final_ln, dec.eps, out_bf16=True)
+    loss, dseq, _ = lm_head_ce(seq, weights.lm_head, labels, grad_scale, want_grad=want_grad)
+    if not want_grad:
+        return loss, None
+    del seq
+    dh, _, _ = rmsnorm_bwd(dseq, h, rstd_f, dec.final_ln, want_dg=False, want_dxsum=False)
+    del dseq, h
+    d_enc = None
+    for i in range(len(dec.blocks) - 1, -1, -1):
+        bw = dec.blocks[i]
+        h_in, sa, h1, ca, h2, rstd, ab = saved.pop()
+        dh, _ = t5_ffn_bwd(dh, h2, rstd, ab, bw.ffn.wi, bw.ffn.wo, bw.ffn.ln_weight)
+        dh, d_enc = t5_cross_attention_layer_bwd(dh, h1, *ca, bw.w_q, bw.w_kv, bw.wo_cross, bw.ln_cross, cu_q, cu_k, max_len_q, max_len_k,
+                                                 bw.n_heads, d_enc_accumulate=d_enc)
+        if i > 0:
+            dh, _ = t5_self_attention_layer_bwd(dh, h_in, *sa, bw.w_qkv, bw.wo_self, bw.ln_self, bias, cu_q, max_len_q, bw.n_heads)
+        del h_in, sa, h1, ca, h2, rstd, ab
+    return loss, d_enc

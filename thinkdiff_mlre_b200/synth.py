@@ -49,3 +49,20 @@ def lvlm_batch_tensors(num_seqs: int, max_len: int, din: int, d: int, seed: int,
     """One whole batch of ``num_seqs`` sequences (a single rank's view when the global batch is not sharded)."""
     lens = global_lengths(num_seqs, max_len, seed)
     return lvlm_sequences(range(num_seqs), lens, din, d, seed, with_target, truncated)
+
+
+EOS_ID = 1  # T5's </s>
+
+
+def t5_labels(num_seqs: int, vocab_size: int, seed: int, min_len: int = 8, max_len: int = 128) -> torch.Tensor:
+    """Seeded caption labels in the tokenizer's layout: int64 ``[num_seqs, T]``, sample i holds ``len_i ~ U{min_len..max_len}`` ids
+    (``max_len`` 128 is the reference's ``max_txt_len``), the last one EOS (1), the others ``U{2..vocab_size - 1}``, then -100 up to
+    ``T = max len_i`` (what the reference's ``targets.masked_fill(pad, -100)`` leaves)."""
+    g = torch.Generator().manual_seed(seed)
+    lens = torch.randint(min_len, max_len + 1, (num_seqs,), generator=g)
+    T = int(lens.max())
+    labels = torch.randint(2, vocab_size, (num_seqs, T), generator=g, dtype=torch.int64)
+    pos = torch.arange(T)[None, :]
+    labels[pos == lens[:, None] - 1] = EOS_ID
+    labels[pos >= lens[:, None]] = -100
+    return labels

@@ -389,3 +389,118 @@ def t5_decoder_stack(dec_rows: torch.Tensor, enc: torch.Tensor, cu_q: torch.Tens
     for bw in weights.blocks:
         h = t5_decoder_block(h, enc, cu_q, cu_k, max_len_q, max_len_k, bw, weights.position_bias)
     return _T5FinalNorm.apply(h, weights.final_ln, weights.eps)
+
+
+# ------------------------------------------------------------------------------------------------ the objective: labels -> CE -> enc grad
+IGNORE_INDEX = -100
+
+
+def pack_labels(labels: torch.Tensor, vocab_size: int):
+    """The tokenizer's right-padded labels ``[B, T]`` int64 (-100 = ignored) -> ``(flat int64 [Mq], lens int32 [B], max_len_q)`` on
+    ``labels``' device: sample b keeps its positions up to and including its last label that is not -100 (none when all are -100),
+    interior -100s included -- the loss ignores them and the decoder input after them is the pad token, as in HF. Packing is exact for
+    the loss: under the causal mask a kept position never sees a dropped one, and dropped positions carry no loss. Rejects labels
+    outside [0, vocab_size) other than -100 (the decoder-input kernel would give them a zero row, HF an index error)."""
+    if labels.dim() != 2 or labels.dtype != torch.int64:
+        raise TypeError(f"pack_labels: labels must be int64 [B, T], got {labels.dtype} {tuple(labels.shape)}")
+    keep = labels != IGNORE_INDEX
+    bad = keep & ((labels < 0) | (labels >= vocab_size))
+    if bool(bad.any()):
+        raise ValueError(f"pack_labels: label ids must be -100 or in [0, {vocab_size}); got {labels[bad][:4].tolist()}")
+    pos = torch.arange(1, labels.shape[1] + 1, device=labels.device)
+    lens = (keep * pos).amax(dim=1) if labels.shape[1] else torch.zeros(labels.shape[0], dtype=torch.int64, device=labels.device)
+    flat = labels[pos[None, :] <= lens[:, None]]
+    return flat.contiguous(), lens.to(torch.int32), int(lens.max()) if lens.numel() else 0
+
+
+def _scales_decoder_output(cfg) -> bool:
+    """Whether the model multiplies the decoder output by d_model^-0.5 before ``lm_head``: ``scale_decoder_outputs`` in transformers
+    5.x, ``tie_word_embeddings`` before it (4.46.1: ``if self.config.tie_word_embeddings: sequence_output *= model_dim**-0.5``)."""
+    scale = getattr(cfg, "scale_decoder_outputs", None)
+    return bool(getattr(cfg, "tie_word_embeddings", True) if scale is None else scale)
+
+
+class T5ForDecoderWeights:
+    """Frozen weights of the reference's objective (``T5ForDecoder.forward``, thinkdiff/models/mllama_vllm_t5_embed_decoder_2.py:211-246):
+    ``decoder`` (``T5DecoderWeights``), ``embed`` and ``lm_head`` ([V, d] bf16), ``decoder_start_token_id`` and ``pad_token_id``. Only the
+    unscaled head is built (Flan-T5-XXL's, untied in its config): a configuration that scales the decoder output before ``lm_head`` is
+    rejected."""
+
+    def __init__(self, decoder: T5DecoderWeights, embed: torch.Tensor, lm_head: torch.Tensor, decoder_start_token_id: int = 0,
+                 pad_token_id: int = 0):
+        _frozen((("embed_tokens.weight", embed), ("lm_head.weight", lm_head)))
+        d = decoder.blocks[0].d
+        if embed.dim() != 2 or embed.shape[1] != d or tuple(lm_head.shape) != tuple(embed.shape):
+            raise ValueError(f"T5ForDecoderWeights: need embed and lm_head [V, {d}], got {tuple(embed.shape)} and {tuple(lm_head.shape)}")
+        if d % 8:
+            raise ValueError(f"T5ForDecoderWeights: d = {d} must be a multiple of 8")
+        self.decoder = decoder
+        self.embed = embed.detach().to(torch.bfloat16).contiguous()
+        self.lm_head = lm_head.detach().to(torch.bfloat16).contiguous()
+        self.vocab_size = int(embed.shape[0])
+        self.decoder_start_token_id, self.pad_token_id = int(decoder_start_token_id), int(pad_token_id)
+        for n, t in (("decoder_start_token_id", self.decoder_start_token_id), ("pad_token_id", self.pad_token_id)):
+            if not 0 <= t < self.vocab_size:
+                raise ValueError(f"T5ForDecoderWeights: {n} = {t} is outside [0, {self.vocab_size})")
+
+    @staticmethod
+    def _check_config(cfg):
+        if _scales_decoder_output(cfg):
+            raise NotImplementedError("T5ForDecoderWeights: this configuration scales the decoder output by d_model^-0.5 before lm_head "
+                                      "(tie_word_embeddings / scale_decoder_outputs); only the unscaled head (Flan-T5) is built")
+
+    @classmethod
+    def from_module(cls, model) -> "T5ForDecoderWeights":
+        """From a live transformers ``T5ForConditionalGeneration`` whose decoder, embedding and head are frozen."""
+        cfg = model.config
+        cls._check_config(cfg)
+        return cls(T5DecoderWeights.from_module(model.decoder), model.get_input_embeddings().weight, model.lm_head.weight,
+                   cfg.decoder_start_token_id, cfg.pad_token_id)
+
+    @classmethod
+    def from_state_dict(cls, sd: dict, config) -> "T5ForDecoderWeights":
+        """From a ``T5ForConditionalGeneration`` state dict (``decoder.block.{i}...``, ``decoder.final_layer_norm.weight``,
+        ``shared.weight``, ``lm_head.weight``) and its ``T5Config``."""
+        cls._check_config(config)
+        dec = T5DecoderWeights.from_state_dict(sd, config.num_heads, config.layer_norm_epsilon, prefix="decoder.",
+                                               num_buckets=config.relative_attention_num_buckets,
+                                               max_distance=config.relative_attention_max_distance)
+        embed = sd["shared.weight"] if "shared.weight" in sd else sd["decoder.embed_tokens.weight"]
+        return cls(dec, embed, sd["lm_head.weight"], config.decoder_start_token_id, config.pad_token_id)
+
+    def to(self, device) -> "T5ForDecoderWeights":
+        self.decoder.to(device)
+        self.embed, self.lm_head = self.embed.to(device), self.lm_head.to(device)
+        return self
+
+
+class _T5DecoderLoss(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, enc, cu_k, max_len_k, labels, cu_q, max_len_q, weights):
+        e2 = enc.reshape(-1, enc.shape[-1])
+        loss, d_enc = ops.t5_decoder_loss_fwd_bwd(e2, cu_k, max_len_k, labels, cu_q, max_len_q, weights, 1.0, want_grad=True)
+        ctx.d_enc, ctx.shape, ctx.dtype = d_enc, enc.shape, enc.dtype
+        return loss
+
+    @staticmethod
+    def backward(ctx, g):
+        d_enc = ctx.d_enc
+        ctx.d_enc = None
+        return d_enc.mul_(g.to(d_enc.dtype)).view(ctx.shape).to(ctx.dtype), None, None, None, None, None, None
+
+
+def t5_decoder_loss(enc: torch.Tensor, cu_k: torch.Tensor, max_len_k: int, labels: torch.Tensor, cu_q: torch.Tensor, max_len_q: int,
+                    weights: T5ForDecoderWeights) -> torch.Tensor:
+    """The loss of ``T5ForDecoder.forward(encoder_outputs=..., labels=...)`` (thinkdiff/models/mllama_vllm_t5_embed_decoder_2.py:211-246,
+    called at :590-598) on packed rows: ``CrossEntropyLoss(ignore_index=-100)`` of the frozen decoder's logits, the decoder reading its
+    inputs from the labels (``_shift_right`` + ``embed_tokens``) and cross-attending to the aligner rows. ``enc [Mk, d]`` (fp32 in
+    training, or bf16) packed with ``cu_k``; ``labels`` / ``cu_q`` / ``max_len_q`` from ``pack_labels`` (``cu_q = ops.cu_seqlens(lens)``).
+
+    One autograd node over ``ops.t5_decoder_loss_fwd_bwd``: the gradient is formed in the forward, summed over the blocks in fp32, and
+    the backward multiplies it by the upstream scalar; it reaches ``enc`` in ``enc``'s dtype, never rounded to bf16 on the way. Without
+    a gradient to form (``no_grad``, or ``enc`` not requiring one) only the forward runs and nothing is kept."""
+    if torch.is_grad_enabled() and enc.requires_grad:
+        return _T5DecoderLoss.apply(enc, cu_k, int(max_len_k), labels, cu_q, int(max_len_q), weights)
+    loss, _ = ops.t5_decoder_loss_fwd_bwd(enc.detach().reshape(-1, enc.shape[-1]), cu_k, int(max_len_k), labels, cu_q, int(max_len_q), weights,
+                                          want_grad=False)
+    return loss

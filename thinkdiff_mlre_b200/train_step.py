@@ -52,6 +52,22 @@ def synthetic_lvlm_batch(num_seqs: int, max_len: int, din: int, d: int, seed: in
     return FlatBatch(flat, start, lens, int(lens.max()), extras)
 
 
+def _optimizer_step(optimizer, loss_scale: float):
+    """Unscale (``FusedAdamW`` folds 1 / loss_scale into its update; a torch optimizer gets the gradients divided first), step, and
+    drop the gradients. No-op without an optimizer."""
+    if optimizer is None:
+        return
+    from .optim import FusedAdamW
+
+    if isinstance(optimizer, FusedAdamW):
+        optimizer.grad_scale = 1.0 / loss_scale
+    elif loss_scale != 1.0:
+        for group in optimizer.param_groups:
+            torch._foreach_mul_([p.grad for p in group["params"] if p.grad is not None], 1.0 / loss_scale)
+    optimizer.step()
+    optimizer.zero_grad(set_to_none=True)
+
+
 class AlignerTrainStep:
     """One data-parallel training step of the aligner against T5-space targets (masked MSE).
 
@@ -148,16 +164,7 @@ class AlignerTrainStep:
                 y = self.aligner.forward_packed(packed.x, packed.cu_seqlens)
             loss, dy = ops.masked_mse_fwd_bwd(y, target, None, self.loss_scale)
             y.backward(dy)
-        if self.optimizer is not None:
-            from .optim import FusedAdamW
-
-            if isinstance(self.optimizer, FusedAdamW):
-                self.optimizer.grad_scale = 1.0 / self.loss_scale
-            elif self.loss_scale != 1.0:
-                for group in self.optimizer.param_groups:
-                    torch._foreach_mul_([p.grad for p in group["params"] if p.grad is not None], 1.0 / self.loss_scale)
-            self.optimizer.step()
-            self.optimizer.zero_grad(set_to_none=True)
+        _optimizer_step(self.optimizer, self.loss_scale)
         return loss
 
     def _step_controlled(self, packed, target) -> torch.Tensor:
@@ -428,3 +435,60 @@ class AlignerTrainStep:
             ev.record()
             cb([ev])
         return self.step_device(flat, start, lens, batch.total_rows, batch.l_max, tgt)
+
+
+class AlignerT5TrainStep:
+    """One training step of the aligner against the reference's objective (thinkdiff/models/mllama_vllm_t5_embed_decoder_2.py:585-598):
+    the aligner output goes into the frozen T5 decoder as its encoder states and the loss is ``CrossEntropyLoss(ignore_index=-100)`` of
+    the decoder's logits against the caption labels. Runs without autograd, as one direct call sequence: pack, aligner forward (fp32
+    output with saved activations, the training regime), ``ops.t5_decoder_loss_fwd_bwd``, aligner backward from the fp32 encoder
+    gradient into flat gradient buckets (the parameters' ``.grad`` are views of them), then the optimizer -- ``FusedAdamW`` with
+    ``grad_scale = 1 / loss_scale``, or a torch optimizer with the gradients unscaled first. Without an optimizer the (scaled) gradients
+    are left in ``.grad``. The static ``loss_scale`` is applied by the aligner backward, whose epilogues multiply in fp32, so a power of
+    two scales every gradient exactly; the cross-entropy kernel folds its own ``grad_scale`` into the exponent of the softmax
+    (``exp2(z log2 e - m + log2(scale / sum))``), where a scale moves the rounding of the logits' gradient.
+
+    Same kernels and arithmetic as ``forward_packed`` under bf16 autocast + ``t5_decoder_loss(...).backward()``. One GPU: data
+    parallel, a GradScaler, clipping and gradient accumulation are not built for this objective."""
+
+    def __init__(self, aligner: ThinkDiffAligner, t5_weights, optimizer=None, loss_scale: float = 1.0, grad_scaler=None,
+                 max_grad_norm: float = 0.0, accum_grad_iters: int = 1):
+        if grad_scaler is not None or max_grad_norm > 0.0 or accum_grad_iters != 1:
+            raise NotImplementedError("AlignerT5TrainStep: a GradScaler, gradient clipping and gradient accumulation are not built for "
+                                      "the T5 objective (use a static loss_scale)")
+        self._single_gpu(aligner)
+        if aligner[0].weight.dtype != torch.float32:
+            raise TypeError("AlignerT5TrainStep is a training step: the aligner's parameters must be float32 masters")
+        self.aligner, self.t5, self.optimizer, self.loss_scale = aligner, t5_weights, optimizer, float(loss_scale)
+
+    @staticmethod
+    def _single_gpu(aligner):
+        if aligner._dp is not None:
+            raise NotImplementedError("AlignerT5TrainStep runs on one GPU: data parallel is not built for the T5 objective "
+                                      "(call aligner.disable_data_parallel())")
+
+    def step_device(self, flat, src_row_start, lens_dev, total_rows: int, l_max: int, labels, lens_q_dev, max_len_q: int) -> torch.Tensor:
+        """Inputs already resident in HBM: the aligner's flat features with ``src_row_start`` / ``lens_dev`` (as ``AlignerTrainStep``),
+        ``labels`` int64 [Mq] and ``lens_q_dev`` int32 [B] from ``t5.pack_labels``, ``max_len_q`` their longest sample. Returns the
+        (unscaled) loss as a device scalar; nothing syncs the host."""
+        from .aligner import GradBuckets
+
+        a = self.aligner
+        self._single_gpu(a)
+        cu_k = ops.cu_seqlens(lens_dev)
+        x = ops.pack_varlen(flat, src_row_start, cu_k, total_rows).to(torch.bfloat16)
+        cu_q = ops.cu_seqlens(lens_q_dev)
+        W1b, b1b, W2b, b2b = a._bf16_params()
+        g = a[3].weight.detach()
+        y, saved = ops.aligner_fwd(x, W1b, b1b, W2b, b2b, g, a.eps, False, True)
+        loss, d_enc = ops.t5_decoder_loss_fwd_bwd(y, cu_k, l_max, labels, cu_q, max_len_q, self.t5)
+        del y
+        bwd = ops.AlignerBackward(x, saved, W2b, g, d_enc, grad_scale=self.loss_scale)
+        gb = GradBuckets(a.mm_hidden_size, a.hidden_size, x.device)
+        a._grad_flats = gb.flats()
+        bwd.norm_and_linear2(gb.dW2, gb.db2, gb.dg)
+        bwd.gelu_and_linear1(gb.dW1, gb.db1)
+        for p, gr in zip((a[0].weight, a[0].bias, a[2].weight, a[2].bias, a[3].weight), gb.in_parameter_order()):
+            p.grad = gr
+        _optimizer_step(self.optimizer, self.loss_scale)
+        return loss
