@@ -25,14 +25,11 @@ The whole step is checked bit-identical to the staged calls (and exactly 65536 t
 PDL-chained step bit-identical to a serialized one (per-launch profiling puts an event between every two kernels), and TMA
 reduce-add gradient accumulation equal to the float64 sum of two micro-batches, per element.
 """
-import ctypes as C
-import json
-import time
-
 import pytest
 import torch
 
 import _aligner_step_ref as R
+from _parity_report import Report, shared_tile, tail_class, workers
 
 pytestmark = pytest.mark.gpu
 
@@ -60,75 +57,9 @@ def gemm_mnk(name, M):
     return {"fwd1": (M, D, DIN), "fwd2": (M, D, D), "dh0": (M, D, D), "dW1": (D, DIN, M), "dW2": (D, D, M)}[name]
 
 
-def schedule(M, N, K, workers):
-    from thinkdiff_mlre_b200 import _lib as L
-
-    f = L.lib().td_gemm_schedule
-    n = f(M, N, K, workers, 1, None, 0)
-    assert n > 0
-    buf = (C.c_int32 * (8 * n))()
-    assert f(M, N, K, workers, 1, buf, n) == n
-    keys = ("unit", "tile", "kb0", "kb1", "kind", "contrib0", "contrib_n", "range")
-    return [dict(zip(keys, buf[8 * i : 8 * i + 8])) for i in range(n)]
-
-
-def tail_class(M, N, K, workers):
-    owners = [s for s in schedule(M, N, K, workers) if s["kind"] == 1]
-    if owners:
-        return f"split({max(s['contrib_n'] for s in owners)})"
-    tiles = -(-M // 256) * -(-N // 256)
-    return "tail unsplit" if tiles % workers else "no tail"
-
-
-def workers():
-    return torch.cuda.get_device_properties(0).multi_processor_count // 2
-
-
 def assert_classes(M, want):
     got = tuple(tail_class(*gemm_mnk(g, M), workers()) for g in GEMMS)
     assert got == want, f"M={M}: tail classes {dict(zip(GEMMS, got))}, this case is meant to cover {dict(zip(GEMMS, want))}"
-
-
-def shared_tile(name, M):
-    """Rows, columns and the smallest contributor's k-range [k0, k1) (elements) of the first shared tail tile of GEMM ``name``."""
-    from thinkdiff_mlre_b200 import _lib as L
-
-    Mg, N, K = gemm_mnk(name, M)
-    segs = schedule(Mg, N, K, workers())
-    owner = next(s for s in segs if s["kind"] == 1)
-    c = min((s for s in segs if s["kind"] == 2 and s["tile"] == owner["tile"]), key=lambda s: s["kb1"] - s["kb0"])
-    m_blk, n_blk = C.c_int32(-1), C.c_int32(-1)
-    # the GEMMs' own tile raster (tile_coords); the row count is rounded up to the multiple of 32 the call checks for, which
-    # never changes the number of 256-row blocks
-    assert L.lib().td_scatter_tile_owner(owner["tile"], -(-Mg // 32) * 32, N, 1, -1, C.addressof(m_blk), C.addressof(n_blk)) == 0
-    rows = slice(m_blk.value * 256, min(Mg, m_blk.value * 256 + 256))
-    cols = slice(n_blk.value * 256, n_blk.value * 256 + 256)
-    return rows, cols, (c["kb0"] * 64, min(K, c["kb1"] * 64))
-
-
-class Report:
-    """Collects every check's worst err / tol and its out-of-bound count, prints one JSON line, then fails on any violation."""
-
-    def __init__(self, label):
-        self.label, self.t0 = label, time.time()
-        self.worst, self.bad, self.info, self.failures = {}, {}, {}, []
-
-    def check(self, name, err, tol):
-        ratio = torch.where(tol > 0, err / torch.where(tol > 0, tol, 1.0), torch.where(err > 0, float("inf"), 0.0))
-        self.worst[name] = max(self.worst.get(name, 0.0), float(ratio.max()))
-        self.bad[name] = self.bad.get(name, 0) + int((err > tol).sum())
-
-    def require(self, ok, msg):
-        if not ok:
-            self.failures.append(msg)
-
-    def finish(self):
-        fails = [f"{n}: {b} elements outside the bound (worst err/tol {self.worst[n]:.3g})" for n, b in self.bad.items() if b]
-        fails += self.failures
-        print("ALIGNER_STEP_PARITY " + json.dumps({"case": self.label, "worst_err_over_tol": {k: round(v, 4) for k, v in self.worst.items()},
-                                                   **self.info, "seconds": round(time.time() - self.t0, 1),
-                                                   "peak_gb": round(torch.cuda.max_memory_allocated() / 2 ** 30, 2)}))
-        assert not fails, f"{self.label}: " + "; ".join(fails)
 
 
 @pytest.fixture(scope="module")
@@ -263,7 +194,7 @@ def check_bounds_can_fail(M, params, x, k, classes, rep):
     for name, cls in zip(GEMMS, classes):
         if not cls.startswith("split"):
             continue
-        rows, cols, (k0, k1) = shared_tile(name, M)
+        rows, cols, (k0, k1) = shared_tile(*gemm_mnk(name, M))
         a, b, bias, gp = tile_operands(name, params, x, k, rows, cols)
         ep = EPILOGUE[name]
         if ep == "f32":
